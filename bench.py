@@ -14,7 +14,8 @@ weights (fc_1 re-randomised, it is zero-initialised in the reference).
 A step = one pass over the whole lattice: fused decode of nx^3 queries + marching cubes.  N>1:
 x-slabs over the ranks, every rank extracts the mesh piece of its slab and the pieces are gathered
 on rank 0 (device-side signalling over NVLink peer memory; --exchange selects the older schemes).
-`value`  : nx^3 / step time, features already resident in HBM (device timed, CUDA events).
+`value`  : nx^3 / step time, features already resident in HBM (device timed, CUDA events); they are computed
+           once on the host (host_grid_features), so that every run decodes the same bits.
 `e2e`    : the same through Generator3D.capture_generate with HOST buffers: pinned point
            cloud -> H2D -> encoder (PointNet kernels + UNet3D) [-> broadcast] -> decode -> MC -> mesh D2H.
 `--impl reference`: the reference's CPU implementation of the path (the oracle port: same
@@ -22,6 +23,8 @@ on rank 0 (device-side signalling over NVLink peer memory; --exchange selects th
            reference is Python and is not present on the GPU box) on a bounded sample of the lattice.
 `identity_ok` (N>1): the mesh assembled from the ranks' pieces equals, bit for bit, the mesh rank 0
            computes alone from the same features (checked before the timed region).
+`--dump-outputs DIR` (N=1): after the timed steps, what the last step computed as DIR/<name>.npy, so that
+           two builds can be compared output for output (see dump_outputs).
 """
 import argparse
 import json
@@ -41,6 +44,8 @@ METRIC = 'occupancy query-points/sec (dense lattice decode + marching cubes)'
 UNIT = 'query-points/s'
 FLOP_PER_QUERY = 30976          # algorithmic MLP FLOPs/query (LocalDecoder.forward; SURVEY §8a a12)
 FLOP_PER_QUERY_IMG = 33024      # forward_img with a dense c_img tensor
+DUMP_BYTES = 64 << 20           # --dump-outputs: upper bound of all files together
+DUMP_LOGITS = 1 << 20           # --dump-outputs: lattice points in the logit sample
 
 
 def env_int(name, default):
@@ -79,6 +84,26 @@ def build_models(device, seed=0):
             for b in m.blocks:
                 b.fc_1.weight.normal_(0, 0.1)
     return ConvolutionalOccupancyNetwork(dec, enc, device=device).eval()
+
+
+def host_grid_features(net, cloud):
+    """The encoder's grid features of `cloud` (numpy (T, 3)) computed on the host by the reference computation
+    (the oracle's PointNet and the UNet3D modules' torch.nn path, fp32): (1, 32, 64, 64, 64) float32.
+    The timed step decodes these so that its input is the same bits on every run; the GPU encoder sums the
+    grid's scatter-mean and its GroupNorm statistics with atomics, whose order varies from run to run.  One host
+    thread: the summation order of the host convolution depends on the thread count."""
+    import copy
+    from oracle import convonet as oc
+    enc = net.encoder
+    W = {k: v.detach().cpu() for k, v in enc.state_dict().items()}
+    threads = torch.get_num_threads()
+    torch.set_num_threads(1)
+    try:
+        with torch.no_grad():
+            fea = oc.encoder_pointnet(torch.from_numpy(cloud)[None], W, plane_type='grid', reso_grid=64)['grid']
+            return copy.deepcopy(enc.unet3d).cpu()(fea)
+    finally:
+        torch.set_num_threads(threads)
 
 
 # --------------------------------------------------------------------------------------
@@ -271,11 +296,39 @@ def workload_config(nx, args):
             'l2': 'flushed between timed steps (256 MiB write outside the step events; N>1: followed by an untimed '
                   'device-side rendezvous so that every rank\'s step event starts aligned)',
             'kernel_variant': args.variant,
+            'features': 'timed step: the grid features of the synthetic cloud computed once on the host (host_grid_features: '
+                        'fp32 reference computation of the same encoder weights); e2e: the GPU encoder',
             'unet3d_conv_math': 'e2e only: UNet3D runs on our tcgen05 implicit-GEMM kernels (csrc/conv3d.cu) in single-pass TF32 '
                                 'with fp32 accumulation - the arithmetic of the reference on a GPU (cuDNN, '
                                 'torch.backends.cudnn.allow_tf32 = True by default; tests/test_unet3d_gpu.py: same deviation '
                                 'from fp32 as cuDNN TF32, 4.4e-3 mean); PointNet, decoder and marching cubes are fp32-accurate '
                                 '(3xTF32 on the tensor pipe)'}
+
+
+def dump_outputs(path, mesh, grid):
+    """Write what one step computed as float32 / float64 .npy files under `path`:
+    vertices.npy (V, 3) float32 and faces.npy (F, 3) float64 (the int32 vertex ids, exact): the mesh the step
+        returns; if the two together exceed DUMP_BYTES less the logit sample, both keep the same fraction of
+        their rows, drawn with RandomState(0) and kept in order;
+    logits_sample.npy (DUMP_LOGITS,) float32: the step's lattice logits at DUMP_LOGITS distinct flat (x, y, z)
+        indices of the nx^3 grid, drawn with RandomState(0) and sorted.
+    Vertex and face order are those of the extractor, so equal meshes give equal files."""
+    v, f, counts = mesh
+    V, F = [int(x) for x in counts[:2].cpu()]
+    out = {'vertices': v[:V].cpu().numpy().astype(np.float32), 'faces': f[:F].cpu().numpy().astype(np.float64)}
+    flat = grid.reshape(-1)
+    idx = np.sort(np.random.RandomState(0).choice(flat.numel(), min(DUMP_LOGITS, flat.numel()), replace=False))
+    out['logits_sample'] = flat[torch.from_numpy(idx).to(flat.device)].cpu().numpy().astype(np.float32)
+    mesh_bytes = out['vertices'].nbytes + out['faces'].nbytes
+    budget = DUMP_BYTES - out['logits_sample'].nbytes - 3 * 1024      # (and the three .npy headers)
+    if mesh_bytes > budget:
+        for k in ('vertices', 'faces'):
+            a = out[k]
+            keep = int(len(a) * budget // mesh_bytes)
+            out[k] = a[np.sort(np.random.RandomState(0).choice(len(a), keep, replace=False))]
+    os.makedirs(path, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(path, k + '.npy'), a)
 
 
 # --------------------------------------------------------------------------------------
@@ -303,9 +356,11 @@ def run_ours(args, rank, local_rank, world):
     tip_feat_host = torch.from_numpy(tip_feat_np).pin_memory()
     tip_feat = tip_feat_host.to(dev)
 
-    def encode_features():
+    def encode_features(host_grid=None):
         with torch.no_grad():
-            if rank == 0:
+            if rank == 0 and host_grid is not None:
+                g = host_grid.to(dev).contiguous(memory_format=torch.channels_last_3d)   # the encoder's layout
+            elif rank == 0:
                 c = net.encode_inputs(cloud_host.to(dev, non_blocking=True))
                 g = c['grid']
             else:
@@ -322,7 +377,7 @@ def run_ours(args, rank, local_rank, world):
         with torch.no_grad():
             return net.encode_inputs(cloud_host.to(dev, non_blocking=True))
 
-    c = encode_features()
+    c = encode_features(host_grid_features(net, cloud_np) if rank == 0 else None)
     tips_arg = (tips, tip_feat, touch, 0.05)
     exchange_note = None
     if world > 1 and args.exchange == 'root':
@@ -430,10 +485,11 @@ def run_ours(args, rank, local_rank, world):
 
     # ---- CUDA graph of the step (decode [+ exchange] + marching cubes) ----
     graph, graph_note = None, 'eager launches'
+    step_out = None         # (vertex buffer, face buffer, counts) the timed step writes, for --dump-outputs
     if not args.no_graph and (world == 1 or args.exchange in ('fused', 'root', 'mesh')):
         ok = torch.ones(1, device=dev)
         try:
-            graph, _ = gen.capture_step(c, tips=tips_arg, group=group, exchange=args.exchange)
+            graph, step_out = gen.capture_step(c, tips=tips_arg, group=group, exchange=args.exchange)
             graph.replay()
             torch.cuda.synchronize(dev)
         except Exception as e:  # noqa: BLE001
@@ -477,10 +533,13 @@ def run_ours(args, rank, local_rank, world):
                 grid, keys = gen.eval_lattice(c, tips=tips_arg, group=None if world == 1 else group,
                                               exchange=args.exchange)
                 e_dec.record()
-                gen.mc(grid, level_keys=keys, voffset=np.float32(nx / 2), vscale=np.float32(1.1 / nx), sync=False)
+                step_out = gen.mc(grid, level_keys=keys, voffset=np.float32(nx / 2), vscale=np.float32(1.1 / nx),
+                                  sync=False)
             e1.record()
         barrier()
     wall = time.perf_counter() - wall0
+    if args.dump_outputs:   # before the decoder-alone and e2e runs below re-use the generator's buffers
+        dump_outputs(args.dump_outputs, step_out, gen._grid)
     step_ms = [e0.elapsed_time(e1) for e0, _, e1 in ev]
     dec_ms = [e0.elapsed_time(ed) for e0, ed, _ in ev]
     if graph is not None:   # stages are inside one graph launch: split by the separately timed decoder kernel below
@@ -736,8 +795,15 @@ def main():
                          'root = slabs pushed into rank 0 only by bulk peer copies (double-buffered, 1 barrier/step, MC on '
                          'rank 0, rank 0 decodes fewer rows); fused = decoder stores slabs into every rank (NVLS multicast); '
                          'nccl = all_gather_into_tensor')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='one GPU: after the timed steps write the mesh and a fixed sample of the lattice logits of '
+                         'the last step as DIR/<name>.npy (float32 / float64, at most 64 MB)')
     args = ap.parse_args()
     rank, local_rank, world = env_int('RANK', 0), env_int('LOCAL_RANK', 0), env_int('WORLD_SIZE', 1)
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'ours' or world > 1):
+        ap.error('--dump-outputs applies to --impl ours on one GPU')
     if args.exchange == 'auto':
         args.exchange = 'mesh'
     os.environ.setdefault('MASTER_ADDR', '127.0.0.1')
