@@ -83,27 +83,29 @@ int vtaco_relayout_cf(const float* src, float* dst, int B, int C, int64_t S, voi
  * In dense mode it also replaces make_3d_grid (src/common.py:178-197) and the
  * chunk loop of Generator3D.eval_points (src/conv_onet/generation.py:338-383).
  *
- * Packed weight buffer (fp32, device), hidden = c_dim = 32, K-major ("[in][out]"):
- *   off 0      fc_p.weight^T        [3][32]
- *   off 96     fc_p.bias            [32]
- *   off 128    fc_p_img.weight[:, :3]^T [3][32]
- *   off 224    fc_p_img.bias        [32]
- *   off 256    fc_p_img.weight[:, 3:]^T [32][32]
- *   off 1280   per block i (stride 3168):
- *                fc_c[i].weight^T [32][32], fc_c[i].bias [32],
- *                blocks[i].fc_0.weight^T [32][32], .bias [32],
- *                blocks[i].fc_1.weight^T [32][32], .bias [32]
- *   off 1280+3168*n_blocks  fc_out.weight [32], fc_out_contact.weight [32],
- *                fc_out.bias, fc_out_contact.bias, 2 pad
+ * Packed weight buffer (fp32, device), hidden = c_dim = 32: every weight K-major ("[in][out]", the
+ * transpose of nn.Linear's), fc_p_img.weight split by columns into the 3 point inputs (OFF_WPI) and the
+ * 32 c_img inputs (OFF_WIMG).  n_blocks blocks of BLOCK_STRIDE floats start at OFF_BLOCKS (offsets
+ * VTACO_DEC_BLK_* inside a block), then the tail (offsets VTACO_DEC_TAIL_*; 2 floats of padding).
  * ------------------------------------------------------------------------- */
 #define VTACO_DEC_HIDDEN 32
-#define VTACO_DEC_OFF_WP 0
-#define VTACO_DEC_OFF_BP 96
-#define VTACO_DEC_OFF_WPI 128
-#define VTACO_DEC_OFF_BPI 224
-#define VTACO_DEC_OFF_WIMG 256
+#define VTACO_DEC_OFF_WP 0        /* fc_p.weight^T [3][32] */
+#define VTACO_DEC_OFF_BP 96       /* fc_p.bias [32] */
+#define VTACO_DEC_OFF_WPI 128     /* fc_p_img.weight[:, :3]^T [3][32] */
+#define VTACO_DEC_OFF_BPI 224     /* fc_p_img.bias [32] */
+#define VTACO_DEC_OFF_WIMG 256    /* fc_p_img.weight[:, 3:]^T [32][32] */
 #define VTACO_DEC_OFF_BLOCKS 1280
 #define VTACO_DEC_BLOCK_STRIDE 3168
+#define VTACO_DEC_BLK_WC 0        /* fc_c[i].weight^T [32][32] */
+#define VTACO_DEC_BLK_BC 1024     /* fc_c[i].bias [32] */
+#define VTACO_DEC_BLK_W0 1056     /* blocks[i].fc_0.weight^T [32][32] */
+#define VTACO_DEC_BLK_B0 2080     /* blocks[i].fc_0.bias [32] */
+#define VTACO_DEC_BLK_W1 2112     /* blocks[i].fc_1.weight^T [32][32] */
+#define VTACO_DEC_BLK_B1 3136     /* blocks[i].fc_1.bias [32] */
+#define VTACO_DEC_TAIL_WOUT 0     /* fc_out.weight [32] */
+#define VTACO_DEC_TAIL_WCON 32    /* fc_out_contact.weight [32] */
+#define VTACO_DEC_TAIL_BOUT 64    /* fc_out.bias */
+#define VTACO_DEC_TAIL_BCON 65    /* fc_out_contact.bias */
 #define VTACO_DEC_TAIL 68
 #define VTACO_DEC_PACKED_FLOATS(n_blocks) (VTACO_DEC_OFF_BLOCKS + VTACO_DEC_BLOCK_STRIDE * (n_blocks) + VTACO_DEC_TAIL)
 #define VTACO_MAX_TIPS 8
@@ -203,12 +205,9 @@ int vtaco_sample_features(const vtaco_decoder_args* args, const float* p, int64_
  * produced (the reference never asks for it).
  *
  * d_params: flat fp32 buffer of VTACO_DEC_PACKED_FLOATS(n_blocks) floats, ACCUMULATED into
- * (zero it first): same offsets as the packed forward weights, but each matrix in nn.Linear's
- * native [out][in] orientation — fc_p.weight [32][3] at OFF_WP, fc_p.bias at OFF_BP,
- * fc_p_img.weight[:, :3] [32][3] at OFF_WPI, fc_p_img.bias at OFF_BPI, fc_p_img.weight[:, 3:]
- * [32][32] at OFF_WIMG; per block at OFF_BLOCKS + i*BLOCK_STRIDE: fc_c[i].weight, .bias (+1024),
- * fc_0.weight (+1056), .bias (+2080), fc_1.weight (+2112), .bias (+3136); tail: fc_out.weight
- * [32], fc_out_contact.weight [32] (+32), fc_out.bias (+64), fc_out_contact.bias (+65).
+ * (zero it first): the fields of the packed forward weights (VTACO_DEC_OFF_*, _BLK_*, _TAIL_*), but
+ * each matrix in nn.Linear's native [out][in] orientation (fc_p_img.weight[:, :3] [32][3] at OFF_WPI,
+ * fc_p_img.weight[:, 3:] [32][32] at OFF_WIMG).
  * d_grid / d_plane[k]: channels-last gradients [B][R..][32], ACCUMULATED into with vector
  * atomics (NULL = not wanted).  d_c_img: [B][N][32], overwritten (NULL = not wanted).
  * workspace: vtaco_decoder_backward_workspace_bytes(B*N, n_blocks) bytes of device memory. */
@@ -293,15 +292,23 @@ float vtaco_key_to_float_host(int32_t key);
  * memory format, so values/shapes are the reference's and the decoder reads them
  * without a copy.
  *
- * Packed weights (hidden_dim = 32, c_dim = 32), K-major:
- *   off 0    fc_pos.weight^T [3][64];  off 192  fc_pos.bias [64]
- *   off 256  per block i (stride 5184): fc_0.weight^T [64][32], fc_0.bias [32],
- *            fc_1.weight^T [32][32], fc_1.bias [32], shortcut.weight^T [64][32]
- *   off 256+5184*n_blocks  fc_c.weight^T [32][32], fc_c.bias [32]
+ * Packed weights (hidden_dim = 32, c_dim = 32), every weight K-major ("[in][out]"): fc_pos, then
+ * n_blocks blocks of BLOCK_STRIDE floats from OFF_BLOCKS (offsets VTACO_ENC_BLK_* inside a block),
+ * then the fc_c section of VTACO_ENC_TAIL floats (offsets VTACO_ENC_FCC_*).
  * ------------------------------------------------------------------------- */
+#define VTACO_ENC_OFF_WPOS 0      /* fc_pos.weight^T [3][64] */
+#define VTACO_ENC_OFF_BPOS 192    /* fc_pos.bias [64] */
 #define VTACO_ENC_OFF_BLOCKS 256
 #define VTACO_ENC_BLOCK_STRIDE 5184
-#define VTACO_ENC_PACKED_FLOATS(n_blocks) (VTACO_ENC_OFF_BLOCKS + VTACO_ENC_BLOCK_STRIDE * (n_blocks) + 1056)
+#define VTACO_ENC_BLK_W0 0        /* blocks[i].fc_0.weight^T [64][32] */
+#define VTACO_ENC_BLK_B0 2048     /* blocks[i].fc_0.bias [32] */
+#define VTACO_ENC_BLK_W1 2080     /* blocks[i].fc_1.weight^T [32][32] */
+#define VTACO_ENC_BLK_B1 3104     /* blocks[i].fc_1.bias [32] */
+#define VTACO_ENC_BLK_WS 3136     /* blocks[i].shortcut.weight^T [64][32] */
+#define VTACO_ENC_FCC_W 0         /* fc_c.weight^T [32][32] */
+#define VTACO_ENC_FCC_B 1024      /* fc_c.bias [32] */
+#define VTACO_ENC_TAIL 1056
+#define VTACO_ENC_PACKED_FLOATS(n_blocks) (VTACO_ENC_OFF_BLOCKS + VTACO_ENC_BLOCK_STRIDE * (n_blocks) + VTACO_ENC_TAIL)
 
 typedef struct vtaco_encoder_args {
   const float* p;          /* [B][T][3] */
@@ -329,11 +336,9 @@ int vtaco_encoder_pointnet(const vtaco_encoder_args* args, void* stream);
  * src/encoder/pointnet.py:135-172 when training.py trains the encoder.  Given the gradients of
  * the scatter_mean feature tensors (channels-last, [B][cells][32] per key, NULL = no gradient
  * for that key; same key order as vtaco_encoder_args) it ACCUMULATES parameter gradients into
- * d_params (zero it first): the packed layout of the forward weights with every matrix in
- * nn.Linear's native [out][in] orientation — fc_pos.weight [64][3] at 0, fc_pos.bias at 192;
- * block i at 256 + 5184*i: fc_0.weight [32][64] (+0), fc_0.bias (+2048), fc_1.weight [32][32]
- * (+2080), fc_1.bias (+3104), shortcut.weight [32][64] (+3136); fc_c.weight [32][32] at
- * 256 + 5184*n_blocks, fc_c.bias (+1024).  The forward is recomputed inside (nothing is saved
+ * d_params (zero it first): the fields of the packed forward weights (VTACO_ENC_OFF_*, _BLK_*,
+ * _FCC_*) with every matrix in nn.Linear's native [out][in] orientation (fc_pos.weight [64][3],
+ * fc_0.weight [32][64]).  The forward is recomputed inside (nothing is saved
  * by vtaco_encoder_pointnet).  scatter_max routes a cell's gradient to the lowest-index point
  * among exact ties (torch_scatter: one arg-max point, unspecified which). */
 typedef struct vtaco_encoder_bwd_args {

@@ -167,7 +167,7 @@ def test_ctypes_structs_match_the_c_header(tmp_path):
     import shutil
     import subprocess
     from vtaco_b200 import _abi
-    from vtaco_b200.encoder.pointnet import EncoderArgs, EncoderBwdArgs
+    from vtaco_b200._abi import EncoderArgs, EncoderBwdArgs
     if shutil.which('gcc') is None:
         pytest.skip('no C compiler')
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))

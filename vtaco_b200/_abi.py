@@ -19,12 +19,23 @@ KIND = {'xz': PLANE_XZ, 'xy': PLANE_XY, 'yz': PLANE_YZ, 'grid': GRID}
 DIV_RECIPROCAL, DIV_TRUE = 0, 1
 SAMPLE = {'bilinear': 0, 'nearest': 1}
 
+# packed parameter layouts (VTACO_DEC_* / VTACO_ENC_* of include/vtaco_b200.h)
+DEC_HIDDEN = 32
 DEC_OFF_WP, DEC_OFF_BP, DEC_OFF_WPI, DEC_OFF_BPI, DEC_OFF_WIMG = 0, 96, 128, 224, 256
 DEC_OFF_BLOCKS, DEC_BLOCK_STRIDE, DEC_TAIL = 1280, 3168, 68
+DEC_BLK_WC, DEC_BLK_BC, DEC_BLK_W0, DEC_BLK_B0, DEC_BLK_W1, DEC_BLK_B1 = 0, 1024, 1056, 2080, 2112, 3136
+DEC_TAIL_WOUT, DEC_TAIL_WCON, DEC_TAIL_BOUT, DEC_TAIL_BCON = 0, 32, 64, 65
+ENC_OFF_WPOS, ENC_OFF_BPOS, ENC_OFF_BLOCKS, ENC_BLOCK_STRIDE = 0, 192, 256, 5184
+ENC_BLK_W0, ENC_BLK_B0, ENC_BLK_W1, ENC_BLK_B1, ENC_BLK_WS = 0, 2048, 2080, 3104, 3136
+ENC_FCC_W, ENC_FCC_B, ENC_TAIL = 0, 1024, 1056
 
 
 def dec_packed_floats(n_blocks):
     return DEC_OFF_BLOCKS + DEC_BLOCK_STRIDE * n_blocks + DEC_TAIL
+
+
+def enc_packed_floats(n_blocks):
+    return ENC_OFF_BLOCKS + ENC_BLOCK_STRIDE * n_blocks + ENC_TAIL
 
 
 class DecoderArgs(C.Structure):
@@ -55,6 +66,28 @@ class DecoderBwdArgs(C.Structure):
         ('c_img', C.c_void_p), ('dlogits', C.c_void_p), ('dcontact', C.c_void_p),
         ('workspace', C.c_void_p), ('workspace_bytes', C.c_size_t),
         ('d_params', C.c_void_p), ('d_grid', C.c_void_p), ('d_plane', C.c_void_p * 3), ('d_c_img', C.c_void_p),
+    ]
+
+
+class EncoderArgs(C.Structure):
+    _fields_ = [
+        ('p', C.c_void_p), ('B', C.c_int32), ('T', C.c_int64),
+        ('padding', C.c_double), ('div_mode', C.c_int32),
+        ('n_keys', C.c_int32), ('kind', C.c_int32 * 4), ('reso', C.c_int32 * 4),
+        ('pool_mean', C.c_int32), ('n_blocks', C.c_int32),
+        ('weights', C.c_void_p), ('workspace', C.c_void_p), ('workspace_bytes', C.c_int64),
+        ('out_cl', C.c_void_p * 4), ('c_out', C.c_void_p), ('index_out', C.c_void_p * 4),
+    ]
+
+
+class EncoderBwdArgs(C.Structure):
+    _fields_ = [
+        ('p', C.c_void_p), ('B', C.c_int32), ('T', C.c_int64),
+        ('padding', C.c_double), ('div_mode', C.c_int32),
+        ('n_keys', C.c_int32), ('kind', C.c_int32 * 4), ('reso', C.c_int32 * 4),
+        ('pool_mean', C.c_int32), ('n_blocks', C.c_int32),
+        ('weights', C.c_void_p), ('workspace', C.c_void_p), ('workspace_bytes', C.c_int64),
+        ('d_out_cl', C.c_void_p * 4), ('d_params', C.c_void_p),
     ]
 
 
@@ -148,6 +181,42 @@ def pack_linear(entries, dst, cache=None):
         cache['descs'] = (key, descs)
 
 
+def layout_entries(layout, params, n_blocks):
+    """pack_linear entries of every field of a packed parameter buffer, in layout order.
+    layout = (offset of the blocks, block stride, head, block, tail): head entries (parameter name, offset[, first
+    column, columns]), block entries (name with %d for the block index, offset inside the block) for each of the
+    n_blocks blocks, tail entries (name, offset from the end of the blocks).  params: name -> parameter."""
+    off, stride, head, block, tail = layout
+    end = off + n_blocks * stride
+    return ([(params[e[0]],) + e[1:] for e in head] +
+            [(params[name % i], off + i * stride + o) for i in range(n_blocks) for name, o in block] +
+            [(params[name], end + o) for name, o in tail])
+
+
+def layout_grads(layout, params, flat, n_blocks):
+    """name -> gradient of every parameter of `layout` (see layout_entries) from `flat`, a buffer in that layout with
+    every matrix in nn.Linear's [out][in] orientation: views of `flat`, except for a weight packed as column ranges,
+    whose gradient is their concatenation."""
+    off, stride, head, block, tail = layout
+    base, end = flat.storage_offset(), off + n_blocks * stride
+    g, ranges = {}, {}
+    for name, o, *cols in list(head) + [(name, end + o) for name, o in tail]:
+        shape = tuple(params[name].shape)
+        if cols:    # columns [first, first + count) of an [out][in] weight, stored as [out][count]
+            ranges.setdefault(name, []).append(flat.as_strided((shape[0], cols[1]), (cols[1], 1), base + o))
+        else:       # [out][in] or [out], contiguous
+            g[name] = flat.as_strided(shape, shape[1:] + (1,), base + o)
+    for name, parts in ranges.items():
+        g[name] = torch.cat(parts, 1)
+    # a block field is the same view every `stride` floats: one strided view and one unbind per field
+    for name, o in block if n_blocks else ():
+        shape = tuple(params[name % 0].shape)
+        fields = flat.as_strided((n_blocks,) + shape, (stride,) + shape[1:] + (1,), base + off + o).unbind(0)
+        for i, t in enumerate(fields):
+            g[name % i] = t
+    return g
+
+
 _lib = None
 
 
@@ -181,6 +250,20 @@ def lib():
     L.vtaco_decoder_tc_floats.restype = C.c_int64
     L.vtaco_decoder_tc_floats.argtypes = [C.c_int32]
     L.vtaco_decoder_pack_tc.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]
+    L.vtaco_encoder_workspace_bytes.restype = C.c_int64
+    L.vtaco_encoder_workspace_bytes.argtypes = [C.c_int32, C.c_int64, C.c_int32, C.POINTER(C.c_int32),
+                                                C.POINTER(C.c_int32)]
+    L.vtaco_encoder_pointnet.argtypes = [C.POINTER(EncoderArgs), C.c_void_p]
+    L.vtaco_encoder_backward_workspace_bytes.restype = C.c_int64
+    L.vtaco_encoder_backward_workspace_bytes.argtypes = [C.c_int32, C.c_int64, C.c_int32, C.POINTER(C.c_int32),
+                                                         C.POINTER(C.c_int32), C.c_int32]
+    L.vtaco_encoder_backward.argtypes = [C.POINTER(EncoderBwdArgs), C.c_void_p]
+    L.vtaco_pool_workspace_bytes.restype = C.c_int64
+    L.vtaco_pool_workspace_bytes.argtypes = [C.c_int32, C.c_int64, C.c_int32, C.POINTER(C.c_int64)]
+    L.vtaco_pool_local.argtypes = [C.c_void_p, C.c_int32, C.c_int64, C.c_int32, C.POINTER(C.c_void_p),
+                                   C.POINTER(C.c_int64), C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]
+    L.vtaco_scatter_mean.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_int64, C.c_void_p, C.c_int64,
+                                     C.c_void_p, C.c_void_p]
     for name, argtypes in _OPTIONAL.items():
         getattr(L, name).argtypes = argtypes
     L.vtaco_mc_scratch_bytes.restype = C.c_int64

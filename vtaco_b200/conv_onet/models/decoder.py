@@ -137,6 +137,12 @@ class LocalDecoder(nn.Module):
             self.__dict__['_named_params'] = (tuple(names), tuple(params))
         return self.__dict__['_named_params']
 
+    def _params_by_name(self):
+        """name -> parameter, cached like `_param_tuple` (the packed layout names its fields by parameter)."""
+        if self.__dict__.get('_by_name') is None:
+            self.__dict__['_by_name'] = dict(zip(*self._named_param_tuples()))
+        return self.__dict__['_by_name']
+
     def _param_tuple(self):
         """The module's parameters as a cached tuple: `self.parameters()` walks the module tree (37 modules,
         ~25 us) and the hot path needs the list three times per call — it was most of the 0.13 ms a flat call
@@ -168,6 +174,7 @@ class LocalDecoder(nn.Module):
         self._params = None
         self.__dict__['_desc_cache'] = {}
         self.__dict__['_named_params'] = None
+        self.__dict__['_by_name'] = None
 
     def _apply(self, fn, *args, **kwargs):
         self.invalidate()
@@ -176,6 +183,20 @@ class LocalDecoder(nn.Module):
     def _load_from_state_dict(self, *args, **kwargs):
         self.invalidate()
         return super()._load_from_state_dict(*args, **kwargs)
+
+    def _layout(self):
+        """The fields of the packed buffer (include/vtaco_b200.h) this module has, as _abi.layout_entries takes them."""
+        head = [('fc_p.weight', _abi.DEC_OFF_WP), ('fc_p.bias', _abi.DEC_OFF_BP),
+                ('fc_p_img.weight', _abi.DEC_OFF_WPI, 0, self.dim), ('fc_p_img.bias', _abi.DEC_OFF_BPI)]
+        block = [('blocks.%d.fc_0.weight', _abi.DEC_BLK_W0), ('blocks.%d.fc_0.bias', _abi.DEC_BLK_B0),
+                 ('blocks.%d.fc_1.weight', _abi.DEC_BLK_W1), ('blocks.%d.fc_1.bias', _abi.DEC_BLK_B1)]
+        tail = [('fc_out.weight', _abi.DEC_TAIL_WOUT), ('fc_out.bias', _abi.DEC_TAIL_BOUT)]
+        if self.c_dim:
+            head.append(('fc_p_img.weight', _abi.DEC_OFF_WIMG, self.dim, self.c_dim))
+            block[:0] = [('fc_c.%d.weight', _abi.DEC_BLK_WC), ('fc_c.%d.bias', _abi.DEC_BLK_BC)]
+        if hasattr(self, 'fc_out_contact'):
+            tail += [('fc_out_contact.weight', _abi.DEC_TAIL_WCON), ('fc_out_contact.bias', _abi.DEC_TAIL_BCON)]
+        return _abi.DEC_OFF_BLOCKS, _abi.DEC_BLOCK_STRIDE, head, block, tail
 
     def _packed_weights(self):
         """Flat fp32 buffer in the layout documented in include/vtaco_b200.h — one launch of
@@ -190,21 +211,7 @@ class LocalDecoder(nn.Module):
         if nb > _abi.MAX_BLOCKS:
             raise NotImplementedError('vtaco_b200 decoder kernels hold at most %d blocks in shared memory' % _abi.MAX_BLOCKS)
         buf = torch.zeros(_abi.dec_packed_floats(nb), dtype=torch.float32, device=dev)
-        ent = [(self.fc_p.weight, 0), (self.fc_p.bias, 96),
-               (self.fc_p_img.weight, 128, 0, 3), (self.fc_p_img.bias, 224)]
-        if self.c_dim:
-            ent.append((self.fc_p_img.weight, 256, 3, 32))
-        for i in range(nb):
-            o = _abi.DEC_OFF_BLOCKS + i * _abi.DEC_BLOCK_STRIDE
-            if self.c_dim:
-                ent += [(self.fc_c[i].weight, o), (self.fc_c[i].bias, o + 1024)]
-            blk = self.blocks[i]
-            ent += [(blk.fc_0.weight, o + 1056), (blk.fc_0.bias, o + 2080),
-                    (blk.fc_1.weight, o + 2112), (blk.fc_1.bias, o + 3136)]
-        o = _abi.DEC_OFF_BLOCKS + nb * _abi.DEC_BLOCK_STRIDE
-        ent += [(self.fc_out.weight, o), (self.fc_out.bias, o + 64)]
-        if hasattr(self, 'fc_out_contact'):
-            ent += [(self.fc_out_contact.weight, o + 32), (self.fc_out_contact.bias, o + 65)]
+        ent = _abi.layout_entries(self._layout(), self._params_by_name(), nb)
         _abi.pack_linear(ent, buf, cache=self.__dict__.setdefault('_desc_cache', {}))
         self._pack_cache = (key, buf)
         self._pack_tc_cache = None
@@ -436,38 +443,13 @@ class LocalDecoder(nn.Module):
         return d_params, d_feat, d_cimg
 
     def _unpack_param_grads(self, flat, use_img, contact):
-        """name -> gradient views of the flat buffer written by vtaco_decoder_backward."""
-        g = {}
-        nb = self.n_blocks
-        if use_img:
-            parts = [flat[_abi.DEC_OFF_WPI:_abi.DEC_OFF_WPI + 96].view(32, 3)]
-            if self.c_dim:
-                parts.append(flat[_abi.DEC_OFF_WIMG:_abi.DEC_OFF_WIMG + 1024].view(32, 32))
-            g['fc_p_img.weight'] = torch.cat(parts, 1)
-            g['fc_p_img.bias'] = flat[_abi.DEC_OFF_BPI:_abi.DEC_OFF_BPI + 32]
-        else:
-            g['fc_p.weight'] = flat[0:96].view(32, 3)
-            g['fc_p.bias'] = flat[_abi.DEC_OFF_BP:_abi.DEC_OFF_BP + 32]
-        # the blocks are nb consecutive records of (W_c 1024, b_c 32, W_0 1024, b_0 32, W_1 1024, b_1 32) floats:
-        # one view + one unbind per field instead of six slices per block
-        blk = flat[_abi.DEC_OFF_BLOCKS:_abi.DEC_OFF_BLOCKS + nb * _abi.DEC_BLOCK_STRIDE].view(nb, _abi.DEC_BLOCK_STRIDE)
-        fields = (('fc_c.%d.weight', 0, 1024, self.c_dim), ('fc_c.%d.bias', 1024, 32, self.c_dim),
-                  ('blocks.%d.fc_0.weight', 1056, 1024, True), ('blocks.%d.fc_0.bias', 2080, 32, True),
-                  ('blocks.%d.fc_1.weight', 2112, 1024, True), ('blocks.%d.fc_1.bias', 3136, 32, True))
-        for fmt, off, n, on in fields:
-            if not on:
-                continue
-            seg = blk[:, off:off + n]
-            rows = (seg.reshape(nb, 32, 32) if n == 1024 else seg).unbind(0)
-            for i, r in enumerate(rows):
-                g[fmt % i] = r
-        o = _abi.DEC_OFF_BLOCKS + nb * _abi.DEC_BLOCK_STRIDE
-        g['fc_out.weight'] = flat[o:o + 32].view(1, 32)
-        g['fc_out.bias'] = flat[o + 64:o + 65]
-        if contact:
-            g['fc_out_contact.weight'] = flat[o + 32:o + 64].view(1, 32)
-            g['fc_out_contact.bias'] = flat[o + 65:o + 66]
-        return g
+        """name -> gradient of every parameter vtaco_decoder_backward wrote into `flat`: the input layer used
+        (fc_p or fc_p_img), fc_c with c_dim, fc_out_contact with `contact`."""
+        off, stride, head, block, tail = self._layout()
+        unwritten = ('fc_p.' if use_img else 'fc_p_img.',) + (() if contact else ('fc_out_contact.',))
+        head = [e for e in head if not e[0].startswith(unwritten)]
+        tail = [e for e in tail if not e[0].startswith(unwritten)]
+        return _abi.layout_grads((off, stride, head, block, tail), self._params_by_name(), flat, self.n_blocks)
 
     # ------------------------------------------------------------------ reference API
     def forward(self, p, c_plane, **kwargs):

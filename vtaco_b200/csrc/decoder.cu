@@ -204,7 +204,7 @@ __global__ void __launch_bounds__(kThreads, 1) decoder_kernel(const __grid_const
       const float2* w0 = reinterpret_cast<const float2*>(Wp);
       const float2* w1 = reinterpret_cast<const float2*>(Wp + 32);
       const float2* w2 = reinterpret_cast<const float2*>(Wp + 64);
-      const float2* bp = reinterpret_cast<const float2*>(Wp + 96);
+      const float2* bp = reinterpret_cast<const float2*>(Wp + (VTACO_DEC_OFF_BP - VTACO_DEC_OFF_WP));  // = BPI - WPI
 #pragma unroll
       for (int j = 0; j < 16; ++j) {
         const float2 a0 = w0[j], a1 = w1[j], a2 = w2[j], bb = bp[j];
@@ -230,24 +230,25 @@ __global__ void __launch_bounds__(kThreads, 1) decoder_kernel(const __grid_const
     for (int i = 0; i < P.n_blocks; ++i) {
       const float* Wb = sW + VTACO_DEC_OFF_BLOCKS + i * VTACO_DEC_BLOCK_STRIDE;
       if (P.has_c) {  // net = net + fc_c[i](c)                       decoder.py:92-94
-        matvec<F2>(net, Wb, ccol);
-        add_bias(net, Wb + 1024);
+        matvec<F2>(net, Wb + VTACO_DEC_BLK_WC, ccol);
+        add_bias(net, Wb + VTACO_DEC_BLK_BC);
       }
       store_relu(net, xcol);            // ResnetBlockFC: fc_0(relu(x))     layers.py:42
-      set_bias(acc, Wb + 1056 + 1024);
-      matvec<F2>(acc, Wb + 1056, xcol);
+      set_bias(acc, Wb + VTACO_DEC_BLK_B0);
+      matvec<F2>(acc, Wb + VTACO_DEC_BLK_W0, xcol);
       store_relu(acc, xcol);            // fc_1(relu(net))                  layers.py:43
-      matvec<F2>(net, Wb + 2112, xcol);
-      add_bias(net, Wb + 2112 + 1024);  // x_s + dx (identity shortcut)     layers.py:45-50
+      matvec<F2>(net, Wb + VTACO_DEC_BLK_W1, xcol);
+      add_bias(net, Wb + VTACO_DEC_BLK_B1);  // x_s + dx (identity shortcut)     layers.py:45-50
     }
     {
       const float* Wo = sW + VTACO_DEC_OFF_BLOCKS + P.n_blocks * VTACO_DEC_BLOCK_STRIDE;
       const float slope = P.leaky ? 0.2f : 0.0f;
-      float o[2] = {Wo[64], Wo[64]}, oc[2] = {Wo[65], Wo[65]};
+      float o[2] = {Wo[VTACO_DEC_TAIL_BOUT], Wo[VTACO_DEC_TAIL_BOUT]};
+      float oc[2] = {Wo[VTACO_DEC_TAIL_BCON], Wo[VTACO_DEC_TAIL_BCON]};
 #pragma unroll
       for (int j = 0; j < 16; ++j) {
-        const float2 w = reinterpret_cast<const float2*>(Wo)[j];
-        const float2 wc = reinterpret_cast<const float2*>(Wo + 32)[j];
+        const float2 w = reinterpret_cast<const float2*>(Wo + VTACO_DEC_TAIL_WOUT)[j];
+        const float2 wc = reinterpret_cast<const float2*>(Wo + VTACO_DEC_TAIL_WCON)[j];
 #pragma unroll
         for (int s = 0; s < 2; ++s) {
           const float ax = net[s][j].x > 0.f ? net[s][j].x : net[s][j].x * slope;

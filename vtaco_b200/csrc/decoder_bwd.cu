@@ -242,7 +242,7 @@ __global__ void __launch_bounds__(kBT, 1) decoder_bwd_query_kernel(const __grid_
       const float* Wp = sW + (P.use_img ? VTACO_DEC_OFF_WPI : VTACO_DEC_OFF_WP);
 #pragma unroll
       for (int j = 0; j < 32; ++j)
-        n[j] = fmaf(Wp[64 + j], pz, fmaf(Wp[32 + j], py, fmaf(Wp[j], px, Wp[96 + j])));
+        n[j] = fmaf(Wp[64 + j], pz, fmaf(Wp[32 + j], py, fmaf(Wp[j], px, Wp[VTACO_DEC_OFF_BP - VTACO_DEC_OFF_WP + j])));  // = BPI - WPI
       if (P.use_img && P.c_img) {
         const float4* ci = reinterpret_cast<const float4*>(P.c_img) + q * 8;
 #pragma unroll
@@ -258,9 +258,9 @@ __global__ void __launch_bounds__(kBT, 1) decoder_bwd_query_kernel(const __grid_
     for (int i = 0; i < nb; ++i) {
       const float* Wb = sW + VTACO_DEC_OFF_BLOCKS + i * VTACO_DEC_BLOCK_STRIDE;
       if (P.has_c) {
-        mv_fwd(n, Wb, ccol);
+        mv_fwd(n, Wb + VTACO_DEC_BLK_WC, ccol);
 #pragma unroll
-        for (int k = 0; k < 32; ++k) n[k] += Wb[1024 + k];
+        for (int k = 0; k < 32; ++k) n[k] += Wb[VTACO_DEC_BLK_BC + k];
       }
       uint32_t mm = 0, mh = 0;
 #pragma unroll
@@ -271,8 +271,8 @@ __global__ void __launch_bounds__(kBT, 1) decoder_bwd_query_kernel(const __grid_
       }
       store_row(wsq + slot_rm(i) * slot_stride, h);
 #pragma unroll
-      for (int k = 0; k < 32; ++k) h[k] = Wb[1056 + 1024 + k];
-      mv_fwd(h, Wb + 1056, xcol);
+      for (int k = 0; k < 32; ++k) h[k] = Wb[VTACO_DEC_BLK_B0 + k];
+      mv_fwd(h, Wb + VTACO_DEC_BLK_W0, xcol);
 #pragma unroll
       for (int k = 0; k < 32; ++k) {
         mh |= (h[k] > 0.f ? 1u : 0u) << k;
@@ -280,9 +280,9 @@ __global__ void __launch_bounds__(kBT, 1) decoder_bwd_query_kernel(const __grid_
         xcol[k * kBS] = h[k];
       }
       store_row(wsq + slot_rh(nb, i) * slot_stride, h);
-      mv_fwd(n, Wb + 2112, xcol);
+      mv_fwd(n, Wb + VTACO_DEC_BLK_W1, xcol);
 #pragma unroll
-      for (int k = 0; k < 32; ++k) n[k] += Wb[2112 + 1024 + k];
+      for (int k = 0; k < 32; ++k) n[k] += Wb[VTACO_DEC_BLK_B1 + k];
       mcol[(2 * i) * kBT] = mm;
       mcol[(2 * i + 1) * kBT] = mh;
     }
@@ -295,7 +295,7 @@ __global__ void __launch_bounds__(kBT, 1) decoder_bwd_query_kernel(const __grid_
       for (int k = 0; k < 32; ++k) {
         const bool pos = n[k] > 0.f;
         h[k] = pos ? n[k] : n[k] * slope;
-        n[k] = fmaf(dcon, Wo[32 + k], dout * Wo[k]) * (pos ? 1.f : slope);
+        n[k] = fmaf(dcon, Wo[VTACO_DEC_TAIL_WCON + k], dout * Wo[VTACO_DEC_TAIL_WOUT + k]) * (pos ? 1.f : slope);
       }
       store_row(wsq + slot_aout(nb) * slot_stride, h);
       store_row(wsq + slot_gm(nb, nb) * slot_stride, n);
@@ -306,15 +306,15 @@ __global__ void __launch_bounds__(kBT, 1) decoder_bwd_query_kernel(const __grid_
     for (int i = nb - 1; i >= 0; --i) {
       const float* Wb = sW + VTACO_DEC_OFF_BLOCKS + i * VTACO_DEC_BLOCK_STRIDE;
       const uint32_t mm = mcol[(2 * i) * kBT], mh = mcol[(2 * i + 1) * kBT];
-      mv_bwd<false>(xcol, Wb + 2112, n);                 // W1^T g
+      mv_bwd<false>(xcol, Wb + VTACO_DEC_BLK_W1, n);       // W1^T g
 #pragma unroll
       for (int k = 0; k < 32; ++k) h[k] = ((mh >> k) & 1u) ? xcol[k * kBS] : 0.f;
       store_row(wsq + slot_gh(nb, i) * slot_stride, h);
-      mv_bwd<false>(xcol, Wb + 1056, h);                 // W0^T gh
+      mv_bwd<false>(xcol, Wb + VTACO_DEC_BLK_W0, h);       // W0^T gh
 #pragma unroll
       for (int k = 0; k < 32; ++k) n[k] += ((mm >> k) & 1u) ? xcol[k * kBS] : 0.f;
       store_row(wsq + slot_gm(nb, i) * slot_stride, n);
-      if (P.has_c) mv_bwd<true>(dcol, Wb, n);            // dc += Wc^T g
+      if (P.has_c) mv_bwd<true>(dcol, Wb + VTACO_DEC_BLK_WC, n);  // dc += Wc^T g
     }
 
     // ---------------- d c_img = W_img^T g_0 ----------------
@@ -419,12 +419,12 @@ extern "C" int vtaco_decoder_backward(const vtaco_decoder_bwd_args* a, void* str
   }
   for (int i = 0; i < nb; ++i) {
     float* d = dp + VTACO_DEC_OFF_BLOCKS + i * VTACO_DEC_BLOCK_STRIDE;
-    if (has_c) add(slot(slot_gm(nb, i)), 32, 32, slot(kSlotC), 32, 32, d, 32, d + 1024);
-    add(slot(slot_gh(nb, i)), 32, 32, slot(slot_rm(i)), 32, 32, d + 1056, 32, d + 1056 + 1024);
-    add(slot(slot_gm(nb, i + 1)), 32, 32, slot(slot_rh(nb, i)), 32, 32, d + 2112, 32, d + 2112 + 1024);
+    if (has_c) add(slot(slot_gm(nb, i)), 32, 32, slot(kSlotC), 32, 32, d + VTACO_DEC_BLK_WC, 32, d + VTACO_DEC_BLK_BC);
+    add(slot(slot_gh(nb, i)), 32, 32, slot(slot_rm(i)), 32, 32, d + VTACO_DEC_BLK_W0, 32, d + VTACO_DEC_BLK_B0);
+    add(slot(slot_gm(nb, i + 1)), 32, 32, slot(slot_rh(nb, i)), 32, 32, d + VTACO_DEC_BLK_W1, 32, d + VTACO_DEC_BLK_B1);
   }
   float* dt = dp + VTACO_DEC_OFF_BLOCKS + nb * VTACO_DEC_BLOCK_STRIDE;
-  if (a->dlogits) add(a->dlogits, 1, 1, slot(slot_aout(nb)), 32, 32, dt, 32, dt + 64);
-  if (a->dcontact) add(a->dcontact, 1, 1, slot(slot_aout(nb)), 32, 32, dt + 32, 32, dt + 65);
+  if (a->dlogits) add(a->dlogits, 1, 1, slot(slot_aout(nb)), 32, 32, dt + VTACO_DEC_TAIL_WOUT, 32, dt + VTACO_DEC_TAIL_BOUT);
+  if (a->dcontact) add(a->dcontact, 1, 1, slot(slot_aout(nb)), 32, 32, dt + VTACO_DEC_TAIL_WCON, 32, dt + VTACO_DEC_TAIL_BCON);
   return launch_wgrad(W, np, stream);
 }

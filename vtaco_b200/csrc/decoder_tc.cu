@@ -41,7 +41,7 @@ __host__ __device__ inline TcSmem tc_smem_layout(int n_blocks) {
   s.w = 0;                                          // 3*nb matrices x (hi 4 KB | lo 4 KB)
   s.bias = s.w + 3 * n_blocks * 8192;               // (2*nb+1) bias K-blocks of 1 KB
   s.small = s.bias + (2 * n_blocks + 1) * 1024 + 8192;   // (+ fc_p_img.weight[:, 3:] hi|lo) Wp[3][32], bp[32], Wout[64], bout[2]+pad
-  s.tips = s.small + (128 + 68) * 4;
+  s.tips = s.small + (128 + VTACO_DEC_TAIL) * 4;
   s.stage = s.tips + VTACO_MAX_TIPS * 32 * 4;
   s.stage = (s.stage + 15) / 16 * 16;
   s.bars = s.stage + (kTcThreads / 32) * 32 * kStageStride * 4;
@@ -104,7 +104,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) decoder_tc_kernel(const __grid_
   for (int i = tid; i < wtc_floats / 4; i += kTcThreads)
     reinterpret_cast<float4*>(sWtc)[i] = __ldg(reinterpret_cast<const float4*>(wtc) + i);
   for (int i = tid; i < 128; i += kTcThreads) sSmall[i] = P.weights[(P.use_img ? VTACO_DEC_OFF_WPI : VTACO_DEC_OFF_WP) + i];
-  for (int i = tid; i < 68; i += kTcThreads)
+  for (int i = tid; i < VTACO_DEC_TAIL; i += kTcThreads)
     sSmall[128 + i] = P.weights[VTACO_DEC_OFF_BLOCKS + nb * VTACO_DEC_BLOCK_STRIDE + i];
   if (P.n_tips > 0) {
     for (int o = tid; o < P.n_tips * 32; o += kTcThreads) {
@@ -404,15 +404,15 @@ __global__ void __launch_bounds__(kTcThreads, 1) decoder_tc_kernel(const __grid_
     {
       const float* Wo = sSmall + 128;
       const float slope = P.leaky ? 0.2f : 0.0f;
-      float o = Wo[64], oc = Wo[65];
+      float o = Wo[VTACO_DEC_TAIL_BOUT], oc = Wo[VTACO_DEC_TAIL_BCON];
 #pragma unroll
       for (int j = 0; j < 32; ++j) {
         net[j] = net[j] > 0.f ? net[j] : net[j] * slope;
-        o = fmaf(Wo[j], net[j], o);
+        o = fmaf(Wo[VTACO_DEC_TAIL_WOUT + j], net[j], o);
       }
       if (P.contact) {
 #pragma unroll
-        for (int j = 0; j < 32; ++j) oc = fmaf(Wo[32 + j], net[j], oc);
+        for (int j = 0; j < 32; ++j) oc = fmaf(Wo[VTACO_DEC_TAIL_WCON + j], net[j], oc);
       }
       if (valid) {
         store_logit(P, oidx, o);
@@ -483,7 +483,7 @@ __host__ __device__ inline Tc2Smem tc2_smem_layout(int n_blocks) {
   s.w = 0;
   s.bias = s.w + 3 * n_blocks * 8192;
   s.small = s.bias + (2 * n_blocks + 1) * 1024 + 8192;   // bias blocks, then fc_p_img.weight[:, 3:] hi|lo
-  s.tips = s.small + (128 + 68) * 4;
+  s.tips = s.small + (128 + VTACO_DEC_TAIL) * 4;
   s.stage = s.tips + VTACO_MAX_TIPS * 32 * 4;
   s.stage = (s.stage + 15) / 16 * 16;
   s.head = s.stage + (kTc2Threads / 32) * 32 * kTc2Stage * 4;   // per warp: 32 rows x 16 channels
@@ -523,7 +523,7 @@ __global__ void __launch_bounds__(kTc2Threads, 1) decoder_tc2_kernel(const __gri
   for (int i = tid; i < wtc_floats / 4; i += kTc2Threads)
     reinterpret_cast<float4*>(sWtc)[i] = __ldg(reinterpret_cast<const float4*>(wtc) + i);
   for (int i = tid; i < 128; i += kTc2Threads) sSmall[i] = P.weights[(P.use_img ? VTACO_DEC_OFF_WPI : VTACO_DEC_OFF_WP) + i];
-  for (int i = tid; i < 68; i += kTc2Threads)
+  for (int i = tid; i < VTACO_DEC_TAIL; i += kTc2Threads)
     sSmall[128 + i] = P.weights[VTACO_DEC_OFF_BLOCKS + nb * VTACO_DEC_BLOCK_STRIDE + i];
   const bool axis_sm = DENSE && nx <= kTcMaxAxis;
   if (axis_sm)
@@ -819,18 +819,18 @@ __global__ void __launch_bounds__(kTc2Threads, 1) decoder_tc2_kernel(const __gri
 #pragma unroll
       for (int j = 0; j < 16; ++j) {
         net[j] = net[j] > 0.f ? net[j] : net[j] * slope;
-        o = fmaf(Wo[ch0 + j], net[j], o);
+        o = fmaf(Wo[VTACO_DEC_TAIL_WOUT + ch0 + j], net[j], o);
       }
       if (P.contact) {
 #pragma unroll
-        for (int j = 0; j < 16; ++j) oc = fmaf(Wo[32 + ch0 + j], net[j], oc);
+        for (int j = 0; j < 16; ++j) oc = fmaf(Wo[VTACO_DEC_TAIL_WCON + ch0 + j], net[j], oc);
       }
       if (hv == 1) { head[tq] = o; head[128 + tq] = oc; }
       group_sync2();
       if (hv == 0 && valid) {
-        o = (Wo[64] + o) + head[tq];
+        o = (Wo[VTACO_DEC_TAIL_BOUT] + o) + head[tq];
         store_logit(P, oidx, o);
-        if (P.contact) P.contact[oidx] = (Wo[65] + oc) + head[128 + tq];
+        if (P.contact) P.contact[oidx] = (Wo[VTACO_DEC_TAIL_BCON] + oc) + head[128 + tq];
         vmin = fminf(vmin, o);
         vmax = fmaxf(vmax, o);
       }

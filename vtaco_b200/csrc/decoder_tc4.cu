@@ -42,7 +42,7 @@ __host__ __device__ inline Tc4Smem tc4_smem_layout(int n_blocks) {
   s.bias = s.w + (3 * n_blocks + 1) * kT4MatBytes;           // (2*nb+1) fp32 bias vectors
   s.pw = (s.bias + (2 * n_blocks + 1) * 128 + 127) / 128 * 128;   // fc_p | fc_p_img[:, :3] as two K = 8 operand blocks (1 KB each)
   s.small = s.pw + 2048;
-  s.tips = s.small + (128 + 68) * 4;
+  s.tips = s.small + (128 + VTACO_DEC_TAIL) * 4;
   s.stage = s.tips + VTACO_MAX_TIPS * 32 * 4;
   s.stage = (s.stage + 15) / 16 * 16;
   s.head = s.stage + (kT4Threads / 32) * kT4StageRows * 16 * 4;
@@ -189,7 +189,7 @@ __global__ void __launch_bounds__(kT4Threads, 1) decoder_tc4_kernel(const __grid
     if (i >= 96 && P.has_c) v += __ldg(wtc + (3 * nb + 1) * (kT4MatBytes / 4) + (i - 96));
     sSmall[i] = v;
   }
-  for (int i = tid; i < 68; i += kT4Threads)
+  for (int i = tid; i < VTACO_DEC_TAIL; i += kT4Threads)
     sSmall[128 + i] = P.weights[VTACO_DEC_OFF_BLOCKS + nb * VTACO_DEC_BLOCK_STRIDE + i];
   const bool axis_sm = DENSE && nx <= kT4MaxAxis;
   if (axis_sm)
@@ -575,21 +575,22 @@ __global__ void __launch_bounds__(kT4Threads, 1) decoder_tc4_kernel(const __grid
         float2 acc = make_float2(0.f, 0.f);
 #pragma unroll
         for (int j = 0; j < 8; ++j)
-          acc = __ffma2_rn(make_float2(Wo[ch0 + 2 * j], Wo[ch0 + 2 * j + 1]), make_float2(net[2 * j], net[2 * j + 1]), acc);
+          acc = __ffma2_rn(make_float2(Wo[VTACO_DEC_TAIL_WOUT + ch0 + 2 * j], Wo[VTACO_DEC_TAIL_WOUT + ch0 + 2 * j + 1]),
+                           make_float2(net[2 * j], net[2 * j + 1]), acc);
         o = acc.x + acc.y;
       }
       if (P.contact) {
 #pragma unroll
-        for (int j = 0; j < 16; ++j) oc = fmaf(Wo[32 + ch0 + j], net[j], oc);
+        for (int j = 0; j < 16; ++j) oc = fmaf(Wo[VTACO_DEC_TAIL_WCON + ch0 + j], net[j], oc);
       }
       if (hv == 1) { head[tq] = o; head[128 + tq] = oc; }
       group_sync();
       if (hv == 0) {   // warp-uniform
         const bool valid = oidx >= 0;
-        o = (Wo[64] + o) + head[tq];
+        o = (Wo[VTACO_DEC_TAIL_BOUT] + o) + head[tq];
         if (valid) {
           store_logit(P, oidx, o);
-          if (P.contact) P.contact[oidx] = (Wo[65] + oc) + head[128 + tq];
+          if (P.contact) P.contact[oidx] = (Wo[VTACO_DEC_TAIL_BCON] + oc) + head[128 + tq];
         }
         if (P.minmax_key) {   // running min / max as ordered-int keys, one pair per warp in shared memory
           const int key = float_to_key(o);

@@ -29,18 +29,6 @@ constexpr int kET = 128;        // threads per block
 constexpr int kES = kET + 1;    // shared column stride
 constexpr unsigned kFullMask = 0xffffffffu;
 
-// packed encoder weights (hidden_dim = 32, c_dim = 32), K-major
-constexpr int ENC_OFF_WPOS = 0;      // fc_pos.weight^T [3][64]
-constexpr int ENC_OFF_BPOS = 192;    // fc_pos.bias [64]
-constexpr int ENC_OFF_BLOCKS = 256;
-constexpr int ENC_BLOCK_STRIDE = 5184;
-constexpr int ENC_B_W0 = 0;          // fc_0.weight^T [64][32]
-constexpr int ENC_B_B0 = 2048;
-constexpr int ENC_B_W1 = 2080;       // fc_1.weight^T [32][32]
-constexpr int ENC_B_B1 = 3104;
-constexpr int ENC_B_WS = 3136;       // shortcut.weight^T [64][32]
-constexpr int ENC_FCC_FLOATS = 1056; // fc_c.weight^T [32][32] + bias
-
 struct EncParams {
   const float* p;
   long long n, T;
@@ -184,7 +172,7 @@ __device__ __forceinline__ void scatter_rows(const float* __restrict__ sX, int c
 // channel the accumulation order over k is unchanged, so the results are bit-identical to that version.
 constexpr int kEG = 32;          // points per group
 constexpr int kEGS = kEG + 1;    // shared column stride (conflict-free for lane == point and lane == channel)
-constexpr size_t kEncBlockSmem = (ENC_BLOCK_STRIDE + 256 + 96 * kEGS) * sizeof(float);
+constexpr size_t kEncBlockSmem = (VTACO_ENC_BLOCK_STRIDE + VTACO_ENC_OFF_BLOCKS + 96 * kEGS) * sizeof(float);
 
 __device__ __forceinline__ void axpy8(float (&acc)[8], const float* __restrict__ Wk, float x) {
   const float4 w0 = reinterpret_cast<const float4*>(Wk)[0], w1 = reinterpret_cast<const float4*>(Wk)[1];
@@ -235,15 +223,15 @@ __global__ void __launch_bounds__(128) enc_block_kernel(const __grid_constant__ 
                                                         int r_write, int r_init, int net_in, int net_out,
                                                         long long n_groups) {
   extern __shared__ __align__(16) float esm[];
-  float* sW = esm;                          // block weights (5184) [+ fc_pos 256]
-  float* sX = sW + ENC_BLOCK_STRIDE + 256;  // [64][kEGS] inputs, later [32][kEGS] outputs
+  float* sW = esm;                                                // block weights [+ fc_pos]
+  float* sX = sW + VTACO_ENC_BLOCK_STRIDE + VTACO_ENC_OFF_BLOCKS;  // [64][kEGS] inputs, later [32][kEGS] outputs
   float* sH = sX + 64 * kEGS;               // [32][kEGS] hidden activations
-  const float* Wg = P.W + ENC_OFF_BLOCKS + (long long)blk * ENC_BLOCK_STRIDE;
-  for (int i = threadIdx.x; i < ENC_BLOCK_STRIDE / 4; i += 128)
+  const float* Wg = P.W + VTACO_ENC_OFF_BLOCKS + (long long)blk * VTACO_ENC_BLOCK_STRIDE;
+  for (int i = threadIdx.x; i < VTACO_ENC_BLOCK_STRIDE / 4; i += 128)
     reinterpret_cast<float4*>(sW)[i] = __ldg(reinterpret_cast<const float4*>(Wg) + i);
   if (FIRST) {
-    for (int i = threadIdx.x; i < 256 / 4; i += 128)
-      reinterpret_cast<float4*>(sW + ENC_BLOCK_STRIDE)[i] = __ldg(reinterpret_cast<const float4*>(P.W) + i);
+    for (int i = threadIdx.x; i < VTACO_ENC_OFF_BLOCKS / 4; i += 128)
+      reinterpret_cast<float4*>(sW + VTACO_ENC_BLOCK_STRIDE)[i] = __ldg(reinterpret_cast<const float4*>(P.W) + i);
     __syncthreads();   // fc_pos is read right away; otherwise the weight fill overlaps the first input gather
   }
   const int tid = threadIdx.x, lane = tid & 31, q = tid >> 5;
@@ -259,12 +247,12 @@ __global__ void __launch_bounds__(128) enc_block_kernel(const __grid_constant__ 
     for (int k = 0; k < P.nkeys; ++k) myslot[k] = valid ? P.slot[k][n] : 0;
 
     if (FIRST) {   // lane == point: channels [16q, 16q+16) of fc_pos(p)
-      const float* Wp = sW + ENC_BLOCK_STRIDE;
+      const float* Wp = sW + VTACO_ENC_BLOCK_STRIDE;
       const float px = valid ? P.p[n * 3] : 0.f, py = valid ? P.p[n * 3 + 1] : 0.f, pz = valid ? P.p[n * 3 + 2] : 0.f;
 #pragma unroll 8
       for (int jj = 0; jj < 16; ++jj) {
         const int j = 16 * q + jj;
-        sX[j * kEGS + lane] = fmaf(Wp[128 + j], pz, fmaf(Wp[64 + j], py, fmaf(Wp[j], px, Wp[ENC_OFF_BPOS + j])));
+        sX[j * kEGS + lane] = fmaf(Wp[128 + j], pz, fmaf(Wp[64 + j], py, fmaf(Wp[j], px, Wp[VTACO_ENC_OFF_BPOS + j])));
       }
     } else {       // lane == channel: warp q assembles points 8q .. 8q+7, all their global loads in flight together
       const float* netin = P.net[net_in];
@@ -297,18 +285,18 @@ __global__ void __launch_bounds__(128) enc_block_kernel(const __grid_constant__ 
 
     float h[8], o[8];
 #pragma unroll
-    for (int j = 0; j < 8; ++j) { h[j] = sW[ENC_B_B0 + 8 * q + j]; o[j] = sW[ENC_B_B1 + 8 * q + j]; }
+    for (int j = 0; j < 8; ++j) { h[j] = sW[VTACO_ENC_BLK_B0 + 8 * q + j]; o[j] = sW[VTACO_ENC_BLK_B1 + 8 * q + j]; }
 #pragma unroll 4
     for (int k = 0; k < 64; ++k) {
       const float x = sX[k * kEGS + lane];
-      axpy8(h, sW + ENC_B_W0 + k * 32 + 8 * q, fmaxf(x, 0.f));  // fc_0(relu(x))
-      axpy8(o, sW + ENC_B_WS + k * 32 + 8 * q, x);              // shortcut(x), no bias
+      axpy8(h, sW + VTACO_ENC_BLK_W0 + k * 32 + 8 * q, fmaxf(x, 0.f));  // fc_0(relu(x))
+      axpy8(o, sW + VTACO_ENC_BLK_WS + k * 32 + 8 * q, x);              // shortcut(x), no bias
     }
 #pragma unroll
     for (int j = 0; j < 8; ++j) sH[(8 * q + j) * kEGS + lane] = fmaxf(h[j], 0.f);
     __syncthreads();   // hidden activations complete; nobody reads the input columns any more
 #pragma unroll 4
-    for (int k = 0; k < 32; ++k) axpy8(o, sW + ENC_B_W1 + k * 32 + 8 * q, sH[k * kEGS + lane]);  // fc_1(relu(net))
+    for (int k = 0; k < 32; ++k) axpy8(o, sW + VTACO_ENC_BLK_W1 + k * 32 + 8 * q, sH[k * kEGS + lane]);  // fc_1(relu(net))
 #pragma unroll
     for (int j = 0; j < 8; ++j) sX[(8 * q + j) * kEGS + lane] = o[j];
     __syncthreads();
@@ -337,14 +325,14 @@ static unsigned enc_block_grid(long long n_groups) {
 
 // c = fc_c(net) (pointnet.py:162) and the atomicAdd half of scatter_mean (:93,108).  Same shape as the block
 // kernel: four warps per group of 32 points, warp q computes channels [8q, 8q+8).
-constexpr size_t kEncFinalSmem = (ENC_FCC_FLOATS + 64 * kEGS) * sizeof(float);
+constexpr size_t kEncFinalSmem = (VTACO_ENC_TAIL + 64 * kEGS) * sizeof(float);
 __global__ void __launch_bounds__(128) enc_final_kernel(const __grid_constant__ EncParams P, int net_in, long long n_groups) {
   extern __shared__ __align__(16) float esm[];
-  float* sW = esm;                   // fc_c (1056)
-  float* sX = sW + ENC_FCC_FLOATS;   // [32][kEGS] inputs
+  float* sW = esm;                   // fc_c section
+  float* sX = sW + VTACO_ENC_TAIL;   // [32][kEGS] inputs
   float* sO = sX + 32 * kEGS;        // [32][kEGS] outputs
-  const float* Wg = P.W + ENC_OFF_BLOCKS + (long long)P.n_blocks * ENC_BLOCK_STRIDE;
-  for (int i = threadIdx.x; i < ENC_FCC_FLOATS / 4; i += 128)
+  const float* Wg = P.W + VTACO_ENC_OFF_BLOCKS + (long long)P.n_blocks * VTACO_ENC_BLOCK_STRIDE;
+  for (int i = threadIdx.x; i < VTACO_ENC_TAIL / 4; i += 128)
     reinterpret_cast<float4*>(sW)[i] = __ldg(reinterpret_cast<const float4*>(Wg) + i);
   const int tid = threadIdx.x, lane = tid & 31, q = tid >> 5;
   float* dst[4] = {nullptr, nullptr, nullptr, nullptr};
@@ -363,9 +351,9 @@ __global__ void __launch_bounds__(128) enc_final_kernel(const __grid_constant__ 
     __syncthreads();
     float c[8];
 #pragma unroll
-    for (int j = 0; j < 8; ++j) c[j] = sW[1024 + 8 * q + j];
+    for (int j = 0; j < 8; ++j) c[j] = sW[VTACO_ENC_FCC_B + 8 * q + j];
 #pragma unroll 4
-    for (int k = 0; k < 32; ++k) axpy8(c, sW + k * 32 + 8 * q, sX[k * kEGS + lane]);
+    for (int k = 0; k < 32; ++k) axpy8(c, sW + VTACO_ENC_FCC_W + k * 32 + 8 * q, sX[k * kEGS + lane]);
 #pragma unroll
     for (int j = 0; j < 8; ++j) sO[(8 * q + j) * kEGS + lane] = c[j];
     __syncthreads();

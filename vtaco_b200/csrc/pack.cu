@@ -151,7 +151,7 @@ extern "C" int vtaco_decoder_pack_tc(const float* packed, int32_t n_blocks, int3
   const int mat_floats = (mixed == 2) ? 2560 : 2048;
   for (int i = 0; i < nb; ++i) {
     const int o = VTACO_DEC_OFF_BLOCKS + i * VTACO_DEC_BLOCK_STRIDE;
-    const int srcs[3] = {o, o + 1056, o + 2112};   // fc_c[i], fc_0, fc_1
+    const int srcs[3] = {o + VTACO_DEC_BLK_WC, o + VTACO_DEC_BLK_W0, o + VTACO_DEC_BLK_W1};   // fc_c[i], fc_0, fc_1
     for (int j = 0; j < 3; ++j) {
       Pn.mat_src[3 * i + j] = srcs[j];
       Pn.mat_dst[3 * i + j] = (3 * i + j) * mat_floats;
@@ -164,14 +164,14 @@ extern "C" int vtaco_decoder_pack_tc(const float* packed, int32_t n_blocks, int3
   // bias steps: bc_0 | b0_i, b1_i + bc_{i+1}
   Pn.bias_dst = (mixed == 2) ? (3 * nb + 1) * mat_floats : 3 * nb * 2048;
   Pn.n_bias = 2 * nb + 1;
-  Pn.bias_src0[0] = nb > 0 ? VTACO_DEC_OFF_BLOCKS + 1024 : -1;
+  Pn.bias_src0[0] = nb > 0 ? VTACO_DEC_OFF_BLOCKS + VTACO_DEC_BLK_BC : -1;
   Pn.bias_src1[0] = -1;
   for (int i = 0; i < nb; ++i) {
     const int o = VTACO_DEC_OFF_BLOCKS + i * VTACO_DEC_BLOCK_STRIDE;
-    Pn.bias_src0[2 * i + 1] = o + 2080;
+    Pn.bias_src0[2 * i + 1] = o + VTACO_DEC_BLK_B0;
     Pn.bias_src1[2 * i + 1] = -1;
-    Pn.bias_src0[2 * i + 2] = o + 3136;
-    Pn.bias_src1[2 * i + 2] = (i + 1 < nb) ? o + VTACO_DEC_BLOCK_STRIDE + 1024 : -1;
+    Pn.bias_src0[2 * i + 2] = o + VTACO_DEC_BLK_B1;
+    Pn.bias_src1[2 * i + 2] = (i + 1 < nb) ? o + VTACO_DEC_BLOCK_STRIDE + VTACO_DEC_BLK_BC : -1;
   }
   Pn.pw_dst = Pn.bias_dst + (2 * nb + 1) * 32;     // layout 2 only
   pack_tc_kernel<<<Pn.n_mats + Pn.n_bias + (mixed == 2 ? 4 : 0), 256, 0, (cudaStream_t)stream>>>(Pn, packed, dst);

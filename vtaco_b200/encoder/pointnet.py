@@ -22,6 +22,7 @@ import torch
 import torch.nn as nn
 
 from .. import _abi
+from .._abi import EncoderArgs, EncoderBwdArgs
 from ..common import _div_mode
 from ..layers import ResnetBlockFC
 from .unet import UNet
@@ -31,52 +32,13 @@ _KEY_ORDER_IN = ('xz', 'xy', 'yz', 'grid')    # insertion order of coord/index d
 _KEY_ORDER_OUT = ('grid', 'xz', 'xy', 'yz')   # insertion order of the returned dict (pointnet.py:165-172)
 
 
-class EncoderArgs(C.Structure):
-    _fields_ = [
-        ('p', C.c_void_p), ('B', C.c_int32), ('T', C.c_int64),
-        ('padding', C.c_double), ('div_mode', C.c_int32),
-        ('n_keys', C.c_int32), ('kind', C.c_int32 * 4), ('reso', C.c_int32 * 4),
-        ('pool_mean', C.c_int32), ('n_blocks', C.c_int32),
-        ('weights', C.c_void_p), ('workspace', C.c_void_p), ('workspace_bytes', C.c_int64),
-        ('out_cl', C.c_void_p * 4), ('c_out', C.c_void_p), ('index_out', C.c_void_p * 4),
-    ]
-
-
-class EncoderBwdArgs(C.Structure):
-    _fields_ = [
-        ('p', C.c_void_p), ('B', C.c_int32), ('T', C.c_int64),
-        ('padding', C.c_double), ('div_mode', C.c_int32),
-        ('n_keys', C.c_int32), ('kind', C.c_int32 * 4), ('reso', C.c_int32 * 4),
-        ('pool_mean', C.c_int32), ('n_blocks', C.c_int32),
-        ('weights', C.c_void_p), ('workspace', C.c_void_p), ('workspace_bytes', C.c_int64),
-        ('d_out_cl', C.c_void_p * 4), ('d_params', C.c_void_p),
-    ]
-
-
-def _bind(L):
-    if getattr(L, '_enc_bound', False):
-        return
-    L.vtaco_encoder_backward_workspace_bytes.restype = C.c_int64
-    L.vtaco_encoder_backward_workspace_bytes.argtypes = [C.c_int32, C.c_int64, C.c_int32, C.POINTER(C.c_int32),
-                                                         C.POINTER(C.c_int32), C.c_int32]
-    L.vtaco_encoder_backward.argtypes = [C.POINTER(EncoderBwdArgs), C.c_void_p]
-    L.vtaco_encoder_workspace_bytes.restype = C.c_int64
-    L.vtaco_encoder_workspace_bytes.argtypes = [C.c_int32, C.c_int64, C.c_int32, C.POINTER(C.c_int32),
-                                                C.POINTER(C.c_int32)]
-    L.vtaco_encoder_pointnet.argtypes = [C.POINTER(EncoderArgs), C.c_void_p]
-    L.vtaco_pool_workspace_bytes.restype = C.c_int64
-    L.vtaco_pool_workspace_bytes.argtypes = [C.c_int32, C.c_int64, C.c_int32, C.POINTER(C.c_int64)]
-    L.vtaco_pool_local.argtypes = [C.c_void_p, C.c_int32, C.c_int64, C.c_int32, C.POINTER(C.c_void_p),
-                                   C.POINTER(C.c_int64), C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]
-    L.vtaco_scatter_mean.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_int64, C.c_void_p, C.c_int64,
-                                     C.c_void_p, C.c_void_p]
-    L._enc_bound = True
-
-
-def _lib():
-    L = _abi.lib()
-    _bind(L)
-    return L
+# The fields of the packed buffer (include/vtaco_b200.h), as _abi.layout_entries takes them
+_LAYOUT = (_abi.ENC_OFF_BLOCKS, _abi.ENC_BLOCK_STRIDE,
+           [('fc_pos.weight', _abi.ENC_OFF_WPOS), ('fc_pos.bias', _abi.ENC_OFF_BPOS)],
+           [('blocks.%d.fc_0.weight', _abi.ENC_BLK_W0), ('blocks.%d.fc_0.bias', _abi.ENC_BLK_B0),
+            ('blocks.%d.fc_1.weight', _abi.ENC_BLK_W1), ('blocks.%d.fc_1.bias', _abi.ENC_BLK_B1),
+            ('blocks.%d.shortcut.weight', _abi.ENC_BLK_WS)],
+           [('fc_c.weight', _abi.ENC_FCC_W), ('fc_c.bias', _abi.ENC_FCC_B)])
 
 
 class _PointnetFn(torch.autograd.Function):
@@ -196,22 +158,12 @@ class LocalPoolPointnet(nn.Module):
 
     def _packed_weights(self):
         """K-major fp32 buffer (layout in include/vtaco_b200.h), one vtaco_pack_linear launch."""
-        if self._pack_params is None:      # cached: walking the module tree costs more than the check it feeds
-            self._pack_params = tuple([self.fc_pos.weight, self.fc_pos.bias, self.fc_c.weight, self.fc_c.bias] +
-                                      [p for b in self.blocks for p in b.parameters()])
-        params = self._pack_params
-        key = tuple((p.data_ptr(), p._version) for p in params)
+        params = self._params_by_name()
+        key = tuple((p.data_ptr(), p._version) for p in params.values())
         if self._pack_cache is not None and self._pack_cache[0] == key:
             return self._pack_cache[1]
-        nb = self.n_blocks
-        buf = torch.zeros(256 + 5184 * nb + 1056, dtype=torch.float32, device=self.fc_pos.weight.device)
-        ent = [(self.fc_pos.weight, 0), (self.fc_pos.bias, 192)]
-        for i, blk in enumerate(self.blocks):
-            o = 256 + 5184 * i
-            ent += [(blk.fc_0.weight, o), (blk.fc_0.bias, o + 2048), (blk.fc_1.weight, o + 2080),
-                    (blk.fc_1.bias, o + 3104), (blk.shortcut.weight, o + 3136)]
-        o = 256 + 5184 * nb
-        ent += [(self.fc_c.weight, o), (self.fc_c.bias, o + 1024)]
+        buf = torch.zeros(_abi.enc_packed_floats(self.n_blocks), dtype=torch.float32, device=self.fc_pos.weight.device)
+        ent = _abi.layout_entries(_LAYOUT, params, self.n_blocks)
         for j in range(0, len(ent), _abi.PACK_MAX_DESCS):
             _abi.pack_linear(ent[j:j + _abi.PACK_MAX_DESCS], buf,
                              cache=self.__dict__.setdefault('_desc_cache', {}).setdefault(j, {}))
@@ -248,8 +200,15 @@ class LocalPoolPointnet(nn.Module):
     def _pointnet_params(self):
         return [(n, t) for n, t in self.named_parameters() if not n.startswith(('unet.', 'unet3d.'))]
 
+    def _params_by_name(self):
+        """name -> parameter of the PointNet part (cached: walking the module tree costs more than the check it
+        feeds)."""
+        if self._pack_params is None:
+            self._pack_params = dict(self._pointnet_params())
+        return self._pack_params
+
     def _pointnet_impl(self, p, return_code=False, return_index=False):
-        L = _lib()
+        L = _abi.lib()
         B, T = p.shape[0], p.shape[1]
         keys = self._keys_in()
         if not keys:
@@ -306,7 +265,7 @@ class LocalPoolPointnet(nn.Module):
     def _pointnet_backward(self, p, w, grads):
         """vtaco_encoder_backward: `grads` maps key -> gradient of the (B,32,R,R[,R]) feature tensor
         (or None); returns the flat parameter-gradient buffer (native layout, include/vtaco_b200.h)."""
-        L = _lib()
+        L = _abi.lib()
         B, T = p.shape[0], p.shape[1]
         dev = p.device
         keys = self._keys_in()
@@ -326,7 +285,7 @@ class LocalPoolPointnet(nn.Module):
         a.pool_mean = int(self.scatter_type == 'mean')
         a.n_blocks = self.n_blocks
         a.weights = w.data_ptr()
-        flat = torch.zeros(256 + 5184 * self.n_blocks + 1056, dtype=torch.float32, device=dev)
+        flat = torch.zeros(_abi.enc_packed_floats(self.n_blocks), dtype=torch.float32, device=dev)
         a.d_params = flat.data_ptr()
         nbytes = L.vtaco_encoder_backward_workspace_bytes(B, T, a.n_keys, a.kind, a.reso, self.n_blocks)
         if nbytes < 0:
@@ -339,18 +298,8 @@ class LocalPoolPointnet(nn.Module):
         return flat
 
     def _unpack_param_grads(self, flat):
-        g = {'fc_pos.weight': flat[0:192].view(64, 3), 'fc_pos.bias': flat[192:256]}
-        for i in range(self.n_blocks):
-            o = 256 + 5184 * i
-            g['blocks.%d.fc_0.weight' % i] = flat[o:o + 2048].view(32, 64)
-            g['blocks.%d.fc_0.bias' % i] = flat[o + 2048:o + 2080]
-            g['blocks.%d.fc_1.weight' % i] = flat[o + 2080:o + 3104].view(32, 32)
-            g['blocks.%d.fc_1.bias' % i] = flat[o + 3104:o + 3136]
-            g['blocks.%d.shortcut.weight' % i] = flat[o + 3136:o + 5184].view(32, 64)
-        o = 256 + 5184 * self.n_blocks
-        g['fc_c.weight'] = flat[o:o + 1024].view(32, 32)
-        g['fc_c.bias'] = flat[o + 1024:o + 1056]
-        return g
+        """name -> gradient of every parameter of the PointNet part, from the buffer vtaco_encoder_backward wrote."""
+        return _abi.layout_grads(_LAYOUT, self._params_by_name(), flat, self.n_blocks)
 
     # ------------------------------------------------------------------ reference API
     def forward(self, p):
@@ -374,7 +323,7 @@ class LocalPoolPointnet(nn.Module):
         c (B,T,32) -> (B,T,32).  (`xy` is only used for its keys, as in the reference.)"""
         _abi.require_cuda(c, 'c')
         _abi.forbid_autograd(c)
-        L = _lib()
+        L = _abi.lib()
         B, T, Cc = c.shape
         if Cc != 32:
             raise NotImplementedError('pool_local kernel implements 32 channels')
@@ -398,7 +347,7 @@ class LocalPoolPointnet(nn.Module):
         from ..common import point_to_cell
         _abi.require_cuda(c, 'c')
         _abi.forbid_autograd(p, c)
-        L = _lib()
+        L = _abi.lib()
         B, T = p.shape[0], p.shape[1]
         R = self._reso(key)
         idx = point_to_cell(p, R, key, self.padding, self.division, index_dtype=torch.int32).reshape(-1)

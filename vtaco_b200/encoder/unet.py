@@ -16,6 +16,8 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
+from .unet3d import _pack_conv_weight
+
 
 class _Down(nn.Module):
     def __init__(self, cin, cout, pooling):
@@ -46,15 +48,6 @@ class _Up(nn.Module):
         x = self.upconv(x)
         x = torch.cat((x, skip), 1) if self.merge_mode == 'concat' else x + skip
         return F.relu(self.conv2(F.relu(self.conv1(x))))
-
-
-def _pack_w(w5):
-    """(Cout, Cin, k, k, k) -> the operand layout of vtaco_conv3d_cl, rounded to nearest TF32 (as unet3d._pack_conv_weight)."""
-    Cout, Cin = w5.shape[0], w5.shape[1]
-    taps = w5.shape[2] * w5.shape[3] * w5.shape[4]
-    wt = w5.detach().float().reshape(Cout // 32, 32, Cin // 16, 4, 4, taps).permute(0, 2, 5, 3, 1, 4).contiguous()
-    wt = ((wt.view(torch.int32) + 0x1000) & ~0x1fff).view(torch.float32)
-    return wt.reshape(-1)
 
 
 class UNet(nn.Module):
@@ -124,7 +117,7 @@ class UNet(nn.Module):
             else:                      # ConvTranspose2d (Cin, Cout, 2, 2) -> 1x1 conv to (a*2+b)*Cout + co
                 w5 = w.permute(2, 3, 1, 0).reshape(4 * w.shape[1], w.shape[0], 1, 1, 1)
                 b = conv.bias.detach().float().repeat(4).contiguous()
-            hit = (ver, _pack_w(w5.contiguous()), b)
+            hit = (ver, _pack_conv_weight(w5), b)
             cache[key] = hit
         return hit[1], hit[2]
 

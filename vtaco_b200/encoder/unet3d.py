@@ -129,10 +129,10 @@ class _Decoder(nn.Module):
 
 
 def _pack_conv_weight(w):
-    """(Cout, Cin, k, k, k) -> the tcgen05 operand layout of vtaco_conv3d_cl (include/vtaco_b200.h),
+    """(Cout, Cin, kD, kH, kW) -> the tcgen05 operand layout of vtaco_conv3d_cl (include/vtaco_b200.h),
     values rounded to nearest TF32."""
-    Cout, Cin, k = w.shape[0], w.shape[1], w.shape[2]
-    taps = k ** 3
+    Cout, Cin = w.shape[0], w.shape[1]
+    taps = w.shape[2] * w.shape[3] * w.shape[4]
     wt = w.detach().float().reshape(Cout // 32, 32, Cin // 16, 4, 4, taps)       # [nt][n][ch][kc][kk][tap]
     wt = wt.permute(0, 2, 5, 3, 1, 4).contiguous()                               # [nt][ch][tap][kc][n][kk]
     wt = ((wt.view(torch.int32) + 0x1000) & ~0x1fff).view(torch.float32)
