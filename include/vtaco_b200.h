@@ -110,8 +110,45 @@ int vtaco_relayout_cf(const float* src, float* dst, int B, int C, int64_t S, voi
 #define VTACO_DEC_PACKED_FLOATS(n_blocks) (VTACO_DEC_OFF_BLOCKS + VTACO_DEC_BLOCK_STRIDE * (n_blocks) + VTACO_DEC_TAIL)
 #define VTACO_MAX_TIPS 8
 #define VTACO_MAX_BLOCKS 8   /* n_blocks the shared-memory-resident kernels can hold */
-/* floats of the tcgen05 operand buffer `weights_tc` (layouts below; sized for the largest, variant 7's) */
-#define VTACO_DEC_TC_FLOATS(n_blocks) ((3 * (n_blocks) + 1) * 2560 + (2 * (n_blocks) + 1) * 256 + 1024)
+
+/* tcgen05 operand buffer `weights_tc` (fp32, device), built from `weights` by vtaco_decoder_pack_tc in one of
+ * three pack modes.  Offsets in floats.  A K-block is a 32 (n = out) x 8 (k = in) operand slice in the UMMA
+ * canonical K-major no-swizzle layout: float index of (n, k) = (k/4)*128 + (n/8)*32 + (n%8)*4 + (k%4).
+ * A matrix holds one 32x32 weight: sub-block hi = rn_tf32(W) (4 K-blocks, the same index formula with k in
+ * [0,32)), then lo = tf32(W - hi) (modes 0, 2) or, mode 1, the K = 64 BF16 correction operand
+ * [bf16(W) ; bf16(W - hi)] with bf16 index of (n, k) = (k/8)*256 + (n/8)*64 + (n%8)*8 + (k%8); mode 2 adds
+ * bf16(W) (K = 32, same bf16 index) and stores fc_0 / fc_1 times 0.5 (the kernel feeds them 2*relu(x) = x + |x|).
+ * A bias step is a K-block with row k=0 = bias hi, k=1 = bias lo, other rows 0 (modes 0, 1), or the plain fp32
+ * vector (mode 2).  Mode 2's input-layer K-blocks q = 0, 1 (fc_p) and 2, 3 (fc_p_img[:, :3]) are B1 = rows
+ * (W_hi[:,0..2], (b + bc_0)_hi, W_hi[:,0..2], 0) and B2 = rows (W_lo[:,0..2], (b + bc_0)_lo, 0, 0, 0, 0), the
+ * B operands of A = (px, py, pz, 1, px_lo, py_lo, pz_lo, 0). */
+#define VTACO_DEC_TC_MODE_3XTF32 0   /* TF32 hi | TF32 lo: variants 2, 3, 5 */
+#define VTACO_DEC_TC_MODE_BF16 1     /* TF32 hi | K = 64 BF16 correction: variants 4, 6 */
+#define VTACO_DEC_TC_MODE_TILE4 2    /* TF32 hi | TF32 lo | bf16(W), fp32 bias vectors, K-block input layer: variant 7 */
+#define VTACO_DEC_TC_MODE(variant) ((variant) == 7 ? 2 : ((variant) == 4 || (variant) == 6) ? 1 : 0)
+#define VTACO_DEC_TC_KBLK_FLOATS 256
+#define VTACO_DEC_TC_BVEC_FLOATS 32  /* a mode-2 bias step */
+#define VTACO_DEC_TC_SUB_HI 0        /* sub-blocks of a matrix */
+#define VTACO_DEC_TC_SUB_LO 1024
+#define VTACO_DEC_TC_SUB_BF16 2048   /* mode 2 only */
+#define VTACO_DEC_TC_MAT_FLOATS(mode) ((mode) == 2 ? 2560 : 2048)
+/* matrix m = 3*i + {0, 1, 2}: fc_c[i].weight, blocks[i].fc_0.weight, blocks[i].fc_1.weight; in mode 2 also
+ * m = 3*n_blocks: fc_p_img.weight[:, 3:] */
+#define VTACO_DEC_TC_MAT(mode, m) ((m) * VTACO_DEC_TC_MAT_FLOATS(mode))
+/* bias step s = 0 .. 2*n_blocks: bc_0 | b0_i, b1_i + bc_{i+1} (i = 0..n_blocks-1); after the matrices */
+#define VTACO_DEC_TC_BIAS_STEP_FLOATS(mode) ((mode) == 2 ? VTACO_DEC_TC_BVEC_FLOATS : VTACO_DEC_TC_KBLK_FLOATS)
+#define VTACO_DEC_TC_BIAS(mode, n_blocks, s) \
+  (VTACO_DEC_TC_MAT(mode, 3 * (n_blocks) + ((mode) == 2)) + (s) * VTACO_DEC_TC_BIAS_STEP_FLOATS(mode))
+/* fc_p_img.weight[:, 3:] (the product with a per-query c_img tensor): after the bias steps in modes 0 and 1 */
+#define VTACO_DEC_TC_WIMG(mode, n_blocks) \
+  ((mode) == 2 ? VTACO_DEC_TC_MAT(mode, 3 * (n_blocks)) : VTACO_DEC_TC_BIAS(mode, n_blocks, 2 * (n_blocks) + 1))
+/* mode 2: input-layer K-block q = 0..3 */
+#define VTACO_DEC_TC_INPUT(n_blocks, q) (VTACO_DEC_TC_BIAS(2, n_blocks, 2 * (n_blocks) + 1) + (q) * VTACO_DEC_TC_KBLK_FLOATS)
+#define VTACO_DEC_TC_USED_FLOATS(mode, n_blocks) \
+  ((mode) == 2 ? VTACO_DEC_TC_INPUT(n_blocks, 4) : VTACO_DEC_TC_WIMG(mode, n_blocks) + VTACO_DEC_TC_MAT_FLOATS(mode))
+/* floats reserved for `weights_tc` in any mode: the widest matrices, a K-block per bias step, mode 2's input layer */
+#define VTACO_DEC_TC_FLOATS(n_blocks) \
+  ((3 * (n_blocks) + 1) * VTACO_DEC_TC_MAT_FLOATS(2) + (2 * (n_blocks) + 1 + 4) * VTACO_DEC_TC_KBLK_FLOATS)
 
 typedef struct vtaco_decoder_args {
   /* ---- queries ---- */
@@ -154,26 +191,8 @@ typedef struct vtaco_decoder_args {
                             * 5 / 6 = 2 / 4 with two threads per query (768-thread CTAs, 3 tiles per SM);
                             * 7 = four tiles per SM (1024-thread CTAs): TF32 hi products + BF16 residual product, biases
                             *     on the CUDA cores (fastest; needs fewer than 2^31 outputs per call, else 5 is used) */
-  /* variants 2-6: the 3*n_blocks hidden matrices (per block: fc_c[i], fc_0, fc_1) as TF32 hi / lo
-   * pairs in the UMMA canonical K-major no-swizzle layout, 2048 floats per matrix:
-   *   float index of element (n = out, k = in) = (k/4)*128 + (n/8)*32 + (n%8)*4 + (k%4),
-   *   hi block (1024 floats) = rn_tf32(W), lo block (1024 floats) = tf32(W - hi);
-   *   variants 4 and 6: the lo block instead holds 2048 BF16 values, the K = 64 correction operand
-   *   [bf16(W) ; bf16(W - hi)], bf16 index of (n, k) = (k/8)*256 + (n/8)*64 + (n%8)*8 + (k%8);
-   * followed by 2*n_blocks+1 bias K-blocks of 256 floats in the same layout with k in [0,8): row k=0
-   * = bias hi, k=1 = bias lo, for the steps bc_0 | b0_i, b1_i + bc_{i+1} (i = 0..n_blocks-1);
-   * followed by one more 2048-float matrix block in the matrix layout: fc_p_img.weight[:, 3:]
-   * (the product with a per-query c_img tensor, decoder.py:83-85).
-   *   variant 7 (pack mode 2): fc_0 / fc_1 are stored times 0.5 (the kernel feeds them 2*relu(x) = x + |x|);
-   *   2560 floats per matrix — hi block, lo block as above, then 1024 BF16
-   *   values bf16(W) with bf16 index (k/8)*256 + (n/8)*64 + (n%8)*8 + (k%8); the 3*n_blocks matrices are
-   *   followed by the fc_p_img.weight[:, 3:] block (same 2560-float layout) and then by 2*n_blocks+1
-   *   plain fp32 bias vectors [32] for the same steps, and by four K = 8 blocks of 256 floats (K-block layout
-   *   above) that put the 3-wide input layer on the tensor core as well: for fc_p, then for
-   *   fc_p_img[:, :3], B1 = rows (W_hi[:,0..2], (b + bc_0)_hi, W_hi[:,0..2], 0) and B2 = rows
-   *   (W_lo[:,0..2], (b + bc_0)_lo, 0, 0, 0, 0), multiplied by A = (px, py, pz, 1, px_lo, py_lo, pz_lo, 0).
-   * VTACO_DEC_TC_FLOATS floats are reserved for any layout; vtaco_decoder_pack_tc builds the buffer
-   * from `weights` (it writes every float its layout uses). */
+  /* variants 2-7: VTACO_DEC_TC_FLOATS(n_blocks) floats in pack mode VTACO_DEC_TC_MODE(variant) (layout
+   * VTACO_DEC_TC_*, above), built by vtaco_decoder_pack_tc */
   const float* weights_tc;
   /* dense mode, multi-GPU: when n_peers > 0 every logit of the slab is stored to
    * logits_peers[0..n_peers) instead of `logits` — the (nx,nx,nx) grids of all ranks (own one
@@ -260,8 +279,8 @@ int vtaco_tactile_point_map(const float* p, int64_t n, const float* axis, int32_
  * (bias vectors: in_dim = 1).  At most VTACO_PACK_MAX_DESCS descriptors per call; `dst` must be
  * zero-initialised where no descriptor writes (padding, absent fc_c when c_dim = 0).
  * vtaco_decoder_pack_tc derives the tcgen05 operand buffer (`weights_tc`, VTACO_DEC_TC_FLOATS
- * floats) from the packed decoder buffer; mixed = 0 for variants 2 / 3 / 5, 1 for variants 4 / 6,
- * 2 for variant 7.
+ * floats) from the packed decoder buffer; `mixed` is the pack mode, VTACO_DEC_TC_MODE(variant).  It writes
+ * every float of the mode's VTACO_DEC_TC_USED_FLOATS.
  * ------------------------------------------------------------------------- */
 #define VTACO_PACK_MAX_DESCS 64
 typedef struct vtaco_pack_desc {

@@ -4,7 +4,9 @@ Both models read their weights from one flat fp32 buffer and their backward kern
 gradients into a flat buffer with the same offsets.  The expected offsets below are written out from the
 layouts include/vtaco_b200.h documents, independently of the constants the package derives them from: the
 header macros must equal their Python mirror, the pack descriptors the modules hand to vtaco_pack_linear must
-land each parameter where the header says, and the gradient views must be cut from the same places."""
+land each parameter where the header says, and the gradient views must be cut from the same places.  The same
+goes for the tcgen05 operand buffer the decoder derives from its packed buffer (`weights_tc`)."""
+import itertools
 import os
 import re
 import shutil
@@ -92,30 +94,95 @@ def _check_views(grads, fields, flat):
 
 
 # ---------------------------------------------------------------------------------------------------------------
+# arguments every function-like layout macro is evaluated at: pack modes 0-2, 0-8 blocks, every decoder variant,
+# every matrix index m (3*n_blocks + 1 of them), bias step s (2*n_blocks + 1) and input-layer K-block q (4, + the end)
+MACRO_ARGS = {'n_blocks': range(9), 'mode': range(3), 'variant': range(8), 'm': range(3 * 8 + 1), 's': range(2 * 8 + 1),
+              'q': range(5)}
+
+
 def test_layout_macros_match_the_python_mirror(tmp_path):
     """Every VTACO_DEC_* / VTACO_ENC_* layout and size macro of the header, as a C compiler evaluates it, equals
-    its mirror in vtaco_b200._abi (VTACO_X -> _abi.X; VTACO_X(n_blocks) -> _abi.x(n_blocks) for 0..8 blocks)."""
+    its mirror in vtaco_b200._abi (VTACO_X -> _abi.X; VTACO_X(args) -> _abi.x(args) at every combination of
+    MACRO_ARGS)."""
     if shutil.which('gcc') is None:
         pytest.skip('no C compiler')
     hdr = open(os.path.join(ROOT, 'include', 'vtaco_b200.h')).read()
     consts = re.findall(r'^#define (VTACO_(?:DEC|ENC)_[A-Z0-9_]+)[ \t]', hdr, flags=re.M)
-    funcs = re.findall(r'^#define (VTACO_(?:DEC|ENC)_[A-Z0-9_]+)\(n_blocks\)', hdr, flags=re.M)
+    funcs = {m: tuple(a.strip() for a in args.split(','))
+             for m, args in re.findall(r'^#define (VTACO_(?:DEC|ENC)_[A-Z0-9_]+)\(([^)]*)\)', hdr, flags=re.M)}
     assert {'VTACO_DEC_BLK_W1', 'VTACO_DEC_TAIL_BCON', 'VTACO_ENC_BLK_WS', 'VTACO_ENC_FCC_B'} <= set(consts)
     assert {'VTACO_DEC_PACKED_FLOATS', 'VTACO_ENC_PACKED_FLOATS'} <= set(funcs)
+    assert {'VTACO_DEC_TC_SUB_BF16', 'VTACO_DEC_TC_KBLK_FLOATS', 'VTACO_DEC_TC_MODE_TILE4'} <= set(consts)
+    assert {'VTACO_DEC_TC_MODE', 'VTACO_DEC_TC_MAT', 'VTACO_DEC_TC_BIAS', 'VTACO_DEC_TC_WIMG', 'VTACO_DEC_TC_INPUT',
+            'VTACO_DEC_TC_USED_FLOATS', 'VTACO_DEC_TC_FLOATS'} <= set(funcs)
+    calls = [(m, args) for m, names in funcs.items() for args in itertools.product(*(MACRO_ARGS[n] for n in names))]
     lines = ['#include <stdio.h>', '#include "vtaco_b200.h"', 'int main(void) {']
-    lines += ['  printf("%s -1 %%ld\\n", (long)(%s));' % (m, m) for m in consts]
-    lines += ['  printf("%s %d %%ld\\n", (long)(%s(%d)));' % (m, nb, m, nb) for m in funcs for nb in range(9)]
+    lines += ['  printf("%s %%ld\\n", (long)(%s));' % (m, m) for m in consts]
+    lines += ['  printf("%s %%ld\\n", (long)(%s(%s)));' % (m, m, ', '.join(map(str, a))) for m, a in calls]
     lines += ['  return 0;', '}']
     src = tmp_path / 'layout.c'
     src.write_text('\n'.join(lines))
     exe = str(tmp_path / 'layout')
     subprocess.run(['gcc', '-std=c99', '-I', os.path.join(ROOT, 'include'), str(src), '-o', exe], check=True)
-    out = subprocess.run([exe], check=True, capture_output=True, text=True).stdout.split()
-    assert len(out) == 3 * (len(consts) + 9 * len(funcs))
-    for macro, nb, val in zip(out[0::3], out[1::3], out[2::3]):
-        name, nb = macro[len('VTACO_'):], int(nb)
-        want = getattr(_abi, name) if nb < 0 else getattr(_abi, name.lower())(nb)
-        assert int(val) == want, (macro, nb, int(val), want)
+    out = subprocess.run([exe], check=True, capture_output=True, text=True).stdout.split('\n')[:-1]
+    assert len(out) == len(consts) + len(calls)
+    for line, (macro, args) in zip(out, [(m, None) for m in consts] + calls):
+        name, val = line.split()
+        assert name == macro
+        name = macro[len('VTACO_'):]
+        want = getattr(_abi, name) if args is None else getattr(_abi, name.lower())(*args)
+        assert int(val) == want, (macro, args, int(val), want)
+
+
+# weights_tc section offsets as vtaco_decoder_pack_tc placed them before they were named, per pack mode:
+# n_blocks -> (floats per matrix, W_img block, first bias step, floats per bias step, first input-layer K-block or
+# None, floats used); and the floats reserved, VTACO_DEC_TC_FLOATS
+TC_LAYOUT = {
+    0: {1: (2048, 6912, 6144, 256, None, 8960), 3: (2048, 20224, 18432, 256, None, 22272),
+        5: (2048, 33536, 30720, 256, None, 35584)},
+    2: {1: (2560, 7680, 10240, 32, 10336, 11360), 3: (2560, 23040, 25600, 32, 25824, 26848),
+        5: (2560, 38400, 40960, 32, 41312, 42336)},
+}
+TC_LAYOUT[1] = TC_LAYOUT[0]     # mode 1 differs from mode 0 only inside a matrix's lo sub-block
+TC_FLOATS = {1: 12032, 3: 28416, 5: 44800}
+
+
+@pytest.mark.parametrize('nb', N_BLOCKS)
+@pytest.mark.parametrize('mode', (0, 1, 2))
+def test_tc_section_offsets_match_the_documented_layout(mode, nb):
+    mat, wimg, bias0, step, input0, used = TC_LAYOUT[mode][nb]
+    assert [_abi.dec_tc_mat(mode, m) for m in range(3 * nb)] == [m * mat for m in range(3 * nb)]
+    assert _abi.dec_tc_mat_floats(mode) == mat
+    assert _abi.dec_tc_wimg(mode, nb) == wimg
+    if mode == 2:
+        assert _abi.dec_tc_mat(mode, 3 * nb) == wimg
+        assert [_abi.dec_tc_input(nb, q) for q in range(4)] == [input0 + 256 * q for q in range(4)]
+    assert [_abi.dec_tc_bias(mode, nb, s) for s in range(2 * nb + 1)] == [bias0 + step * s for s in range(2 * nb + 1)]
+    assert _abi.dec_tc_used_floats(mode, nb) == used
+    assert _abi.dec_tc_floats(nb) == TC_FLOATS[nb]
+
+
+@pytest.mark.parametrize('mode', (0, 1, 2))
+def test_tc_sections_tile_the_used_floats(mode):
+    """For 0-8 blocks the matrices, the W_img block, the bias steps and (mode 2) the input-layer K-blocks do not
+    overlap, leave no gap (vtaco_decoder_pack_tc writes every float in front of VTACO_DEC_TC_USED_FLOATS) and fit
+    the VTACO_DEC_TC_FLOATS reserved for the buffer; the sub-blocks fit their matrix."""
+    mat = _abi.dec_tc_mat_floats(mode)
+    subs = [(_abi.DEC_TC_SUB_HI, 1024), (_abi.DEC_TC_SUB_LO, 1024)] + ([(_abi.DEC_TC_SUB_BF16, 512)] if mode == 2 else [])
+    assert sorted(subs) == subs and all(a + n == b for (a, n), (b, _) in zip(subs, subs[1:] + [(mat, 0)]))
+    for nb in range(9):
+        sec = [(_abi.dec_tc_mat(mode, m), mat) for m in range(3 * nb)] + [(_abi.dec_tc_wimg(mode, nb), mat)]
+        sec += [(_abi.dec_tc_bias(mode, nb, s), _abi.dec_tc_bias_step_floats(mode)) for s in range(2 * nb + 1)]
+        if mode == 2:
+            sec += [(_abi.dec_tc_input(nb, q), _abi.DEC_TC_KBLK_FLOATS) for q in range(4)]
+        sec.sort()
+        assert sec[0][0] == 0, nb
+        assert all(a + n == b for (a, n), (b, _) in zip(sec, sec[1:])), nb
+        assert sec[-1][0] + sec[-1][1] == _abi.dec_tc_used_floats(mode, nb) <= _abi.dec_tc_floats(nb), nb
+
+
+def test_tc_pack_mode_of_each_variant():
+    assert {v: _abi.dec_tc_mode(v) for v in range(2, 8)} == {2: 0, 3: 0, 4: 1, 5: 0, 6: 1, 7: 2}
 
 
 @pytest.mark.parametrize('nb', N_BLOCKS)

@@ -136,9 +136,47 @@ class PackDesc(C.Structure):
 PACK_MAX_DESCS = 64
 
 
+# tcgen05 operand buffer `weights_tc` (VTACO_DEC_TC_* of include/vtaco_b200.h): pack modes, sizes and offsets
+DEC_TC_MODE_3XTF32, DEC_TC_MODE_BF16, DEC_TC_MODE_TILE4 = 0, 1, 2
+DEC_TC_KBLK_FLOATS, DEC_TC_BVEC_FLOATS = 256, 32
+DEC_TC_SUB_HI, DEC_TC_SUB_LO, DEC_TC_SUB_BF16 = 0, 1024, 2048
+
+
+def dec_tc_mode(variant):
+    return 2 if variant == 7 else 1 if variant in (4, 6) else 0
+
+
+def dec_tc_mat_floats(mode):
+    return 2560 if mode == 2 else 2048
+
+
+def dec_tc_mat(mode, m):
+    return m * dec_tc_mat_floats(mode)
+
+
+def dec_tc_bias_step_floats(mode):
+    return DEC_TC_BVEC_FLOATS if mode == 2 else DEC_TC_KBLK_FLOATS
+
+
+def dec_tc_bias(mode, n_blocks, s):
+    return dec_tc_mat(mode, 3 * n_blocks + int(mode == 2)) + s * dec_tc_bias_step_floats(mode)
+
+
+def dec_tc_wimg(mode, n_blocks):
+    return dec_tc_mat(mode, 3 * n_blocks) if mode == 2 else dec_tc_bias(mode, n_blocks, 2 * n_blocks + 1)
+
+
+def dec_tc_input(n_blocks, q):
+    return dec_tc_bias(2, n_blocks, 2 * n_blocks + 1) + q * DEC_TC_KBLK_FLOATS
+
+
+def dec_tc_used_floats(mode, n_blocks):
+    return dec_tc_input(n_blocks, 4) if mode == 2 else dec_tc_wimg(mode, n_blocks) + dec_tc_mat_floats(mode)
+
+
 def dec_tc_floats(n_blocks):
-    """VTACO_DEC_TC_FLOATS: floats reserved for any tcgen05 operand layout (variant 7's is the largest)."""
-    return (3 * n_blocks + 1) * 2560 + (2 * n_blocks + 1) * 256 + 1024
+    """VTACO_DEC_TC_FLOATS: floats reserved for `weights_tc` in any pack mode."""
+    return (3 * n_blocks + 1) * dec_tc_mat_floats(2) + (2 * n_blocks + 1 + 4) * DEC_TC_KBLK_FLOATS
 
 
 def pack_linear(entries, dst, cache=None):

@@ -218,11 +218,8 @@ class LocalDecoder(nn.Module):
         return buf
 
     def _packed_weights_tc(self, mixed=False):
-        """The 3*n_blocks hidden matrices (+ fc_p_img.weight[:, 3:]) in the UMMA canonical K-major
-        layout expected by the tcgen05 kernels (include/vtaco_b200.h, `weights_tc`): per matrix 4 KB
-        of TF32 hi followed by 4 KB of either TF32 lo (3xTF32; mixed = 0) or — mixed = 1, variants
-        4 / 6 — the BF16 correction operand with K = 64; then the bias K-blocks.  mixed = 2
-        (variant 7): hi, lo and a 2 KB bf16(W) block per matrix, biases as fp32 vectors.  One launch
+        """The tcgen05 operand buffer `weights_tc` in pack mode `mixed` (False / True / 2 = modes 0 / 1 / 2; the
+        layout is VTACO_DEC_TC_* in include/vtaco_b200.h, mirrored by _abi.dec_tc_*).  One launch
         (vtaco_decoder_pack_tc) from the packed fp32 buffer."""
         w = self._packed_weights()
         if self._pack_tc_cache is None:
@@ -305,7 +302,7 @@ class LocalDecoder(nn.Module):
             a.variant = 5      # the four-tile kernel indexes its outputs with 32 bits
         keep = [cl, w]
         if a.variant in (2, 3, 4, 5, 6, 7):
-            wtc = self._packed_weights_tc(mixed=2 if a.variant == 7 else int(a.variant in (4, 6)))
+            wtc = self._packed_weights_tc(mixed=_abi.dec_tc_mode(a.variant))
             a.weights_tc = wtc.data_ptr()
             keep.append(wtc)
         return a, keep

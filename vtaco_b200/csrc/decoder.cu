@@ -483,7 +483,7 @@ extern "C" int vtaco_decoder_forward(const vtaco_decoder_args* a, void* stream) 
     }
     P.mcast = a->logits_multicast;
   }
-  P.tc_products = (a->variant == 3) ? 1 : (a->variant == 4 || a->variant == 6) ? 2 : 3;
+  P.tc_products = (a->variant == 3) ? 1 : (VTACO_DEC_TC_MODE(a->variant) == VTACO_DEC_TC_MODE_BF16) ? 2 : 3;
   P.tc_split = (a->variant == 5 || a->variant == 6) ? 2 : 1;
   if (a->variant == 7) return launch_decoder_tc4(P, dense, a->weights_tc, st);
   if (a->variant >= 2 && a->variant <= 6) return launch_decoder_tc(P, dense, a->weights_tc, st);

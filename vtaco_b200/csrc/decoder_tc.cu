@@ -32,15 +32,26 @@
 namespace vtaco {
 
 
+// weights_tc is copied to shared memory as it is.  Pack modes 0 and 1 place every block alike (they differ only
+// inside a matrix's lo sub-block), so the offsets are mode 0's; byte sizes of the pieces an MMA reads:
+constexpr int kTcMode = VTACO_DEC_TC_MODE_3XTF32;
+constexpr int kMatBytes = 4 * VTACO_DEC_TC_MAT_FLOATS(kTcMode);
+constexpr int kKBlkBytes = 4 * VTACO_DEC_TC_KBLK_FLOATS;   // a K = 8 TF32 block (also a bias step), or a K = 16 BF16 block
+constexpr int kLoBytes = 4 * VTACO_DEC_TC_SUB_LO;
+// the layouts below and wimg_sm find fc_p_img.weight[:, 3:] right after the 2*nb+1 bias K-blocks
+static_assert(VTACO_DEC_TC_WIMG(kTcMode, VTACO_MAX_BLOCKS) ==
+                  VTACO_DEC_TC_BIAS(kTcMode, VTACO_MAX_BLOCKS, 0) + (2 * VTACO_MAX_BLOCKS + 1) * VTACO_DEC_TC_KBLK_FLOATS,
+              "W_img block must follow the bias K-blocks");
+
 struct TcSmem {
   // byte offsets into dynamic shared memory
   int w, bias, small, tips, stage, bars, tmem_ptr, total;
 };
 __host__ __device__ inline TcSmem tc_smem_layout(int n_blocks) {
   TcSmem s;
-  s.w = 0;                                          // 3*nb matrices x (hi 4 KB | lo 4 KB)
-  s.bias = s.w + 3 * n_blocks * 8192;               // (2*nb+1) bias K-blocks of 1 KB
-  s.small = s.bias + (2 * n_blocks + 1) * 1024 + 8192;   // (+ fc_p_img.weight[:, 3:] hi|lo) Wp[3][32], bp[32], Wout[64], bout[2]+pad
+  s.w = 0;                                                      // weights_tc: 3*nb matrices,
+  s.bias = s.w + 4 * VTACO_DEC_TC_BIAS(kTcMode, n_blocks, 0);   // the bias K-blocks, then fc_p_img.weight[:, 3:]
+  s.small = s.bias + (2 * n_blocks + 1) * kKBlkBytes + kMatBytes;   // Wp[3][32], bp[32], Wout[64], bout[2]+pad
   s.tips = s.small + (128 + VTACO_DEC_TAIL) * 4;
   s.stage = s.tips + VTACO_MAX_TIPS * 32 * 4;
   s.stage = (s.stage + 15) / 16 * 16;
@@ -56,18 +67,18 @@ __device__ __forceinline__ void issue_product(uint32_t d, uint32_t a_hi, uint32_
   const uint32_t a_lo = a_hi + 32;
   if (n_products == 2) {   // mixed: BF16 correction (K = 64) then the TF32 main product
 #pragma unroll
-    for (int kk = 0; kk < 4; ++kk) tc_mma_ts_bf16(d, a_lo + 8 * kk, make_bdesc(w_smem + 4096 + kk * 1024), kk > 0 ? 1u : accumulate_first);
+    for (int kk = 0; kk < 4; ++kk) tc_mma_ts_bf16(d, a_lo + 8 * kk, make_bdesc(w_smem + kLoBytes + kk * kKBlkBytes), kk > 0 ? 1u : accumulate_first);
     accumulate_first = 1;
   }
   if (n_products >= 3) {
 #pragma unroll
-    for (int kk = 0; kk < 4; ++kk) tc_mma_ts(d, a_lo + 8 * kk, make_bdesc(w_smem + kk * 1024), kk > 0 ? 1u : accumulate_first);
+    for (int kk = 0; kk < 4; ++kk) tc_mma_ts(d, a_lo + 8 * kk, make_bdesc(w_smem + kk * kKBlkBytes), kk > 0 ? 1u : accumulate_first);
 #pragma unroll
-    for (int kk = 0; kk < 4; ++kk) tc_mma_ts(d, a_hi + 8 * kk, make_bdesc(w_smem + 4096 + kk * 1024), 1);
+    for (int kk = 0; kk < 4; ++kk) tc_mma_ts(d, a_hi + 8 * kk, make_bdesc(w_smem + kLoBytes + kk * kKBlkBytes), 1);
     accumulate_first = 1;
   }
 #pragma unroll
-  for (int kk = 0; kk < 4; ++kk) tc_mma_ts(d, a_hi + 8 * kk, make_bdesc(w_smem + kk * 1024), kk > 0 ? 1u : accumulate_first);
+  for (int kk = 0; kk < 4; ++kk) tc_mma_ts(d, a_hi + 8 * kk, make_bdesc(w_smem + kk * kKBlkBytes), kk > 0 ? 1u : accumulate_first);
 }
 
 // Debug-only phase tracing (VTACO_TC_TRACE=1): clock64 stamps of one warp of block 0, group 0.
@@ -100,7 +111,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) decoder_tc_kernel(const __grid_
 
   // ---- one-time setup: weights + bias blocks (contiguous in wtc), small vectors, barriers, TMEM ----
   const bool cimg = P.use_img && P.c_img;   // per-query tactile feature tensor (decoder.py:83-85)
-  const int wtc_floats = 3 * nb * 2048 + (2 * nb + 1) * 256 + (cimg ? 2048 : 0);
+  const int wtc_floats = VTACO_DEC_TC_WIMG(kTcMode, nb) + (cimg ? VTACO_DEC_TC_MAT_FLOATS(kTcMode) : 0);
   for (int i = tid; i < wtc_floats / 4; i += kTcThreads)
     reinterpret_cast<float4*>(sWtc)[i] = __ldg(reinterpret_cast<const float4*>(wtc) + i);
   for (int i = tid; i < 128; i += kTcThreads) sSmall[i] = P.weights[(P.use_img ? VTACO_DEC_OFF_WPI : VTACO_DEC_OFF_WP) + i];
@@ -135,7 +146,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) decoder_tc_kernel(const __grid_
   const uint32_t mC = mbase, mX = mbase + 64, mOnes = mbase + 128, mD = mbase + 136;
   const uint32_t bar = smem_u32(sBars + g);
   const uint32_t wsm = smem_u32(sWtc), bsm = smem_u32(tsm + L.bias);
-  const uint32_t wimg_sm = bsm + (uint32_t)(2 * nb + 1) * 1024u;
+  const uint32_t wimg_sm = bsm + (uint32_t)(2 * nb + 1) * (uint32_t)kKBlkBytes;   // after the bias steps
   uint32_t ph = 0;
   {  // the constant A block that multiplies the bias rows: columns (1, 1, 0, 0, 0, 0, 0, 0)
     const uint32_t one = __float_as_uint(1.0f);
@@ -360,8 +371,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) decoder_tc_kernel(const __grid_
       TC_STAMP(4);   // group barrier passed
       if (wg == (step & 3) && elect_one()) {     // D = relu(net)*W0_i + ones*b0_i
         tc_fence_after();
-        issue_product(mD, mX, wsm + (3 * i + 1) * 8192, 0, P.tc_products);
-        tc_mma_ts(mD, mOnes, make_bdesc(bsm + (2 * i + 1) * 1024), 1);
+        issue_product(mD, mX, wsm + 4 * VTACO_DEC_TC_MAT(kTcMode, 3 * i + 1), 0, P.tc_products);
+        tc_mma_ts(mD, mOnes, make_bdesc(bsm + (2 * i + 1) * kKBlkBytes), 1);
         tc_commit(bar);
       }
       ++step;
@@ -382,9 +393,9 @@ __global__ void __launch_bounds__(kTcThreads, 1) decoder_tc_kernel(const __grid_
       TC_STAMP(9 + 16 * (i & 1));
       if (wg == (step & 3) && elect_one()) {     // D = relu(h)*W1_i + ones*(b1_i + bc_{i+1}) [+ C*Wc_{i+1}]
         tc_fence_after();
-        issue_product(mD, mX, wsm + (3 * i + 2) * 8192, 0, P.tc_products);
-        tc_mma_ts(mD, mOnes, make_bdesc(bsm + (2 * i + 2) * 1024), 1);
-        if (P.has_c && i + 1 < nb) issue_product(mD, mC, wsm + (3 * (i + 1)) * 8192, 1, P.tc_products);
+        issue_product(mD, mX, wsm + 4 * VTACO_DEC_TC_MAT(kTcMode, 3 * i + 2), 0, P.tc_products);
+        tc_mma_ts(mD, mOnes, make_bdesc(bsm + (2 * i + 2) * kKBlkBytes), 1);
+        if (P.has_c && i + 1 < nb) issue_product(mD, mC, wsm + 4 * VTACO_DEC_TC_MAT(kTcMode, 3 * (i + 1)), 1, P.tc_products);
         tc_commit(bar);
       }
       ++step;
@@ -481,8 +492,8 @@ struct Tc2Smem { int w, bias, small, tips, stage, head, axis, bars, tmem_ptr, to
 __host__ __device__ inline Tc2Smem tc2_smem_layout(int n_blocks) {
   Tc2Smem s;
   s.w = 0;
-  s.bias = s.w + 3 * n_blocks * 8192;
-  s.small = s.bias + (2 * n_blocks + 1) * 1024 + 8192;   // bias blocks, then fc_p_img.weight[:, 3:] hi|lo
+  s.bias = s.w + 4 * VTACO_DEC_TC_BIAS(kTcMode, n_blocks, 0);
+  s.small = s.bias + (2 * n_blocks + 1) * kKBlkBytes + kMatBytes;   // bias K-blocks, then fc_p_img.weight[:, 3:]
   s.tips = s.small + (128 + VTACO_DEC_TAIL) * 4;
   s.stage = s.tips + VTACO_MAX_TIPS * 32 * 4;
   s.stage = (s.stage + 15) / 16 * 16;
@@ -519,7 +530,7 @@ __global__ void __launch_bounds__(kTc2Threads, 1) decoder_tc2_kernel(const __gri
   const int nx = P.nx;
 
   const bool cimg = P.use_img && P.c_img;   // per-query tactile feature tensor (decoder.py:83-85)
-  const int wtc_floats = 3 * nb * 2048 + (2 * nb + 1) * 256 + (cimg ? 2048 : 0);
+  const int wtc_floats = VTACO_DEC_TC_WIMG(kTcMode, nb) + (cimg ? VTACO_DEC_TC_MAT_FLOATS(kTcMode) : 0);
   for (int i = tid; i < wtc_floats / 4; i += kTc2Threads)
     reinterpret_cast<float4*>(sWtc)[i] = __ldg(reinterpret_cast<const float4*>(wtc) + i);
   for (int i = tid; i < 128; i += kTc2Threads) sSmall[i] = P.weights[(P.use_img ? VTACO_DEC_OFF_WPI : VTACO_DEC_OFF_WP) + i];
@@ -556,7 +567,7 @@ __global__ void __launch_bounds__(kTc2Threads, 1) decoder_tc2_kernel(const __gri
   const uint32_t mC = mbase, mX = mbase + 64, mOnes = mbase + 128, mD = mbase + 136;
   const uint32_t bar = smem_u32(sBars + g);
   const uint32_t wsm = smem_u32(sWtc), bsm = smem_u32(tsm + L.bias);
-  const uint32_t wimg_sm = bsm + (uint32_t)(2 * nb + 1) * 1024u;
+  const uint32_t wimg_sm = bsm + (uint32_t)(2 * nb + 1) * (uint32_t)kKBlkBytes;   // after the bias steps
   const int gsync_id = g + 1;
   auto group_sync2 = [&]() { asm volatile("bar.sync %0, 256;" ::"r"(gsync_id) : "memory"); };
   uint32_t ph = 0;
@@ -775,8 +786,8 @@ __global__ void __launch_bounds__(kTc2Threads, 1) decoder_tc2_kernel(const __gri
       TC_STAMP(4);   // group barrier passed
       if (wq == (step & 7) && elect_one()) {     // D = relu(net)*W0_i + ones*b0_i
         tc_fence_after();
-        issue_product(mD, mX, wsm + (3 * i + 1) * 8192, 0, n_prod);
-        tc_mma_ts(mD, mOnes, make_bdesc(bsm + (2 * i + 1) * 1024), 1);
+        issue_product(mD, mX, wsm + 4 * VTACO_DEC_TC_MAT(kTcMode, 3 * i + 1), 0, n_prod);
+        tc_mma_ts(mD, mOnes, make_bdesc(bsm + (2 * i + 1) * kKBlkBytes), 1);
         tc_commit(bar);
         TC_STAMP(20);  // issuer only: 13 MMAs + commit issued
       }
@@ -796,9 +807,9 @@ __global__ void __launch_bounds__(kTc2Threads, 1) decoder_tc2_kernel(const __gri
       group_sync2();
       if (wq == (step & 7) && elect_one()) {     // D = relu(h)*W1_i + ones*(b1_i + bc_{i+1}) [+ C*Wc_{i+1}]
         tc_fence_after();
-        issue_product(mD, mX, wsm + (3 * i + 2) * 8192, 0, n_prod);
-        tc_mma_ts(mD, mOnes, make_bdesc(bsm + (2 * i + 2) * 1024), 1);
-        if (P.has_c && i + 1 < nb) issue_product(mD, mC, wsm + (3 * (i + 1)) * 8192, 1, n_prod);
+        issue_product(mD, mX, wsm + 4 * VTACO_DEC_TC_MAT(kTcMode, 3 * i + 2), 0, n_prod);
+        tc_mma_ts(mD, mOnes, make_bdesc(bsm + (2 * i + 2) * kKBlkBytes), 1);
+        if (P.has_c && i + 1 < nb) issue_product(mD, mC, wsm + 4 * VTACO_DEC_TC_MAT(kTcMode, 3 * (i + 1)), 1, n_prod);
         tc_commit(bar);
       }
       ++step;

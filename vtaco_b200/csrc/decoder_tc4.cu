@@ -32,16 +32,16 @@ constexpr int kT4Threads = 1024;
 constexpr int kT4Groups = 4;
 constexpr int kT4Cols = 128;
 constexpr int kT4StageRows = 24;          // staged z-rows per warp (separable gather) / 16 queries per pass (generic)
-constexpr int kT4MatBytes = 10240;        // W_hi 4 KB | W_lo 4 KB | bf16(W) 2 KB
+constexpr int kT4Mode = VTACO_DEC_TC_MODE_TILE4;   // weights_tc is copied to shared memory as it is
 constexpr int kT4MaxAxis = 2048;
 
 struct Tc4Smem { int w, bias, pw, small, tips, stage, head, axis, mm, bars, tmem_ptr, total; };
 __host__ __device__ inline Tc4Smem tc4_smem_layout(int n_blocks) {
   Tc4Smem s;
   s.w = 0;                                                   // 3*nb matrices, then fc_p_img.weight[:, 3:]
-  s.bias = s.w + (3 * n_blocks + 1) * kT4MatBytes;           // (2*nb+1) fp32 bias vectors
-  s.pw = (s.bias + (2 * n_blocks + 1) * 128 + 127) / 128 * 128;   // fc_p | fc_p_img[:, :3] as two K = 8 operand blocks (1 KB each)
-  s.small = s.pw + 2048;
+  s.bias = s.w + 4 * VTACO_DEC_TC_BIAS(kT4Mode, n_blocks, 0);   // (2*nb+1) fp32 bias vectors
+  s.pw = (s.bias + (2 * n_blocks + 1) * 4 * VTACO_DEC_TC_BVEC_FLOATS + 127) / 128 * 128;   // fc_p or fc_p_img[:, :3]: two K-blocks
+  s.small = s.pw + 2 * 4 * VTACO_DEC_TC_KBLK_FLOATS;
   s.tips = s.small + (128 + VTACO_DEC_TAIL) * 4;
   s.stage = s.tips + VTACO_MAX_TIPS * 32 * 4;
   s.stage = (s.stage + 15) / 16 * 16;
@@ -105,18 +105,22 @@ __device__ __forceinline__ uint64_t bdesc_at(uint32_t lo, uint32_t units) {
   return ((uint64_t)0x4008u << 32) | (uint64_t)(lo + units);
 }
 
+// descriptor units (16 bytes) of `floats` floats
+__host__ __device__ constexpr uint32_t desc_units(int floats) { return (uint32_t)floats / 4u; }
+constexpr uint32_t kKBlkUnits = desc_units(VTACO_DEC_TC_KBLK_FLOATS);   // a K = 8 TF32 block, or a K = 16 BF16 block
+
 // D (+)= A * W for one 32x32 matrix: A = (a_hi: 32 tf32 columns, a_lo = a_hi + 32: 16 bf16x2 columns),
-// W = the 10 KB block whose descriptor low word is `wlo`
+// W = the matrix whose descriptor low word is `wlo`
 __device__ __forceinline__ void issue_product_t4(uint32_t d, uint32_t a_hi, uint32_t wlo, uint32_t accumulate_first) {
 #pragma unroll
   for (int kk = 0; kk < 4; ++kk)   // hi * W_lo
-    tc_mma_ts(d, a_hi + 8 * kk, bdesc_at(wlo, 256 + kk * 64), kk > 0 ? 1u : accumulate_first);
+    tc_mma_ts(d, a_hi + 8 * kk, bdesc_at(wlo, desc_units(VTACO_DEC_TC_SUB_LO) + kk * kKBlkUnits), kk > 0 ? 1u : accumulate_first);
 #pragma unroll
   for (int kk = 0; kk < 2; ++kk)   // lo * bf16(W)
-    tc_mma_ts_bf16(d, a_hi + 32 + 8 * kk, bdesc_at(wlo, 512 + kk * 64), 1);
+    tc_mma_ts_bf16(d, a_hi + 32 + 8 * kk, bdesc_at(wlo, desc_units(VTACO_DEC_TC_SUB_BF16) + kk * kKBlkUnits), 1);
 #pragma unroll
   for (int kk = 0; kk < 4; ++kk)   // hi * W_hi
-    tc_mma_ts(d, a_hi + 8 * kk, bdesc_at(wlo, kk * 64), 1);
+    tc_mma_ts(d, a_hi + 8 * kk, bdesc_at(wlo, desc_units(VTACO_DEC_TC_SUB_HI) + kk * kKBlkUnits), 1);
 }
 
 #define T4_STAMP(slot)                                                            \
@@ -160,7 +164,7 @@ __global__ void __launch_bounds__(kT4Threads, 1) decoder_tc4_kernel(const __grid
   // issued by one thread; they land while the CTA allocates TMEM and gathers its first tile, and every thread waits
   // for them once, just before the first MMA issue (the plain load / store loop stood in front of everything: a few
   // microseconds per launch, 10 % of a training-shape call and 1 % of an 8-GPU slab).
-  const int wtc_floats = (3 * nb + 1) * (kT4MatBytes / 4) + (2 * nb + 1) * 32;
+  const int wtc_floats = VTACO_DEC_TC_INPUT(nb, 0);   // matrices and bias vectors
   const uint32_t wbar = smem_u32(sBars + kT4Groups);
   const bool w_tma = (reinterpret_cast<uintptr_t>(wtc) & 15) == 0;
   if (w_tma) {
@@ -181,12 +185,13 @@ __global__ void __launch_bounds__(kT4Threads, 1) decoder_tc4_kernel(const __grid
     for (int i = tid; i < wtc_floats / 4; i += kT4Threads)
       reinterpret_cast<float4*>(sWtc)[i] = __ldg(reinterpret_cast<const float4*>(wtc) + i);
   }
-  // the fc_p operand blocks follow the bias vectors in wtc: [fc_p B1 | B2 | fc_p_img B1 | B2], 256 floats each
-  for (int i = tid; i < 512; i += kT4Threads) sPw[i] = __ldg(wtc + wtc_floats + (P.use_img ? 512 : 0) + i);
+  // the two input-layer K-blocks of fc_p or fc_p_img[:, :3]
+  for (int i = tid; i < 2 * VTACO_DEC_TC_KBLK_FLOATS; i += kT4Threads)
+    sPw[i] = __ldg(wtc + wtc_floats + (P.use_img ? 2 * VTACO_DEC_TC_KBLK_FLOATS : 0) + i);
   for (int i = tid; i < 128; i += kT4Threads) {
     float v = P.weights[(P.use_img ? VTACO_DEC_OFF_WPI : VTACO_DEC_OFF_WP) + i];
     // bc_0 joins the fc_p bias: net = (W p + (bp + bc_0)) + Wc_0 c
-    if (i >= 96 && P.has_c) v += __ldg(wtc + (3 * nb + 1) * (kT4MatBytes / 4) + (i - 96));
+    if (i >= 96 && P.has_c) v += __ldg(wtc + VTACO_DEC_TC_BIAS(kT4Mode, nb, 0) + (i - 96));
     sSmall[i] = v;
   }
   for (int i = tid; i < VTACO_DEC_TAIL; i += kT4Threads)
@@ -222,9 +227,9 @@ __global__ void __launch_bounds__(kT4Threads, 1) decoder_tc4_kernel(const __grid
   const uint32_t mbase = tmem_base + (uint32_t)(g * kT4Cols);
   const uint32_t mC = mbase, mX = mbase + 48, mD = mbase + 96;
   const uint32_t bar = smem_u32(sBars + g);
-  // descriptor low word of matrix 0 (start address >> 4 | K-chunk stride 512 B); matrix m is m * 640 units further
+  // descriptor low word of matrix 0 (start address >> 4 | K-chunk stride 512 B); matrix m is m * kMatUnits further
   const uint32_t wlo0 = ((smem_u32(sWtc) >> 4) & 0x3fffu) | ((512u >> 4) << 16);
-  constexpr uint32_t kMatUnits = kT4MatBytes / 16;
+  constexpr uint32_t kMatUnits = desc_units(VTACO_DEC_TC_MAT_FLOATS(kT4Mode));
   const uint32_t pwlo = ((smem_u32(sPw) >> 4) & 0x3fffu) | ((512u >> 4) << 16);
   const int gsync_id = g + 1;
   int step = 0;   // accumulation steps issued so far by this group: rotates the issuing warp, its parity is the mbarrier phase
@@ -434,7 +439,7 @@ __global__ void __launch_bounds__(kT4Threads, 1) decoder_tc4_kernel(const __grid
         if (cimg) {
           issue_product_t4(mD, mX, wlo0 + (uint32_t)(3 * nb) * kMatUnits, acc);
         } else {
-          tc_mma_ts(mD, mX, bdesc_at(pwlo, 64), acc);
+          tc_mma_ts(mD, mX, bdesc_at(pwlo, kKBlkUnits), acc);
           tc_mma_ts(mD, mX, bdesc_at(pwlo, 0), 1);
         }
         tc_commit(bar);
@@ -471,7 +476,7 @@ __global__ void __launch_bounds__(kT4Threads, 1) decoder_tc4_kernel(const __grid
       tc_wait_ld();
 #pragma unroll
       for (int j = 0; j < 16; ++j) net[j] = __uint_as_float(r[j]);
-      if (nb > 0) store_bias16(tD + ch0, sBias + 1 * 32 + ch0);      // b0_0 for the first W0 step
+      if (nb > 0) store_bias16(tD + ch0, sBias + 1 * VTACO_DEC_TC_BVEC_FLOATS + ch0);      // b0_0 for the first W0 step
     }
     if (cimg) {   // c_img occupies the X columns: the 3-wide layer runs on the CUDA cores
       const float4* w0 = reinterpret_cast<const float4*>(sSmall + ch0);
@@ -535,7 +540,7 @@ __global__ void __launch_bounds__(kT4Threads, 1) decoder_tc4_kernel(const __grid
         }
         split_store_t4(tX, hv, y);
       }
-      store_bias16(tD + ch0, sBias + (2 * i + 2) * 32 + ch0);       // b1_i + bc_{i+1} for the W1 step
+      store_bias16(tD + ch0, sBias + (2 * i + 2) * VTACO_DEC_TC_BVEC_FLOATS + ch0);       // b1_i + bc_{i+1} for the W1 step
       tc_wait_st();
       tc_fence_before();
       group_sync();
@@ -556,7 +561,7 @@ __global__ void __launch_bounds__(kT4Threads, 1) decoder_tc4_kernel(const __grid
                                      make_float2(__uint_as_float(r[2 * j]), __uint_as_float(r[2 * j + 1])));
         net[2 * j] = n0.x; net[2 * j + 1] = n0.y;
       }
-      if (i + 1 < nb) store_bias16(tD + ch0, sBias + (2 * i + 3) * 32 + ch0);   // b0_{i+1} for the next W0 step
+      if (i + 1 < nb) store_bias16(tD + ch0, sBias + (2 * i + 3) * VTACO_DEC_TC_BVEC_FLOATS + ch0);   // b0_{i+1} for the next W0 step
     }
 
     T4_STAMP(19);    // blocks done

@@ -34,7 +34,7 @@ __device__ __forceinline__ float tf32_trunc(float w) { return __uint_as_float(__
 struct TcPackPlan {
   int n_mats, n_bias, mixed;
   int mat_src[3 * VTACO_MAX_BLOCKS + 1];    // float offsets into `packed`
-  int mat_dst[3 * VTACO_MAX_BLOCKS + 1];    // float offsets into the tc buffer (2048 floats each)
+  int mat_dst[3 * VTACO_MAX_BLOCKS + 1];    // float offsets into the tc buffer
   int bias_src0[2 * VTACO_MAX_BLOCKS + 1];  // -1 = zero
   int bias_src1[2 * VTACO_MAX_BLOCKS + 1];
   int bias_dst;
@@ -47,24 +47,24 @@ __global__ void __launch_bounds__(256) pack_tc_kernel(const __grid_constant__ Tc
   if (b < Pn.n_mats) {
     const float* src = packed + Pn.mat_src[b];
     float* out = dst + Pn.mat_dst[b];
-    for (int i = threadIdx.x; i < 1024; i += blockDim.x) {
+    for (int i = threadIdx.x; i < VTACO_DEC_HIDDEN * VTACO_DEC_HIDDEN; i += blockDim.x) {
       const int k = i >> 5, n = i & 31;
       float w = __ldg(src + i);                            // W[n][k] (nn.Linear weight[out=n][in=k])
       if (Pn.mixed == 2 && b < 3 * ((Pn.n_mats - 1) / 3) && (b % 3) != 0) w *= 0.5f;   // variant 7: fc_0 / fc_1 take 2*relu(x)
       const float hi = tf32_rn(w);
       const int idx = (k >> 2) * 128 + (n >> 3) * 32 + (n & 7) * 4 + (k & 3);
-      out[idx] = hi;
-      if (Pn.mixed == 2) {   // variant 7: TF32 hi | TF32 lo | bf16(W) (K = 32), 2560 floats per matrix
-        out[1024 + idx] = tf32_trunc(w - hi);
-        __nv_bfloat16* o16 = reinterpret_cast<__nv_bfloat16*>(out + 2048);
+      out[VTACO_DEC_TC_SUB_HI + idx] = hi;
+      if (Pn.mixed == 2) {   // TF32 hi | TF32 lo | bf16(W) (K = 32)
+        out[VTACO_DEC_TC_SUB_LO + idx] = tf32_trunc(w - hi);
+        __nv_bfloat16* o16 = reinterpret_cast<__nv_bfloat16*>(out + VTACO_DEC_TC_SUB_BF16);
         o16[(k >> 3) * 256 + (n >> 3) * 64 + (n & 7) * 8 + (k & 7)] = __float2bfloat16_rn(w);
       } else if (Pn.mixed) {   // K = 64 BF16 correction operand: rows k < 32 bf16(W), rows k >= 32 bf16(W - hi)
-        __nv_bfloat16* o16 = reinterpret_cast<__nv_bfloat16*>(out + 1024);
+        __nv_bfloat16* o16 = reinterpret_cast<__nv_bfloat16*>(out + VTACO_DEC_TC_SUB_LO);
         const int k1 = k + 32;
         o16[(k >> 3) * 256 + (n >> 3) * 64 + (n & 7) * 8 + (k & 7)] = __float2bfloat16_rn(w);
         o16[(k1 >> 3) * 256 + (n >> 3) * 64 + (n & 7) * 8 + (k1 & 7)] = __float2bfloat16_rn(w - hi);
       } else {
-        out[1024 + idx] = tf32_trunc(w - hi);
+        out[VTACO_DEC_TC_SUB_LO + idx] = tf32_trunc(w - hi);
       }
     }
   } else if (b >= Pn.n_mats + Pn.n_bias) {
@@ -73,8 +73,8 @@ __global__ void __launch_bounds__(256) pack_tc_kernel(const __grid_constant__ Tc
     const int q = b - Pn.n_mats - Pn.n_bias;          // 0: fc_p B1, 1: fc_p B2, 2: fc_p_img B1, 3: fc_p_img B2
     const int wsrc = (q >> 1) ? VTACO_DEC_OFF_WPI : VTACO_DEC_OFF_WP;
     const int bsrc = (q >> 1) ? VTACO_DEC_OFF_BPI : VTACO_DEC_OFF_BP;
-    float* out = dst + Pn.pw_dst + q * 256;
-    const int i = threadIdx.x;                        // 256 threads == 256 floats
+    float* out = dst + Pn.pw_dst + q * VTACO_DEC_TC_KBLK_FLOATS;
+    const int i = threadIdx.x;                        // 256 threads == one K-block
     const int k = (i >> 7) * 4 + (i & 3), n = ((i >> 5) & 3) * 8 + ((i >> 2) & 7);
     const int kk = k & 3;
     float v;
@@ -91,17 +91,17 @@ __global__ void __launch_bounds__(256) pack_tc_kernel(const __grid_constant__ Tc
     out[i] = o;
   } else {
     const int s = b - Pn.n_mats;
-    if (Pn.mixed == 2) {   // variant 7 adds the biases on the CUDA cores: plain fp32 vectors
-      if (threadIdx.x < 32) {
+    if (Pn.mixed == 2) {   // the four-tile kernel adds the biases on the CUDA cores: plain fp32 vectors
+      if (threadIdx.x < VTACO_DEC_TC_BVEC_FLOATS) {
         float bsum = 0.f;
         if (Pn.bias_src0[s] >= 0) bsum = __ldg(packed + Pn.bias_src0[s] + threadIdx.x);
         if (Pn.bias_src1[s] >= 0) bsum = bsum + __ldg(packed + Pn.bias_src1[s] + threadIdx.x);
-        dst[Pn.bias_dst + s * 32 + threadIdx.x] = bsum;
+        dst[Pn.bias_dst + s * VTACO_DEC_TC_BVEC_FLOATS + threadIdx.x] = bsum;
       }
       return;
     }
-    float* out = dst + Pn.bias_dst + s * 256;
-    for (int i = threadIdx.x; i < 256; i += blockDim.x) {
+    float* out = dst + Pn.bias_dst + s * VTACO_DEC_TC_KBLK_FLOATS;
+    for (int i = threadIdx.x; i < VTACO_DEC_TC_KBLK_FLOATS; i += blockDim.x) {
       // layout (k/4)*128 + (n/8)*32 + (n%8)*4 + (k%4) with k in [0,8): i -> (k, n)
       const int k = (i >> 7) * 4 + (i & 3), n = ((i >> 5) & 3) * 8 + ((i >> 2) & 7);
       float v = 0.f;
@@ -148,21 +148,19 @@ extern "C" int vtaco_decoder_pack_tc(const float* packed, int32_t n_blocks, int3
   TcPackPlan Pn = {};
   Pn.mixed = mixed;
   const int nb = n_blocks;
-  const int mat_floats = (mixed == 2) ? 2560 : 2048;
   for (int i = 0; i < nb; ++i) {
     const int o = VTACO_DEC_OFF_BLOCKS + i * VTACO_DEC_BLOCK_STRIDE;
     const int srcs[3] = {o + VTACO_DEC_BLK_WC, o + VTACO_DEC_BLK_W0, o + VTACO_DEC_BLK_W1};   // fc_c[i], fc_0, fc_1
     for (int j = 0; j < 3; ++j) {
       Pn.mat_src[3 * i + j] = srcs[j];
-      Pn.mat_dst[3 * i + j] = (3 * i + j) * mat_floats;
+      Pn.mat_dst[3 * i + j] = VTACO_DEC_TC_MAT(mixed, 3 * i + j);
     }
   }
   Pn.mat_src[3 * nb] = VTACO_DEC_OFF_WIMG;                       // fc_p_img.weight[:, 3:]
-  // layouts 0 / 1: the W_img block follows the bias K-blocks; layout 2: it follows the matrices, the bias vectors come last
-  Pn.mat_dst[3 * nb] = (mixed == 2) ? 3 * nb * mat_floats : 3 * nb * 2048 + (2 * nb + 1) * 256;
+  Pn.mat_dst[3 * nb] = VTACO_DEC_TC_WIMG(mixed, nb);
   Pn.n_mats = 3 * nb + 1;
   // bias steps: bc_0 | b0_i, b1_i + bc_{i+1}
-  Pn.bias_dst = (mixed == 2) ? (3 * nb + 1) * mat_floats : 3 * nb * 2048;
+  Pn.bias_dst = VTACO_DEC_TC_BIAS(mixed, nb, 0);
   Pn.n_bias = 2 * nb + 1;
   Pn.bias_src0[0] = nb > 0 ? VTACO_DEC_OFF_BLOCKS + VTACO_DEC_BLK_BC : -1;
   Pn.bias_src1[0] = -1;
@@ -173,7 +171,7 @@ extern "C" int vtaco_decoder_pack_tc(const float* packed, int32_t n_blocks, int3
     Pn.bias_src0[2 * i + 2] = o + VTACO_DEC_BLK_B1;
     Pn.bias_src1[2 * i + 2] = (i + 1 < nb) ? o + VTACO_DEC_BLOCK_STRIDE + VTACO_DEC_BLK_BC : -1;
   }
-  Pn.pw_dst = Pn.bias_dst + (2 * nb + 1) * 32;     // layout 2 only
+  Pn.pw_dst = VTACO_DEC_TC_INPUT(nb, 0);     // mode 2 only
   pack_tc_kernel<<<Pn.n_mats + Pn.n_bias + (mixed == 2 ? 4 : 0), 256, 0, (cudaStream_t)stream>>>(Pn, packed, dst);
   VTACO_LAUNCH_CHECK();
   return VTACO_OK;
