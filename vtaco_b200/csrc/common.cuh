@@ -21,6 +21,9 @@ void set_last_cuda_error(cudaError_t e);
 #define VTACO_LAUNCH_CHECK() VTACO_CUDA_CHECK(cudaPeekAtLastError())
 
 int num_sms();  // SM count of the current device (cached)
+// Lets `kernel` use `bytes` of dynamic shared memory on the current device.  The attribute is set once per
+// (kernel, device), and again only for a larger size; safe to call from several host threads.
+cudaError_t smem_opt_in(const void* kernel, size_t bytes);
 
 // Constants of src/common.py:283,288,302,306 formed like Python does: in double,
 // rounded to fp32 where they meet an fp32 tensor.

@@ -493,15 +493,9 @@ extern "C" int vtaco_conv3d_cl(const vtaco_conv3d_args* a, void* stream) {
   P.n_tiles = (int)tiles;
   const CvSmem L = cv_layout(a->ksize, kz, Cin);
   if (L.total > 227 * 1024) return VTACO_ERR_UNSUPPORTED;
-  static std::atomic<int> configured[64];
-  int dev = 0;
-  VTACO_CUDA_CHECK(cudaGetDevice(&dev));
-  if (configured[dev & 63].load(std::memory_order_relaxed) == 0) {
-    VTACO_CUDA_CHECK(cudaFuncSetAttribute(conv3d_tc_kernel<3, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    VTACO_CUDA_CHECK(cudaFuncSetAttribute(conv3d_tc_kernel<3, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    VTACO_CUDA_CHECK(cudaFuncSetAttribute(conv3d_tc_kernel<1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    configured[dev & 63].store(1, std::memory_order_relaxed);
-  }
+  VTACO_CUDA_CHECK(smem_opt_in((const void*)conv3d_tc_kernel<3, 3>, 227 * 1024));
+  VTACO_CUDA_CHECK(smem_opt_in((const void*)conv3d_tc_kernel<3, 1>, 227 * 1024));
+  VTACO_CUDA_CHECK(smem_opt_in((const void*)conv3d_tc_kernel<1, 1>, 227 * 1024));
   // persistent CTAs: one per SM in total, split over the (out-channel tile, sample) pairs
   long long gx = num_sms() / ((long long)(a->Cout / 32) * a->N);
   if (gx < 1) gx = 1;

@@ -1,6 +1,7 @@
 // Library plumbing (status strings, device query), point->cell indexing and the
 // self-measured FP32 FMA peak used as the decoder's roofline denominator.
 #include "common.cuh"
+#include <map>
 #include <mutex>
 
 namespace vtaco {
@@ -20,6 +21,21 @@ int num_sms() {
     cached[dev & 63].store(n, std::memory_order_relaxed);
   }
   return c;
+}
+
+cudaError_t smem_opt_in(const void* kernel, size_t bytes) {
+  int dev = 0;
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e != cudaSuccess) return e;
+  static std::mutex mu;
+  static std::map<std::pair<const void*, int>, size_t> done;   // largest size set, per (kernel, device)
+  std::lock_guard<std::mutex> lock(mu);
+  size_t& set = done[{kernel, dev}];
+  if (set < bytes) {
+    e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    if (e == cudaSuccess) set = bytes;
+  }
+  return e;
 }
 
 // ---------------------------------------------------------------------------------------

@@ -165,20 +165,7 @@ __global__ void __launch_bounds__(kThreads, 1) decoder_kernel(const __grid_const
           const int b = __shfl_sync(kFull, qb[s], src);
           const int q = s * kThreads + wbase + src;
           if (P.has_c) {
-            float4 c = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (P.grid) {
-              const int R = P.Rg;
-              const float4* vol = reinterpret_cast<const float4*>(P.grid) + (size_t)b * R * R * R * 8 + sub;
-              c = sample_volume(vol, R, norm3d(x, P.nc), norm3d(y, P.nc), norm3d(z, P.nc), P.nearest);
-            }
-            if (P.plane[0] || P.plane[1] || P.plane[2]) {
-              const int R = P.Rp;
-              const float ux = norm2d(x, P.nc), uy = norm2d(y, P.nc), uz = norm2d(z, P.nc);
-              const size_t boff = (size_t)b * R * R * 8 + sub;
-              if (P.plane[0]) c = f4_add(c, sample_plane(reinterpret_cast<const float4*>(P.plane[0]) + boff, R, ux, uz, P.nearest));
-              if (P.plane[1]) c = f4_add(c, sample_plane(reinterpret_cast<const float4*>(P.plane[1]) + boff, R, ux, uy, P.nearest));
-              if (P.plane[2]) c = f4_add(c, sample_plane(reinterpret_cast<const float4*>(P.plane[2]) + boff, R, uy, uz, P.nearest));
-            }
+            const float4 c = sample_feature_sum(P, b, sub, x, y, z);
             float* dst = sC + (4 * sub) * kSC + q;
             dst[0] = c.x; dst[kSC] = c.y; dst[2 * kSC] = c.z; dst[3 * kSC] = c.w;
           }
@@ -270,17 +257,7 @@ __global__ void __launch_bounds__(kThreads, 1) decoder_kernel(const __grid_const
     __syncwarp();
   }
 
-  if (P.minmax_key) {
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) {
-      vmin = fminf(vmin, __shfl_xor_sync(kFull, vmin, d));
-      vmax = fmaxf(vmax, __shfl_xor_sync(kFull, vmax, d));
-    }
-    if (lane == 0 && vmin <= vmax) {
-      atomicMin(P.minmax_key, float_to_key(vmin));
-      atomicMax(P.minmax_key + 1, float_to_key(vmax));
-    }
-  }
+  flush_minmax(P, vmin, vmax, lane);
 }
 
 // Gather-only kernel behind LocalDecoder.sample_plane_feature / sample_grid_feature
@@ -293,20 +270,7 @@ __global__ void __launch_bounds__(256) sample_features_kernel(const __grid_const
     const float x = __ldg(P.p + n * 3), y = __ldg(P.p + n * 3 + 1), z = __ldg(P.p + n * 3 + 2);
     const int b = (int)(n / P.N);
     const long long i = n - (long long)b * P.N;
-    float4 c = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (P.grid) {
-      const int R = P.Rg;
-      const float4* vol = reinterpret_cast<const float4*>(P.grid) + (size_t)b * R * R * R * 8 + sub;
-      c = sample_volume(vol, R, norm3d(x, P.nc), norm3d(y, P.nc), norm3d(z, P.nc), P.nearest);
-    }
-    if (P.plane[0] || P.plane[1] || P.plane[2]) {
-      const int R = P.Rp;
-      const float ux = norm2d(x, P.nc), uy = norm2d(y, P.nc), uz = norm2d(z, P.nc);
-      const size_t boff = (size_t)b * R * R * 8 + sub;
-      if (P.plane[0]) c = f4_add(c, sample_plane(reinterpret_cast<const float4*>(P.plane[0]) + boff, R, ux, uz, P.nearest));
-      if (P.plane[1]) c = f4_add(c, sample_plane(reinterpret_cast<const float4*>(P.plane[1]) + boff, R, ux, uy, P.nearest));
-      if (P.plane[2]) c = f4_add(c, sample_plane(reinterpret_cast<const float4*>(P.plane[2]) + boff, R, uy, uz, P.nearest));
-    }
+    const float4 c = sample_feature_sum(P, b, sub, x, y, z);
     float* o = out + ((size_t)b * 32 + 4 * sub) * P.N + i;
     o[0] = c.x; o[P.N] = c.y; o[2 * P.N] = c.z; o[3 * P.N] = c.w;
   }
@@ -401,14 +365,7 @@ extern "C" int vtaco_relayout_cf(const float* src, float* dst, int B, int C, int
 
 template <bool DENSE, bool F2>
 static int launch_decoder(const DecParams& P, size_t smem_bytes, cudaStream_t stream) {
-  static std::atomic<size_t> configured[64];  // per instantiation, per device; idempotent, thread-safe
-  int dev = 0;
-  VTACO_CUDA_CHECK(cudaGetDevice(&dev));
-  if (configured[dev & 63].load(std::memory_order_relaxed) < smem_bytes) {
-    VTACO_CUDA_CHECK(cudaFuncSetAttribute(decoder_kernel<DENSE, F2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          (int)smem_bytes));
-    configured[dev & 63].store(smem_bytes, std::memory_order_relaxed);
-  }
+  VTACO_CUDA_CHECK(smem_opt_in((const void*)decoder_kernel<DENSE, F2>, smem_bytes));
   const long long grid = P.n_tiles < (long long)num_sms() ? P.n_tiles : (long long)num_sms();
   decoder_kernel<DENSE, F2><<<(unsigned)grid, kThreads, smem_bytes, stream>>>(P);
   VTACO_LAUNCH_CHECK();

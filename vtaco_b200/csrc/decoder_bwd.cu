@@ -382,14 +382,7 @@ extern "C" int vtaco_decoder_backward(const vtaco_decoder_bwd_args* a, void* str
   P.nc = make_norm_const(a->padding, a->div_mode);
 
   const size_t smem = ((size_t)P.wfloats + 3 * 32 * kBS) * sizeof(float) + (size_t)2 * nb * kBT * sizeof(uint32_t);
-  static bool attr_done[64] = {false};
-  int dev = 0;
-  VTACO_CUDA_CHECK(cudaGetDevice(&dev));
-  if (!attr_done[dev & 63]) {
-    VTACO_CUDA_CHECK(cudaFuncSetAttribute(decoder_bwd_query_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          (int)(227 * 1024)));
-    attr_done[dev & 63] = true;
-  }
+  VTACO_CUDA_CHECK(smem_opt_in((const void*)decoder_bwd_query_kernel, 227 * 1024));
   if (smem > 227 * 1024) return VTACO_ERR_UNSUPPORTED;
   const long long tiles = (Q + kBT - 1) / kBT;
   const int grid = (int)std::min<long long>(tiles, num_sms());

@@ -133,6 +133,41 @@ __device__ __forceinline__ float4 sample_plane(const float4* __restrict__ pl, in
   return a;
 }
 
+// c of one query (decoder.py:55-68): the sum of its samples of the grid and the planes, channels
+// [4*sub, 4*sub + 4) of sample b
+__device__ __forceinline__ float4 sample_feature_sum(const DecParams& P, int b, int sub, float x, float y, float z) {
+  float4 c = make_float4(0.f, 0.f, 0.f, 0.f);
+  if (P.grid) {
+    const int R = P.Rg;
+    const float4* vol = reinterpret_cast<const float4*>(P.grid) + (size_t)b * R * R * R * 8 + sub;
+    c = sample_volume(vol, R, norm3d(x, P.nc), norm3d(y, P.nc), norm3d(z, P.nc), P.nearest);
+  }
+  if (P.plane[0] || P.plane[1] || P.plane[2]) {
+    const int R = P.Rp;
+    const float ux = norm2d(x, P.nc), uy = norm2d(y, P.nc), uz = norm2d(z, P.nc);
+    const size_t boff = (size_t)b * R * R * 8 + sub;
+    if (P.plane[0]) c = f4_add(c, sample_plane(reinterpret_cast<const float4*>(P.plane[0]) + boff, R, ux, uz, P.nearest));
+    if (P.plane[1]) c = f4_add(c, sample_plane(reinterpret_cast<const float4*>(P.plane[1]) + boff, R, ux, uy, P.nearest));
+    if (P.plane[2]) c = f4_add(c, sample_plane(reinterpret_cast<const float4*>(P.plane[2]) + boff, R, uy, uz, P.nearest));
+  }
+  return c;
+}
+
+// Warp-reduce the running logit min / max and merge them into P.minmax_key (ordered-int keys)
+__device__ __forceinline__ void flush_minmax(const DecParams& P, float vmin, float vmax, int lane) {
+  if (P.minmax_key) {
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) {
+      vmin = fminf(vmin, __shfl_xor_sync(kFull, vmin, d));
+      vmax = fmaxf(vmax, __shfl_xor_sync(kFull, vmax, d));
+    }
+    if (lane == 0 && vmin <= vmax) {
+      atomicMin(P.minmax_key, float_to_key(vmin));
+      atomicMax(P.minmax_key + 1, float_to_key(vmax));
+    }
+  }
+}
+
 // generation.py:190-200: nearest fingertip in float64 (scipy cdist), within radius, touched.
 __device__ __forceinline__ int tip_assign(const DecParams& P, float x, float y, float z);
 // tactile feature row of a query: from the byte map when given, else the in-kernel fingertip test

@@ -81,13 +81,6 @@ __device__ __forceinline__ void issue_product(uint32_t d, uint32_t a_hi, uint32_
   for (int kk = 0; kk < 4; ++kk) tc_mma_ts(d, a_hi + 8 * kk, make_bdesc(w_smem + kk * kKBlkBytes), kk > 0 ? 1u : accumulate_first);
 }
 
-// Debug-only phase tracing (VTACO_TC_TRACE=1): clock64 stamps of one warp of block 0, group 0.
-#define TC_STAMP(slot)                                                            \
-  do {                                                                            \
-    if (trace && blockIdx.x == 0 && warp == 0 && lane == 0 && trace_n < 4096)     \
-      trace[trace_n++] = ((long long)(slot) << 56) | (clock64() & 0x00ffffffffffffffll); \
-  } while (0)
-
 template <bool DENSE, bool MIXED>
 __global__ void __launch_bounds__(kTcThreads, 1) decoder_tc_kernel(const __grid_constant__ DecParams P,
                                                                    const float* __restrict__ wtc,
@@ -114,31 +107,10 @@ __global__ void __launch_bounds__(kTcThreads, 1) decoder_tc_kernel(const __grid_
   const int wtc_floats = VTACO_DEC_TC_WIMG(kTcMode, nb) + (cimg ? VTACO_DEC_TC_MAT_FLOATS(kTcMode) : 0);
   for (int i = tid; i < wtc_floats / 4; i += kTcThreads)
     reinterpret_cast<float4*>(sWtc)[i] = __ldg(reinterpret_cast<const float4*>(wtc) + i);
-  for (int i = tid; i < 128; i += kTcThreads) sSmall[i] = P.weights[(P.use_img ? VTACO_DEC_OFF_WPI : VTACO_DEC_OFF_WP) + i];
-  for (int i = tid; i < VTACO_DEC_TAIL; i += kTcThreads)
-    sSmall[128 + i] = P.weights[VTACO_DEC_OFF_BLOCKS + nb * VTACO_DEC_BLOCK_STRIDE + i];
-  if (P.n_tips > 0) {
-    for (int o = tid; o < P.n_tips * 32; o += kTcThreads) {
-      const int f = o >> 5, j = o & 31;
-      float a = 0.f;
-      for (int k = 0; k < 32; ++k)
-        a = fmaf(__ldg(P.weights + VTACO_DEC_OFF_WIMG + k * 32 + j), __ldg(P.tip_feat + f * 32 + k), a);
-      sTip[o] = a;
-    }
-  }
-  if (tid == 0) {
-    for (int i = 0; i < kTcGroups; ++i) mbar_init(smem_u32(sBars + i), 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(sTmem)), "r"(512)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = __shfl_sync(kFull, *sTmem, 0);
+  load_small(sSmall, P, nb, tid, kTcThreads);
+  load_tips(sTip, P, tid, kTcThreads);
+  init_group_bars(sBars, kTcGroups, tid);
+  const uint32_t tmem_base = tmem_alloc_all(sTmem, warp);
   // group columns: C_hi 0, C_lo 32, X_hi 64, X_lo 96, ones 128 (8), D 136 (32)
   const uint32_t tbase = tmem_base + ((uint32_t)(32 * wg) << 16) + (uint32_t)(g * kColsPerGroup);
   const uint32_t tC = tbase, tX = tbase + 64, tOnes = tbase + 128, tD = tbase + 136;
@@ -164,36 +136,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) decoder_tc_kernel(const __grid_
 
   for (long long tile = (long long)blockIdx.x * kTcGroups + g; tile < P.n_tiles;
        tile += (long long)gridDim.x * kTcGroups) {
-    // ---------------- this thread's query ----------------
-    float px, py, pz;
-    long long oidx;
-    int qb;
-    bool valid;
-    if (DENSE) {
-      unsigned t = (unsigned)tile;                        // n_tiles < 2^31 (checked at launch)
-      const int bz = (int)(t % (unsigned)P.t_nbz); t /= (unsigned)P.t_nbz;   // bricks: 2 (x) x 2 (y) x 32 (z): a warp = one
-      const int by = (int)(t % (unsigned)P.t_nby); t /= (unsigned)P.t_nby;   // z-run, its 32 logits are one 128-byte store
-      const int bx = (int)(t % (unsigned)P.t_nbx);
-      const int b = (int)(t / (unsigned)P.t_nbx);
-      const int ix = P.x0 + bx * 2 + (tg >> 6), iy = by * 2 + ((tg >> 5) & 1), iz = bz * 32 + (tg & 31);
-      valid = (ix < P.t_xend) && (iy < nx) && (iz < nx);
-      px = __ldg(P.axis + min(ix, nx - 1));
-      py = __ldg(P.axis + min(iy, nx - 1));
-      pz = __ldg(P.axis + min(iz, nx - 1));
-      qb = b;
-      oidx = (((long long)b * nx + ix) * nx + iy) * nx + iz;
-    } else {
-      const long long n = tile * kTcTile + tg;
-      valid = n < P.total;
-      const long long nn = valid ? n : 0;
-      px = __ldg(P.p + nn * 3 + 0);
-      py = __ldg(P.p + nn * 3 + 1);
-      pz = __ldg(P.p + nn * 3 + 2);
-      qb = (int)(nn / P.N);
-      oidx = nn;
-    }
-    if (!valid) oidx = 0;
-    TC_STAMP(13);  // tile start: coordinates loaded
+    const auto [px, py, pz, oidx, qb, valid] = tile_query(P, DENSE, tile, tg, nullptr, false, nx);   // this thread's query
+    TC_STAMP(trace, 13);  // tile start: coordinates loaded
 
     // ---------------- gather (+ the query's c_img row): operands of step 0 ----------------
     if (P.has_c || cimg) {
@@ -201,51 +145,36 @@ __global__ void __launch_bounds__(kTcThreads, 1) decoder_tc_kernel(const __grid_
       float cv[32];
       bool sep_done = false;
       if (DENSE && P.grid && !P.nearest && !(P.plane[0] || P.plane[1] || P.plane[2])) {
-        // Separable dense gather: a warp is one z-run of 32 lattice points at fixed (x, y), so the
-        // (x,y)-bilinear part of the trilinear sample is shared by the whole run.  Reduce the 4
-        // (x,y) corners once per needed z-row into shared memory (4 z-rows x 8 channel quads per
-        // load step), then every thread lerps its two z-rows: ~40 tap loads per run instead of 256.
+        // Separable dense gather (4 z-rows x 8 channel quads per load step): ~40 tap loads per run instead of 256
         const int R = P.Rg;
-        const float tx = unnormalize(norm3d(px, P.nc), R), ty = unnormalize(norm3d(py, P.nc), R);
-        const float tz = unnormalize(norm3d(pz, P.nc), R);
-        const float flx = floorf(tx), fly = floorf(ty), flz = floorf(tz);
-        const int x0 = (int)flx, y0 = (int)fly, z0 = (int)flz;
-        const float fx1 = tx - flx, fx0 = (flx + 1.0f) - tx, fy1 = ty - fly, fy0 = (fly + 1.0f) - ty;
-        const float fz1 = tz - flz, fz0 = (flz + 1.0f) - tz;
-        const int zmin = __shfl_sync(kFull, z0, 0);
-        const int zmax = min(__shfl_sync(kFull, z0, 31) + 1, R - 1);
-        const int nz = zmax - zmin + 1;
-        if (nz <= 32) {   // warp-uniform
-          const int dx = (x0 + 1 < R) ? 8 : 0, dy = (y0 + 1 < R) ? R * 8 : 0;   // clamped corners carry weight 0
-          const float w00 = fx0 * fy0, w01 = fx1 * fy0, w10 = fx0 * fy1, w11 = fx1 * fy1;
+        const SepGather sg = sep_gather_setup(P, px, py, pz, qb, sub);
+        if (sg.nz <= 32) {   // warp-uniform
           const int zr = lane >> 3;
-          const float4* col = reinterpret_cast<const float4*>(P.grid) + (size_t)qb * R * R * R * 8 +
-                              ((size_t)y0 * R + x0) * 8 + sub;
 #pragma unroll 2
-          for (int zb = 0; zb < nz; zb += 4) {
+          for (int zb = 0; zb < sg.nz; zb += 4) {
             const int zrow = zb + zr;
-            if (zrow < nz) {
-              const float4* p = col + (size_t)(zmin + zrow) * R * R * 8;
-              const float4 v00 = __ldg(p), v01 = __ldg(p + dx), v10 = __ldg(p + dy), v11 = __ldg(p + dy + dx);
+            if (zrow < sg.nz) {
+              const float4* p = sg.col + (size_t)(sg.zmin + zrow) * R * R * 8;
+              const float4 v00 = __ldg(p), v01 = __ldg(p + sg.dx), v10 = __ldg(p + sg.dy), v11 = __ldg(p + sg.dy + sg.dx);
               float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
-              a = f4_fma(w00, v00, a);
-              a = f4_fma(w01, v01, a);
-              a = f4_fma(w10, v10, a);
-              a = f4_fma(w11, v11, a);
+              a = f4_fma(sg.w00, v00, a);
+              a = f4_fma(sg.w01, v01, a);
+              a = f4_fma(sg.w10, v10, a);
+              a = f4_fma(sg.w11, v11, a);
               *reinterpret_cast<float4*>(stage + zrow * kStageStride + 4 * sub) = a;
             }
           }
           __syncwarp();
-          const float* r0 = stage + (z0 - zmin) * kStageStride;
-          const float* r1 = stage + (min(z0 + 1, R - 1) - zmin) * kStageStride;
+          const float* r0 = stage + (sg.z0 - sg.zmin) * kStageStride;
+          const float* r1 = stage + (min(sg.z0 + 1, R - 1) - sg.zmin) * kStageStride;
 #pragma unroll
           for (int j = 0; j < 8; ++j) {
             const float4 a = *reinterpret_cast<const float4*>(r0 + 4 * j);
             const float4 b = *reinterpret_cast<const float4*>(r1 + 4 * j);
-            cv[4 * j + 0] = fmaf(b.x, fz1, a.x * fz0);
-            cv[4 * j + 1] = fmaf(b.y, fz1, a.y * fz0);
-            cv[4 * j + 2] = fmaf(b.z, fz1, a.z * fz0);
-            cv[4 * j + 3] = fmaf(b.w, fz1, a.w * fz0);
+            cv[4 * j + 0] = fmaf(b.x, sg.fz1, a.x * sg.fz0);
+            cv[4 * j + 1] = fmaf(b.y, sg.fz1, a.y * sg.fz0);
+            cv[4 * j + 2] = fmaf(b.z, sg.fz1, a.z * sg.fz0);
+            cv[4 * j + 3] = fmaf(b.w, sg.fz1, a.w * sg.fz0);
           }
           __syncwarp();
           sep_done = true;
@@ -253,34 +182,13 @@ __global__ void __launch_bounds__(kTcThreads, 1) decoder_tc_kernel(const __grid_
       }
       if (!sep_done) {
       // generic gather: the owner computes the taps, 8 lanes fetch them
-      TapInfo tv, tp0, tp1, tp2;
-      if (P.grid) tv = tap_volume(norm3d(px, P.nc), norm3d(py, P.nc), norm3d(pz, P.nc), P.Rg, P.nearest);
-      const bool planes = P.plane[0] || P.plane[1] || P.plane[2];
-      if (planes) {
-        const float ux = norm2d(px, P.nc), uy = norm2d(py, P.nc), uz = norm2d(pz, P.nc);
-        if (P.plane[0]) tp0 = tap_plane(ux, uz, P.Rp, P.nearest);
-        if (P.plane[1]) tp1 = tap_plane(ux, uy, P.Rp, P.nearest);
-        if (P.plane[2]) tp2 = tap_plane(uy, uz, P.Rp, P.nearest);
-      }
-      TC_STAMP(14);  // taps computed
+      const QueryTaps taps = query_taps(P, px, py, pz);
+      TC_STAMP(trace, 14);  // taps computed
 #pragma unroll 2
       for (int it = 0; it < 8; ++it) {
         const int src = it * 4 + grp;
         const int b = __shfl_sync(kFull, qb, src);
-        float4 c = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (P.grid) {
-          const int R = P.Rg;
-          const float4* vol = reinterpret_cast<const float4*>(P.grid) + (size_t)b * R * R * R * 8 + sub;
-          c = fetch_volume(vol, R, tap_bcast(tv, src), P.nearest);
-        }
-        if (planes) {
-          const int R = P.Rp;
-          const size_t boff = (size_t)b * R * R * 8 + sub;
-          if (P.plane[0]) c = f4_add(c, fetch_plane(reinterpret_cast<const float4*>(P.plane[0]) + boff, R, tap_bcast(tp0, src), P.nearest));
-          if (P.plane[1]) c = f4_add(c, fetch_plane(reinterpret_cast<const float4*>(P.plane[1]) + boff, R, tap_bcast(tp1, src), P.nearest));
-          if (P.plane[2]) c = f4_add(c, fetch_plane(reinterpret_cast<const float4*>(P.plane[2]) + boff, R, tap_bcast(tp2, src), P.nearest));
-        }
-        *reinterpret_cast<float4*>(stage + src * kStageStride + 4 * sub) = c;
+        *reinterpret_cast<float4*>(stage + src * kStageStride + 4 * sub) = gather_taps(P, taps, src, b, sub);
       }
       __syncwarp();
 #pragma unroll
@@ -290,7 +198,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) decoder_tc_kernel(const __grid_
       }
       __syncwarp();
       }  // generic gather
-      TC_STAMP(15);  // features of the thread's query in registers
+      TC_STAMP(trace, 15);  // features of the thread's query in registers
       split_store(tC, cv, mixed);
      }
       if (cimg) {   // fc_p_img(cat[p, c_img]) = fc_p_img[:, :3] p + b + W_img c_img: the last term rides in step 0
@@ -306,7 +214,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) decoder_tc_kernel(const __grid_
       tc_wait_st();
       tc_fence_before();
       group_sync(g);
-      TC_STAMP(16);  // C in TMEM, group synced
+      TC_STAMP(trace, 16);  // C in TMEM, group synced
       if (wg == (step & 3) && elect_one()) {     // step 0: D = C*Wc_0 + ones*bc_0 [+ c_img*W_img]
         tc_fence_after();
         uint32_t acc = 0;
@@ -344,7 +252,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) decoder_tc_kernel(const __grid_
         for (int j = 0; j < 32; ++j) net[j] += sTip[f * 32 + j];
       }
     }
-    TC_STAMP(17);    // fc_p / tips done
+    TC_STAMP(trace, 17);    // fc_p / tips done
     uint32_t r[32];
     float x[32];
     if (P.has_c || cimg) {  // net += fc_c[0](c) [+ W_img c_img]
@@ -356,19 +264,19 @@ __global__ void __launch_bounds__(kTcThreads, 1) decoder_tc_kernel(const __grid_
       for (int j = 0; j < 32; ++j) net[j] += __uint_as_float(r[j]);
     }
 
-    TC_STAMP(18);    // step 0 consumed
+    TC_STAMP(trace, 18);    // step 0 consumed
     // ---------------- residual blocks: 2 accumulation steps each ----------------
     for (int i = 0; i < nb; ++i) {
-      TC_STAMP(1);   // ALU phase starts (accumulator already read)
+      TC_STAMP(trace, 1);   // ALU phase starts (accumulator already read)
 #pragma unroll
       for (int j = 0; j < 32; ++j) x[j] = fmaxf(net[j], 0.f);
       split_store(tX, x, mixed);
-      TC_STAMP(2);   // operands computed, tcgen05.st issued
+      TC_STAMP(trace, 2);   // operands computed, tcgen05.st issued
       tc_wait_st();
       tc_fence_before();
-      TC_STAMP(3);   // stores complete
+      TC_STAMP(trace, 3);   // stores complete
       group_sync(g);
-      TC_STAMP(4);   // group barrier passed
+      TC_STAMP(trace, 4);   // group barrier passed
       if (wg == (step & 3) && elect_one()) {     // D = relu(net)*W0_i + ones*b0_i
         tc_fence_after();
         issue_product(mD, mX, wsm + 4 * VTACO_DEC_TC_MAT(kTcMode, 3 * i + 1), 0, P.tc_products);
@@ -376,21 +284,21 @@ __global__ void __launch_bounds__(kTcThreads, 1) decoder_tc_kernel(const __grid_
         tc_commit(bar);
       }
       ++step;
-      TC_STAMP(5);   // (issuing warp: MMAs issued)
+      TC_STAMP(trace, 5);   // (issuing warp: MMAs issued)
       mbar_wait(bar, ph); ph ^= 1;
-      TC_STAMP(6);   // MMAs complete
+      TC_STAMP(trace, 6);   // MMAs complete
       tc_fence_after();
       tmem_ld32(tD, r);
       tc_wait_ld();
-      TC_STAMP(7);   // accumulator in registers
+      TC_STAMP(trace, 7);   // accumulator in registers
 #pragma unroll
       for (int j = 0; j < 32; ++j) x[j] = fmaxf(__uint_as_float(r[j]), 0.f);
       split_store(tX, x, mixed);
-      TC_STAMP(8 + 16 * (i & 1));    // W1 step: operands computed (+16: warp 0 is this step's issuer)
+      TC_STAMP(trace, 8 + 16 * (i & 1));    // W1 step: operands computed (+16: warp 0 is this step's issuer)
       tc_wait_st();
       tc_fence_before();
       group_sync(g);
-      TC_STAMP(9 + 16 * (i & 1));
+      TC_STAMP(trace, 9 + 16 * (i & 1));
       if (wg == (step & 3) && elect_one()) {     // D = relu(h)*W1_i + ones*(b1_i + bc_{i+1}) [+ C*Wc_{i+1}]
         tc_fence_after();
         issue_product(mD, mX, wsm + 4 * VTACO_DEC_TC_MAT(kTcMode, 3 * i + 2), 0, P.tc_products);
@@ -399,18 +307,18 @@ __global__ void __launch_bounds__(kTcThreads, 1) decoder_tc_kernel(const __grid_
         tc_commit(bar);
       }
       ++step;
-      TC_STAMP(10 + 16 * (i & 1));
+      TC_STAMP(trace, 10 + 16 * (i & 1));
       mbar_wait(bar, ph); ph ^= 1;
-      TC_STAMP(11 + 16 * (i & 1));
+      TC_STAMP(trace, 11 + 16 * (i & 1));
       tc_fence_after();
       tmem_ld32(tD, r);
       tc_wait_ld();
-      TC_STAMP(12 + 16 * (i & 1));
+      TC_STAMP(trace, 12 + 16 * (i & 1));
 #pragma unroll
       for (int j = 0; j < 32; ++j) net[j] += __uint_as_float(r[j]);
     }
 
-    TC_STAMP(19);    // blocks done
+    TC_STAMP(trace, 19);    // blocks done
     // ---------------- heads ----------------
     {
       const float* Wo = sSmall + 128;
@@ -434,22 +342,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) decoder_tc_kernel(const __grid_
     }
   }
 
-  if (P.minmax_key) {
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) {
-      vmin = fminf(vmin, __shfl_xor_sync(kFull, vmin, d));
-      vmax = fmaxf(vmax, __shfl_xor_sync(kFull, vmax, d));
-    }
-    if (lane == 0 && vmin <= vmax) {
-      atomicMin(P.minmax_key, float_to_key(vmin));
-      atomicMax(P.minmax_key + 1, float_to_key(vmax));
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-  }
+  flush_minmax(P, vmin, vmax, lane);
+  tmem_free_all(tmem_base, warp);
 }
 
 
@@ -533,34 +427,13 @@ __global__ void __launch_bounds__(kTc2Threads, 1) decoder_tc2_kernel(const __gri
   const int wtc_floats = VTACO_DEC_TC_WIMG(kTcMode, nb) + (cimg ? VTACO_DEC_TC_MAT_FLOATS(kTcMode) : 0);
   for (int i = tid; i < wtc_floats / 4; i += kTc2Threads)
     reinterpret_cast<float4*>(sWtc)[i] = __ldg(reinterpret_cast<const float4*>(wtc) + i);
-  for (int i = tid; i < 128; i += kTc2Threads) sSmall[i] = P.weights[(P.use_img ? VTACO_DEC_OFF_WPI : VTACO_DEC_OFF_WP) + i];
-  for (int i = tid; i < VTACO_DEC_TAIL; i += kTc2Threads)
-    sSmall[128 + i] = P.weights[VTACO_DEC_OFF_BLOCKS + nb * VTACO_DEC_BLOCK_STRIDE + i];
+  load_small(sSmall, P, nb, tid, kTc2Threads);
   const bool axis_sm = DENSE && nx <= kTcMaxAxis;
   if (axis_sm)
     for (int i = tid; i < nx; i += kTc2Threads) sAxis[i] = __ldg(P.axis + i);
-  if (P.n_tips > 0) {
-    for (int o = tid; o < P.n_tips * 32; o += kTc2Threads) {
-      const int f = o >> 5, j = o & 31;
-      float a = 0.f;
-      for (int k = 0; k < 32; ++k)
-        a = fmaf(__ldg(P.weights + VTACO_DEC_OFF_WIMG + k * 32 + j), __ldg(P.tip_feat + f * 32 + k), a);
-      sTip[o] = a;
-    }
-  }
-  if (tid == 0) {
-    for (int i = 0; i < kTcGroups; ++i) mbar_init(smem_u32(sBars + i), 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(sTmem)), "r"(512)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = __shfl_sync(kFull, *sTmem, 0);
+  load_tips(sTip, P, tid, kTc2Threads);
+  init_group_bars(sBars, kTcGroups, tid);
+  const uint32_t tmem_base = tmem_alloc_all(sTmem, warp);
   const uint32_t tbase = tmem_base + ((uint32_t)(32 * lq) << 16) + (uint32_t)(g * kColsPerGroup);
   const uint32_t tC = tbase, tX = tbase + 64, tOnes = tbase + 128, tD = tbase + 136;
   const uint32_t mbase = tmem_base + (uint32_t)(g * kColsPerGroup);
@@ -590,35 +463,8 @@ __global__ void __launch_bounds__(kTc2Threads, 1) decoder_tc2_kernel(const __gri
 
   for (long long tile = (long long)blockIdx.x * kTcGroups + g; tile < P.n_tiles;
        tile += (long long)gridDim.x * kTcGroups) {
-    float px, py, pz;
-    long long oidx;
-    int qb;
-    bool valid;
-    if (DENSE) {
-      unsigned t = (unsigned)tile;
-      const int bz = (int)(t % (unsigned)P.t_nbz); t /= (unsigned)P.t_nbz;
-      const int by = (int)(t % (unsigned)P.t_nby); t /= (unsigned)P.t_nby;
-      const int bx = (int)(t % (unsigned)P.t_nbx);
-      qb = (int)(t / (unsigned)P.t_nbx);
-      const int ix = P.x0 + bx * 2 + (tq >> 6), iy = by * 2 + ((tq >> 5) & 1), iz = bz * 32 + (tq & 31);
-      valid = (ix < P.t_xend) && (iy < nx) && (iz < nx);
-      const int cx = min(ix, nx - 1), cy = min(iy, nx - 1), cz = min(iz, nx - 1);
-      px = axis_sm ? sAxis[cx] : __ldg(P.axis + cx);
-      py = axis_sm ? sAxis[cy] : __ldg(P.axis + cy);
-      pz = axis_sm ? sAxis[cz] : __ldg(P.axis + cz);
-      oidx = (((long long)qb * nx + ix) * nx + iy) * nx + iz;
-    } else {
-      const long long n = tile * kTcTile + tq;
-      valid = n < P.total;
-      const long long nn = valid ? n : 0;
-      px = __ldg(P.p + nn * 3 + 0);
-      py = __ldg(P.p + nn * 3 + 1);
-      pz = __ldg(P.p + nn * 3 + 2);
-      qb = (int)(nn / P.N);
-      oidx = nn;
-    }
-    if (!valid) oidx = 0;
-    TC_STAMP(13);  // tile start: coordinates loaded
+    const auto [px, py, pz, oidx, qb, valid] = tile_query(P, DENSE, tile, tq, sAxis, axis_sm, nx);
+    TC_STAMP(trace, 13);  // tile start: coordinates loaded
 
     // ---------------- gather: this thread's 16 channels of its query (+ of its c_img row): operands of step 0 ----------------
     if (P.has_c || cimg) {
@@ -627,78 +473,45 @@ __global__ void __launch_bounds__(kTc2Threads, 1) decoder_tc2_kernel(const __gri
       bool sep_done = false;
       if (sep_cfg) {
         const int R = P.Rg;
-        const float tx = unnormalize(norm3d(px, P.nc), R), ty = unnormalize(norm3d(py, P.nc), R);
-        const float tz = unnormalize(norm3d(pz, P.nc), R);
-        const float flx = floorf(tx), fly = floorf(ty), flz = floorf(tz);
-        const int x0 = (int)flx, y0 = (int)fly, z0 = (int)flz;
-        const float fx1 = tx - flx, fx0 = (flx + 1.0f) - tx, fy1 = ty - fly, fy0 = (fly + 1.0f) - ty;
-        const float fz1 = tz - flz, fz0 = (flz + 1.0f) - tz;
-        const int zmin = __shfl_sync(kFull, z0, 0);
-        const int zmax = min(__shfl_sync(kFull, z0, 31) + 1, R - 1);
-        const int nz = zmax - zmin + 1;
-        if (nz <= 32) {
-          const int dx = (x0 + 1 < R) ? 8 : 0, dy = (y0 + 1 < R) ? R * 8 : 0;
-          const float w00 = fx0 * fy0, w01 = fx1 * fy0, w10 = fx0 * fy1, w11 = fx1 * fy1;
-          const float4* col = reinterpret_cast<const float4*>(P.grid) + (size_t)qb * R * R * R * 8 +
-                              ((size_t)y0 * R + x0) * 8 + 4 * hv + sub;
+        const SepGather sg = sep_gather_setup(P, px, py, pz, qb, 4 * hv + sub);
+        if (sg.nz <= 32) {
 #pragma unroll 2
-          for (int zb = 0; zb < nz; zb += 8) {
+          for (int zb = 0; zb < sg.nz; zb += 8) {
             const int zrow = zb + zr;
-            if (zrow < nz) {
-              const float4* p = col + (size_t)(zmin + zrow) * R * R * 8;
-              const float4 v00 = __ldg(p), v01 = __ldg(p + dx), v10 = __ldg(p + dy), v11 = __ldg(p + dy + dx);
+            if (zrow < sg.nz) {
+              const float4* p = sg.col + (size_t)(sg.zmin + zrow) * R * R * 8;
+              const float4 v00 = __ldg(p), v01 = __ldg(p + sg.dx), v10 = __ldg(p + sg.dy), v11 = __ldg(p + sg.dy + sg.dx);
               float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
-              a = f4_fma(w00, v00, a);
-              a = f4_fma(w01, v01, a);
-              a = f4_fma(w10, v10, a);
-              a = f4_fma(w11, v11, a);
+              a = f4_fma(sg.w00, v00, a);
+              a = f4_fma(sg.w01, v01, a);
+              a = f4_fma(sg.w10, v10, a);
+              a = f4_fma(sg.w11, v11, a);
               *reinterpret_cast<float4*>(stage + zrow * kTc2Stage + 4 * sub) = a;
             }
           }
           __syncwarp();
-          const float* r0 = stage + (z0 - zmin) * kTc2Stage;
-          const float* r1 = stage + (min(z0 + 1, R - 1) - zmin) * kTc2Stage;
+          const float* r0 = stage + (sg.z0 - sg.zmin) * kTc2Stage;
+          const float* r1 = stage + (min(sg.z0 + 1, R - 1) - sg.zmin) * kTc2Stage;
 #pragma unroll
           for (int j = 0; j < 4; ++j) {
             const float4 a = *reinterpret_cast<const float4*>(r0 + 4 * j);
             const float4 b = *reinterpret_cast<const float4*>(r1 + 4 * j);
-            cv[4 * j + 0] = fmaf(b.x, fz1, a.x * fz0);
-            cv[4 * j + 1] = fmaf(b.y, fz1, a.y * fz0);
-            cv[4 * j + 2] = fmaf(b.z, fz1, a.z * fz0);
-            cv[4 * j + 3] = fmaf(b.w, fz1, a.w * fz0);
+            cv[4 * j + 0] = fmaf(b.x, sg.fz1, a.x * sg.fz0);
+            cv[4 * j + 1] = fmaf(b.y, sg.fz1, a.y * sg.fz0);
+            cv[4 * j + 2] = fmaf(b.z, sg.fz1, a.z * sg.fz0);
+            cv[4 * j + 3] = fmaf(b.w, sg.fz1, a.w * sg.fz0);
           }
           __syncwarp();
           sep_done = true;
         }
       }
       if (!sep_done) {   // generic gather: the owner computes the taps, 4 lanes fetch a query's 16 channels
-        TapInfo tv, tp0, tp1, tp2;
-        if (P.grid) tv = tap_volume(norm3d(px, P.nc), norm3d(py, P.nc), norm3d(pz, P.nc), P.Rg, P.nearest);
-        const bool planes = P.plane[0] || P.plane[1] || P.plane[2];
-        if (planes) {
-          const float ux = norm2d(px, P.nc), uy = norm2d(py, P.nc), uz = norm2d(pz, P.nc);
-          if (P.plane[0]) tp0 = tap_plane(ux, uz, P.Rp, P.nearest);
-          if (P.plane[1]) tp1 = tap_plane(ux, uy, P.Rp, P.nearest);
-          if (P.plane[2]) tp2 = tap_plane(uy, uz, P.Rp, P.nearest);
-        }
+        const QueryTaps taps = query_taps(P, px, py, pz);
 #pragma unroll 2
         for (int it = 0; it < 4; ++it) {
           const int src = it * 8 + zr;
           const int b = __shfl_sync(kFull, qb, src);
-          float4 c = make_float4(0.f, 0.f, 0.f, 0.f);
-          if (P.grid) {
-            const int R = P.Rg;
-            const float4* vol = reinterpret_cast<const float4*>(P.grid) + (size_t)b * R * R * R * 8 + 4 * hv + sub;
-            c = fetch_volume(vol, R, tap_bcast(tv, src), P.nearest);
-          }
-          if (planes) {
-            const int R = P.Rp;
-            const size_t boff = (size_t)b * R * R * 8 + 4 * hv + sub;
-            if (P.plane[0]) c = f4_add(c, fetch_plane(reinterpret_cast<const float4*>(P.plane[0]) + boff, R, tap_bcast(tp0, src), P.nearest));
-            if (P.plane[1]) c = f4_add(c, fetch_plane(reinterpret_cast<const float4*>(P.plane[1]) + boff, R, tap_bcast(tp1, src), P.nearest));
-            if (P.plane[2]) c = f4_add(c, fetch_plane(reinterpret_cast<const float4*>(P.plane[2]) + boff, R, tap_bcast(tp2, src), P.nearest));
-          }
-          *reinterpret_cast<float4*>(stage + src * kTc2Stage + 4 * sub) = c;
+          *reinterpret_cast<float4*>(stage + src * kTc2Stage + 4 * sub) = gather_taps(P, taps, src, b, 4 * hv + sub);
         }
         __syncwarp();
 #pragma unroll
@@ -708,7 +521,7 @@ __global__ void __launch_bounds__(kTc2Threads, 1) decoder_tc2_kernel(const __gri
         }
         __syncwarp();
       }
-      TC_STAMP(15);  // features of the thread's query in registers
+      TC_STAMP(trace, 15);  // features of the thread's query in registers
       split_store16<MIXED>(tC, hv, cv);
      }
       if (cimg) {   // fc_p_img(cat[p, c_img]) = fc_p_img[:, :3] p + b + W_img c_img: the last term rides in step 0
@@ -774,31 +587,31 @@ __global__ void __launch_bounds__(kTc2Threads, 1) decoder_tc2_kernel(const __gri
 
     // ---------------- residual blocks ----------------
     for (int i = 0; i < nb; ++i) {
-      TC_STAMP(1);   // ALU phase starts (accumulator already read)
+      TC_STAMP(trace, 1);   // ALU phase starts (accumulator already read)
 #pragma unroll
       for (int j = 0; j < 16; ++j) x[j] = fmaxf(net[j], 0.f);
       split_store16<MIXED>(tX, hv, x);
-      TC_STAMP(2);   // operands computed, tcgen05.st issued
+      TC_STAMP(trace, 2);   // operands computed, tcgen05.st issued
       tc_wait_st();
       tc_fence_before();
-      TC_STAMP(3);   // stores complete
+      TC_STAMP(trace, 3);   // stores complete
       group_sync2();
-      TC_STAMP(4);   // group barrier passed
+      TC_STAMP(trace, 4);   // group barrier passed
       if (wq == (step & 7) && elect_one()) {     // D = relu(net)*W0_i + ones*b0_i
         tc_fence_after();
         issue_product(mD, mX, wsm + 4 * VTACO_DEC_TC_MAT(kTcMode, 3 * i + 1), 0, n_prod);
         tc_mma_ts(mD, mOnes, make_bdesc(bsm + (2 * i + 1) * kKBlkBytes), 1);
         tc_commit(bar);
-        TC_STAMP(20);  // issuer only: 13 MMAs + commit issued
+        TC_STAMP(trace, 20);  // issuer only: 13 MMAs + commit issued
       }
       ++step;
-      TC_STAMP(5);   // (issuing warp: MMAs issued)
+      TC_STAMP(trace, 5);   // (issuing warp: MMAs issued)
       mbar_wait(bar, ph); ph ^= 1;
-      TC_STAMP(6);   // MMAs complete
+      TC_STAMP(trace, 6);   // MMAs complete
       tc_fence_after();
       tmem_ld16(tD + ch0, r);
       tc_wait_ld();
-      TC_STAMP(7);   // accumulator in registers
+      TC_STAMP(trace, 7);   // accumulator in registers
 #pragma unroll
       for (int j = 0; j < 16; ++j) x[j] = fmaxf(__uint_as_float(r[j]), 0.f);
       split_store16<MIXED>(tX, hv, x);
@@ -821,7 +634,7 @@ __global__ void __launch_bounds__(kTc2Threads, 1) decoder_tc2_kernel(const __gri
       for (int j = 0; j < 16; ++j) net[j] += __uint_as_float(r[j]);
     }
 
-    TC_STAMP(19);    // blocks done
+    TC_STAMP(trace, 19);    // blocks done
     // ---------------- heads: partial dot products of the two halves, combined through shared memory ----------------
     {
       const float* Wo = sSmall + 128;
@@ -848,121 +661,69 @@ __global__ void __launch_bounds__(kTc2Threads, 1) decoder_tc2_kernel(const __gri
     }
   }
 
-  if (P.minmax_key) {
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) {
-      vmin = fminf(vmin, __shfl_xor_sync(kFull, vmin, d));
-      vmax = fmaxf(vmax, __shfl_xor_sync(kFull, vmax, d));
-    }
-    if (lane == 0 && vmin <= vmax) {
-      atomicMin(P.minmax_key, float_to_key(vmin));
-      atomicMax(P.minmax_key + 1, float_to_key(vmax));
-    }
+  flush_minmax(P, vmin, vmax, lane);
+  tmem_free_all(tmem_base, warp);
+}
+
+int tc_trace_begin(long long** trace, cudaStream_t stream) {
+  static const bool want = getenv("VTACO_TC_TRACE") != nullptr;
+  *trace = nullptr;
+  if (want) {
+    VTACO_CUDA_CHECK(cudaMalloc(trace, kTraceSlots * sizeof(long long)));
+    VTACO_CUDA_CHECK(cudaMemsetAsync(*trace, 0, kTraceSlots * sizeof(long long), stream));
   }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
+  return VTACO_OK;
+}
+
+int tc_trace_end(long long* trace, const char* tag, cudaStream_t stream) {
+  if (!trace) return VTACO_OK;
+  long long h[kTraceSlots];
+  VTACO_CUDA_CHECK(cudaStreamSynchronize(stream));
+  VTACO_CUDA_CHECK(cudaMemcpy(h, trace, sizeof(h), cudaMemcpyDeviceToHost));
+  cudaFree(trace);
+  double sum[32][32] = {};
+  long long cnt[32][32] = {};
+  for (int i = 1; i < kTraceSlots && h[i]; ++i) {
+    const int a = (int)(h[i - 1] >> 56) & 31, b = (int)(h[i] >> 56) & 31;
+    const long long d = (h[i] & 0x00ffffffffffffffll) - (h[i - 1] & 0x00ffffffffffffffll);
+    if (d >= 0 && d < 1000000) { sum[a][b] += (double)d; cnt[a][b]++; }
   }
+  for (int a = 0; a < 32; ++a)
+    for (int b = 0; b < 32; ++b)
+      if (cnt[a][b]) fprintf(stderr, "[vtaco %s trace] %d -> %d : %8.0f cycles (n=%lld)\n", tag, a, b, sum[a][b] / cnt[a][b], cnt[a][b]);
+  return VTACO_OK;
 }
 
 int launch_decoder_tc(DecParams P, bool dense, const float* wtc, cudaStream_t stream) {
   if (!wtc) return VTACO_ERR_INVALID_ARG;
-  if (dense) {
-    P.t_xend = P.x1;
-    P.t_nbz = (P.nx + 31) / 32;
-    P.t_nby = (P.nx + 1) / 2;
-    P.t_nbx = (P.x1 - P.x0 + 1) / 2;
-    P.n_tiles = (long long)P.B * P.t_nbx * P.t_nby * P.t_nbz;
-  } else {
-    P.n_tiles = (P.total + kTcTile - 1) / kTcTile;
-  }
-  if (P.n_tiles >= (1ll << 31)) return VTACO_ERR_UNSUPPORTED;
+  if (const int e = set_tc_tiles(P, dense)) return e;
   const bool mixed = (P.tc_products == 2);
-  if (P.tc_split == 2) {   // two threads per query
-    const Tc2Smem L2 = tc2_smem_layout(P.n_blocks);
-    if (L2.total > 227 * 1024) return VTACO_ERR_UNSUPPORTED;
-    using Kernel2 = void (*)(DecParams, const float*, long long*);
-    const Kernel2 k2 = dense ? (mixed ? (Kernel2)decoder_tc2_kernel<true, true> : (Kernel2)decoder_tc2_kernel<true, false>)
-                             : (mixed ? (Kernel2)decoder_tc2_kernel<false, true> : (Kernel2)decoder_tc2_kernel<false, false>);
-    static std::atomic<size_t> configured2[4][64];   // idempotent opt-in cache, safe across host threads
-    int dev2 = 0;
-    VTACO_CUDA_CHECK(cudaGetDevice(&dev2));
-    const int ki2 = (dense ? 2 : 0) + (mixed ? 1 : 0);
-    if (configured2[ki2][dev2 & 63].load(std::memory_order_relaxed) < (size_t)L2.total) {
-      VTACO_CUDA_CHECK(cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, L2.total));
-      configured2[ki2][dev2 & 63].store(L2.total, std::memory_order_relaxed);
-    }
-    long long grid2 = (P.n_tiles + kTcGroups - 1) / kTcGroups;
-    if (grid2 > num_sms()) grid2 = num_sms();
-    long long* trace2 = nullptr;
-    static const bool want_trace2 = getenv("VTACO_TC_TRACE") != nullptr;
-    if (want_trace2) {
-      VTACO_CUDA_CHECK(cudaMalloc(&trace2, 4096 * sizeof(long long)));
-      VTACO_CUDA_CHECK(cudaMemsetAsync(trace2, 0, 4096 * sizeof(long long), stream));
-    }
-    k2<<<(unsigned)grid2, kTc2Threads, L2.total, stream>>>(P, wtc, trace2);
-    VTACO_LAUNCH_CHECK();
-    if (trace2) {   // debug: average cycles between consecutive stamps of warp 0 / block 0, per (from -> to) slot pair
-      static long long h2[4096];
-      VTACO_CUDA_CHECK(cudaStreamSynchronize(stream));
-      VTACO_CUDA_CHECK(cudaMemcpy(h2, trace2, sizeof(h2), cudaMemcpyDeviceToHost));
-      cudaFree(trace2);
-      static double sum2[32][32];
-      static long long cnt2[32][32];
-      for (int a = 0; a < 32; ++a) for (int b = 0; b < 32; ++b) { sum2[a][b] = 0; cnt2[a][b] = 0; }
-      for (int i = 1; i < 4096 && h2[i]; ++i) {
-        const int a = (int)(h2[i - 1] >> 56) & 31, b = (int)(h2[i] >> 56) & 31;
-        const long long d = (h2[i] & 0x00ffffffffffffffll) - (h2[i - 1] & 0x00ffffffffffffffll);
-        if (d >= 0 && d < 1000000) { sum2[a][b] += (double)d; cnt2[a][b]++; }
-      }
-      for (int a = 0; a < 32; ++a)
-        for (int b = 0; b < 32; ++b)
-          if (cnt2[a][b]) fprintf(stderr, "[vtaco tc2 trace] %d -> %d : %8.0f cycles (n=%lld)\n", a, b, sum2[a][b] / cnt2[a][b], cnt2[a][b]);
-    }
-    return VTACO_OK;
-  }
-  const TcSmem L = tc_smem_layout(P.n_blocks);
-  if (L.total > 227 * 1024) return VTACO_ERR_UNSUPPORTED;
   using Kernel = void (*)(DecParams, const float*, long long*);
-  const Kernel kernel = dense ? (mixed ? (Kernel)decoder_tc_kernel<true, true> : (Kernel)decoder_tc_kernel<true, false>)
-                              : (mixed ? (Kernel)decoder_tc_kernel<false, true> : (Kernel)decoder_tc_kernel<false, false>);
-  static std::atomic<size_t> configured[4][64];
-  int dev = 0;
-  VTACO_CUDA_CHECK(cudaGetDevice(&dev));
-  const int ki = (dense ? 2 : 0) + (mixed ? 1 : 0);
-  if (configured[ki][dev & 63].load(std::memory_order_relaxed) < (size_t)L.total) {
-    VTACO_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, L.total));
-    configured[ki][dev & 63].store(L.total, std::memory_order_relaxed);
+  Kernel k;
+  int threads, smem;
+  const char* tag;
+  if (P.tc_split == 2) {   // two threads per query
+    k = dense ? (mixed ? decoder_tc2_kernel<true, true> : decoder_tc2_kernel<true, false>)
+              : (mixed ? decoder_tc2_kernel<false, true> : decoder_tc2_kernel<false, false>);
+    threads = kTc2Threads;
+    smem = tc2_smem_layout(P.n_blocks).total;
+    tag = "tc2";
+  } else {
+    k = dense ? (mixed ? decoder_tc_kernel<true, true> : decoder_tc_kernel<true, false>)
+              : (mixed ? decoder_tc_kernel<false, true> : decoder_tc_kernel<false, false>);
+    threads = kTcThreads;
+    smem = tc_smem_layout(P.n_blocks).total;
+    tag = "tc";
   }
+  if (smem > 227 * 1024) return VTACO_ERR_UNSUPPORTED;
+  VTACO_CUDA_CHECK(smem_opt_in((const void*)k, smem));
   long long grid = (P.n_tiles + kTcGroups - 1) / kTcGroups;
   if (grid > num_sms()) grid = num_sms();
-  long long* trace = nullptr;
-  static const bool want_trace = getenv("VTACO_TC_TRACE") != nullptr;
-  if (want_trace) {
-    VTACO_CUDA_CHECK(cudaMalloc(&trace, 4096 * sizeof(long long)));
-    VTACO_CUDA_CHECK(cudaMemsetAsync(trace, 0, 4096 * sizeof(long long), stream));
-  }
-  kernel<<<(unsigned)grid, kTcThreads, L.total, stream>>>(P, wtc, trace);
+  long long* trace;
+  if (const int e = tc_trace_begin(&trace, stream)) return e;
+  k<<<(unsigned)grid, threads, smem, stream>>>(P, wtc, trace);
   VTACO_LAUNCH_CHECK();
-  if (trace) {   // debug: average cycles between consecutive stamps, per (from -> to) slot pair
-    static long long h[4096];
-    VTACO_CUDA_CHECK(cudaStreamSynchronize(stream));
-    VTACO_CUDA_CHECK(cudaMemcpy(h, trace, sizeof(h), cudaMemcpyDeviceToHost));
-    cudaFree(trace);
-    static double sum[32][32];
-    static long long cnt[32][32];
-    for (int a = 0; a < 32; ++a) for (int b = 0; b < 32; ++b) { sum[a][b] = 0; cnt[a][b] = 0; }
-    for (int i = 1; i < 4096 && h[i]; ++i) {
-      const int a = (int)(h[i - 1] >> 56) & 31, b = (int)(h[i] >> 56) & 31;
-      const long long d = (h[i] & 0x00ffffffffffffffll) - (h[i - 1] & 0x00ffffffffffffffll);
-      if (d >= 0 && d < 1000000) { sum[a][b] += (double)d; cnt[a][b]++; }
-    }
-    for (int a = 0; a < 32; ++a)
-      for (int b = 0; b < 32; ++b)
-        if (cnt[a][b]) fprintf(stderr, "[vtaco tc trace] %d -> %d : %8.0f cycles (n=%lld)\n", a, b, sum[a][b] / cnt[a][b], cnt[a][b]);
-  }
-  return VTACO_OK;
+  return tc_trace_end(trace, tag, stream);
 }
 
 }  // namespace vtaco

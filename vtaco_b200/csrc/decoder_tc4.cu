@@ -23,8 +23,6 @@
 // Two threads per query, the separable dense gather, the step structure and the elected issuer rotating over
 // the warps of a group are decoder_tc2_kernel's.
 #include "decoder_tc_common.cuh"
-#include <cstdio>
-#include <cstdlib>
 
 namespace vtaco {
 
@@ -123,12 +121,6 @@ __device__ __forceinline__ void issue_product_t4(uint32_t d, uint32_t a_hi, uint
     tc_mma_ts(d, a_hi + 8 * kk, bdesc_at(wlo, desc_units(VTACO_DEC_TC_SUB_HI) + kk * kKBlkUnits), 1);
 }
 
-#define T4_STAMP(slot)                                                            \
-  do {                                                                            \
-    if (TRACE && blockIdx.x == 0 && warp == 0 && lane == 0 && trace_n < 4096)     \
-      trace[trace_n++] = ((long long)(slot) << 56) | (clock64() & 0x00ffffffffffffffll); \
-  } while (0)
-
 // NB > 0: the network depth as a compile-time constant (the shipped 5): the block loop is unrolled and the operand
 // descriptors of every step are base + immediate
 template <bool DENSE, bool TRACE, int NB>
@@ -199,29 +191,10 @@ __global__ void __launch_bounds__(kT4Threads, 1) decoder_tc4_kernel(const __grid
   const bool axis_sm = DENSE && nx <= kT4MaxAxis;
   if (axis_sm)
     for (int i = tid; i < nx; i += kT4Threads) sAxis[i] = __ldg(P.axis + i);
-  if (P.n_tips > 0) {
-    for (int o = tid; o < P.n_tips * 32; o += kT4Threads) {
-      const int f = o >> 5, j = o & 31;
-      float a = 0.f;
-      for (int k = 0; k < 32; ++k)
-        a = fmaf(__ldg(P.weights + VTACO_DEC_OFF_WIMG + k * 32 + j), __ldg(P.tip_feat + f * 32 + k), a);
-      sTip[o] = a;
-    }
-  }
+  load_tips(sTip, P, tid, kT4Threads);
   if (tid < (kT4Threads / 32) * 2) sMM[tid] = (tid & 1) ? INT32_MIN : INT32_MAX;
-  if (tid == 0) {
-    for (int i = 0; i < kT4Groups; ++i) mbar_init(smem_u32(sBars + i), 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(sTmem)), "r"(512)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = __shfl_sync(kFull, *sTmem, 0);
+  init_group_bars(sBars, kT4Groups, tid);
+  const uint32_t tmem_base = tmem_alloc_all(sTmem, warp);
   const uint32_t tbase = tmem_base + ((uint32_t)(32 * lq) << 16) + (uint32_t)(g * kT4Cols);
   const uint32_t tC = tbase, tX = tbase + 48, tD = tbase + 96;
   const uint32_t mbase = tmem_base + (uint32_t)(g * kT4Cols);
@@ -296,14 +269,14 @@ __global__ void __launch_bounds__(kT4Threads, 1) decoder_tc4_kernel(const __grid
       qb = (int)(nn / (int)P.N);
       oidx = valid ? n : -1;
     }
-    T4_STAMP(13);  // tile start: coordinates loaded
+    TC_STAMP(TRACE, 13);  // tile start: coordinates loaded
 
     // ---------------- gather: this thread's 16 channels of its query (+ of its c_img row): operands of step 0 ----------------
     {
       if (P.has_c) {
         bool sep_done = false;
         if (sep_cfg) {
-          // separable dense gather (see decoder_tc.cu): the warp is one z-run at fixed (x, y); the 4
+          // separable dense gather (see SepGather): the warp is one z-run at fixed (x, y); the 4
           // (x,y) corners are reduced once per needed z-row into shared memory, then each thread
           // lerps its two z-rows
           const int R = P.Rg;
@@ -352,7 +325,7 @@ __global__ void __launch_bounds__(kT4Threads, 1) decoder_tc4_kernel(const __grid
               cv[4 * j + 0] = c0.x; cv[4 * j + 1] = c0.y; cv[4 * j + 2] = c1.x; cv[4 * j + 3] = c1.y;
             }
             __syncwarp();
-            T4_STAMP(15);  // features of the thread's query in registers
+            TC_STAMP(TRACE, 15);  // features of the thread's query in registers
             split_store_t4(tC, hv, cv);
             sep_done = true;
           }
@@ -501,7 +474,7 @@ __global__ void __launch_bounds__(kT4Threads, 1) decoder_tc4_kernel(const __grid
     uint32_t r[16];
 #pragma unroll
     for (int i = 0; i < (NB > 0 ? NB : nb); ++i) {
-      T4_STAMP(1);   // ALU phase starts (accumulator already read)
+      TC_STAMP(TRACE, 1);   // ALU phase starts (accumulator already read)
       {
         float y[16];
 #pragma unroll
@@ -511,26 +484,26 @@ __global__ void __launch_bounds__(kT4Threads, 1) decoder_tc4_kernel(const __grid
         }
         split_store_t4(tX, hv, y);
       }
-      T4_STAMP(2);   // operands computed, tcgen05.st issued
+      TC_STAMP(TRACE, 2);   // operands computed, tcgen05.st issued
       tc_wait_st();
       tc_fence_before();
-      T4_STAMP(3);   // stores complete
+      TC_STAMP(TRACE, 3);   // stores complete
       group_sync();
-      T4_STAMP(4);   // group barrier passed
+      TC_STAMP(TRACE, 4);   // group barrier passed
       if (wq == (step & 7) && elect_one()) {     // D = relu(net)*W0_i
         tc_fence_after();
         issue_product_t4(mD, mX, wlo0 + (uint32_t)(3 * i + 1) * kMatUnits, 1);   // D already holds b0_i
         tc_commit(bar);
-        T4_STAMP(20);  // issuer only: MMAs + commit issued
+        TC_STAMP(TRACE, 20);  // issuer only: MMAs + commit issued
       }
       ++step;
-      T4_STAMP(5);
+      TC_STAMP(TRACE, 5);
       mma_wait();
-      T4_STAMP(6);   // MMAs complete
+      TC_STAMP(TRACE, 6);   // MMAs complete
       tc_fence_after();
       tmem_ld16(tD + ch0, r);
       tc_wait_ld();
-      T4_STAMP(7);   // accumulator in registers
+      TC_STAMP(TRACE, 7);   // accumulator in registers
       {                                           // h = relu(D)   (D = b0_i + relu(net) W0_i)
         float y[16];
 #pragma unroll
@@ -564,7 +537,7 @@ __global__ void __launch_bounds__(kT4Threads, 1) decoder_tc4_kernel(const __grid
       if (i + 1 < nb) store_bias16(tD + ch0, sBias + (2 * i + 3) * VTACO_DEC_TC_BVEC_FLOATS + ch0);   // b0_{i+1} for the next W0 step
     }
 
-    T4_STAMP(19);    // blocks done
+    TC_STAMP(TRACE, 19);    // blocks done
     // ---------------- heads: partial dot products of the two halves, combined through shared memory ----------------
     {
       const float* Wo = sSmall + 128;
@@ -615,71 +588,27 @@ __global__ void __launch_bounds__(kT4Threads, 1) decoder_tc4_kernel(const __grid
     atomicMax(P.minmax_key + 1, sMM[2 * warp + 1]);
   }
   if (w_tma && tid == 0) mbar_wait(wbar, 0);        // a group without tiles never waited: no bulk copy may outlive the CTA
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-  }
+  tmem_free_all(tmem_base, warp);
 }
-
-int tc4_smem_bytes(int n_blocks) { return tc4_smem_layout(n_blocks).total; }
 
 int launch_decoder_tc4(DecParams P, bool dense, const float* wtc, cudaStream_t stream) {
   if (!wtc) return VTACO_ERR_INVALID_ARG;
-  if (dense) {
-    P.t_xend = P.x1;
-    P.t_nbz = (P.nx + 31) / 32;
-    P.t_nby = (P.nx + 1) / 2;
-    P.t_nbx = (P.x1 - P.x0 + 1) / 2;
-    P.n_tiles = (long long)P.B * P.t_nbx * P.t_nby * P.t_nbz;
-  } else {
-    P.n_tiles = (P.total + kTcTile - 1) / kTcTile;
-  }
-  if (P.n_tiles >= (1ll << 31)) return VTACO_ERR_UNSUPPORTED;
+  if (const int e = set_tc_tiles(P, dense)) return e;
   if ((dense ? (long long)P.B * P.nx * P.nx * P.nx : P.total) >= (1ll << 31)) return VTACO_ERR_UNSUPPORTED;   // 32-bit output index
   const Tc4Smem L = tc4_smem_layout(P.n_blocks);
   if (L.total > 227 * 1024) return VTACO_ERR_UNSUPPORTED;
+  long long* trace;
+  if (const int e = tc_trace_begin(&trace, stream)) return e;
   using Kernel = void (*)(DecParams, const float*, long long*);
-  static const bool want_trace = getenv("VTACO_TC_TRACE") != nullptr;
-  const bool nb5 = P.n_blocks == 5;
-  const Kernel k = want_trace ? (dense ? (Kernel)decoder_tc4_kernel<true, true, 0> : (Kernel)decoder_tc4_kernel<false, true, 0>)
-                   : nb5 ? (dense ? (Kernel)decoder_tc4_kernel<true, false, 5> : (Kernel)decoder_tc4_kernel<false, false, 5>)
-                         : (dense ? (Kernel)decoder_tc4_kernel<true, false, 0> : (Kernel)decoder_tc4_kernel<false, false, 0>);
-  static std::atomic<size_t> configured[8][64];   // idempotent opt-in cache, safe across host threads
-  int dev = 0;
-  VTACO_CUDA_CHECK(cudaGetDevice(&dev));
-  const int ki = (dense ? 1 : 0) + (want_trace ? 2 : 0) + ((nb5 && !want_trace) ? 4 : 0);
-  if (configured[ki][dev & 63].load(std::memory_order_relaxed) < (size_t)L.total) {
-    VTACO_CUDA_CHECK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, L.total));
-    configured[ki][dev & 63].store(L.total, std::memory_order_relaxed);
-  }
+  const Kernel k = trace ? (dense ? decoder_tc4_kernel<true, true, 0> : decoder_tc4_kernel<false, true, 0>)
+                   : P.n_blocks == 5 ? (dense ? decoder_tc4_kernel<true, false, 5> : decoder_tc4_kernel<false, false, 5>)
+                                     : (dense ? decoder_tc4_kernel<true, false, 0> : decoder_tc4_kernel<false, false, 0>);
+  VTACO_CUDA_CHECK(smem_opt_in((const void*)k, L.total));
   long long grid = (P.n_tiles + kT4Groups - 1) / kT4Groups;
   if (grid > num_sms()) grid = num_sms();
-  long long* trace = nullptr;
-  if (want_trace) {
-    VTACO_CUDA_CHECK(cudaMalloc(&trace, 4096 * sizeof(long long)));
-    VTACO_CUDA_CHECK(cudaMemsetAsync(trace, 0, 4096 * sizeof(long long), stream));
-  }
   k<<<(unsigned)grid, kT4Threads, L.total, stream>>>(P, wtc, trace);
   VTACO_LAUNCH_CHECK();
-  if (trace) {   // debug: average cycles between consecutive stamps of warp 0 / block 0, per (from -> to) slot pair
-    static long long h[4096];
-    VTACO_CUDA_CHECK(cudaStreamSynchronize(stream));
-    VTACO_CUDA_CHECK(cudaMemcpy(h, trace, sizeof(h), cudaMemcpyDeviceToHost));
-    cudaFree(trace);
-    static double sum[32][32];
-    static long long cnt[32][32];
-    for (int a = 0; a < 32; ++a) for (int b = 0; b < 32; ++b) { sum[a][b] = 0; cnt[a][b] = 0; }
-    for (int i = 1; i < 4096 && h[i]; ++i) {
-      const int a = (int)(h[i - 1] >> 56) & 31, b = (int)(h[i] >> 56) & 31;
-      const long long d = (h[i] & 0x00ffffffffffffffll) - (h[i - 1] & 0x00ffffffffffffffll);
-      if (d >= 0 && d < 1000000) { sum[a][b] += (double)d; cnt[a][b]++; }
-    }
-    for (int a = 0; a < 32; ++a)
-      for (int b = 0; b < 32; ++b)
-        if (cnt[a][b]) fprintf(stderr, "[vtaco tc4 trace] %d -> %d : %8.0f cycles (n=%lld)\n", a, b, sum[a][b] / cnt[a][b], cnt[a][b]);
-  }
-  return VTACO_OK;
+  return tc_trace_end(trace, "tc4", stream);
 }
 
 }  // namespace vtaco

@@ -1,4 +1,4 @@
-// tcgen05 / TMEM PTX wrappers and the gather helpers shared by the tensor-core decoder kernels
+// tcgen05 / TMEM PTX wrappers and the gather, set-up and tracing helpers shared by the tensor-core decoder kernels
 // (decoder_tc.cu: 3 tiles per SM, 3xTF32; decoder_tc4.cu: 4 tiles per SM, TF32 + BF16 residual).
 #pragma once
 #include "decoder_common.cuh"
@@ -248,6 +248,182 @@ __device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t (&r)[8])
   asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%8], {%0,%1,%2,%3,%4,%5,%6,%7};" ::"r"(r[0]), "r"(r[1]),
                "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(taddr)
                : "memory");
+}
+
+// ---------------------------------------------------------------------------------------
+// Per-query helpers of the tcgen05 kernels
+// ---------------------------------------------------------------------------------------
+// Taps of one query in every feature tensor, computed by the thread that owns the query
+struct QueryTaps { TapInfo v, p0, p1, p2; bool planes; };
+__device__ __forceinline__ QueryTaps query_taps(const DecParams& P, float px, float py, float pz) {
+  QueryTaps t;
+  if (P.grid) t.v = tap_volume(norm3d(px, P.nc), norm3d(py, P.nc), norm3d(pz, P.nc), P.Rg, P.nearest);
+  t.planes = P.plane[0] || P.plane[1] || P.plane[2];
+  if (t.planes) {
+    const float ux = norm2d(px, P.nc), uy = norm2d(py, P.nc), uz = norm2d(pz, P.nc);
+    if (P.plane[0]) t.p0 = tap_plane(ux, uz, P.Rp, P.nearest);
+    if (P.plane[1]) t.p1 = tap_plane(ux, uy, P.Rp, P.nearest);
+    if (P.plane[2]) t.p2 = tap_plane(uy, uz, P.Rp, P.nearest);
+  }
+  return t;
+}
+// c of the query whose taps lane `src` holds, summed over the grid and the planes: float4 `ch` (channels
+// 4*ch .. 4*ch+3) of sample b
+__device__ __forceinline__ float4 gather_taps(const DecParams& P, QueryTaps t, int src, int b, int ch) {
+  float4 c = make_float4(0.f, 0.f, 0.f, 0.f);
+  if (P.grid) {
+    const int R = P.Rg;
+    const float4* vol = reinterpret_cast<const float4*>(P.grid) + (size_t)b * R * R * R * 8 + ch;
+    c = fetch_volume(vol, R, tap_bcast(t.v, src), P.nearest);
+  }
+  if (t.planes) {
+    const int R = P.Rp;
+    const size_t boff = (size_t)b * R * R * 8 + ch;
+    if (P.plane[0]) c = f4_add(c, fetch_plane(reinterpret_cast<const float4*>(P.plane[0]) + boff, R, tap_bcast(t.p0, src), P.nearest));
+    if (P.plane[1]) c = f4_add(c, fetch_plane(reinterpret_cast<const float4*>(P.plane[1]) + boff, R, tap_bcast(t.p1, src), P.nearest));
+    if (P.plane[2]) c = f4_add(c, fetch_plane(reinterpret_cast<const float4*>(P.plane[2]) + boff, R, tap_bcast(t.p2, src), P.nearest));
+  }
+  return c;
+}
+
+// Separable dense gather (grid only, bilinear): a warp is one z-run of lattice points at fixed (x, y), so the
+// (x,y)-bilinear part of the trilinear sample is shared by the run.  The kernels reduce the 4 (x,y) corners once
+// per needed z-row into shared memory, then every thread lerps its two z-rows.
+struct SepGather {
+  int z0, zmin, nz;        // the query's lower z-row; the run needs rows [zmin, zmin + nz)
+  int dx, dy;              // float4 offsets of the x+1 / y+1 corners (0 where clamped: their weight is 0)
+  float w00, w01, w10, w11, fz0, fz1;
+  const float4* col;       // corner (x0, y0) at z = 0: float4 `ch` of the query's sample
+};
+__device__ __forceinline__ SepGather sep_gather_setup(const DecParams& P, float px, float py, float pz, int qb, int ch) {
+  const int R = P.Rg;
+  const float tx = unnormalize(norm3d(px, P.nc), R), ty = unnormalize(norm3d(py, P.nc), R);
+  const float tz = unnormalize(norm3d(pz, P.nc), R);
+  const float flx = floorf(tx), fly = floorf(ty), flz = floorf(tz);
+  const int x0 = (int)flx, y0 = (int)fly, z0 = (int)flz;
+  const float fx1 = tx - flx, fx0 = (flx + 1.0f) - tx, fy1 = ty - fly, fy0 = (fly + 1.0f) - ty;
+  SepGather s;
+  s.z0 = z0;
+  s.fz1 = tz - flz; s.fz0 = (flz + 1.0f) - tz;
+  s.zmin = __shfl_sync(kFull, z0, 0);
+  const int zmax = min(__shfl_sync(kFull, z0, 31) + 1, R - 1);
+  s.nz = zmax - s.zmin + 1;
+  s.dx = (x0 + 1 < R) ? 8 : 0; s.dy = (y0 + 1 < R) ? R * 8 : 0;
+  s.w00 = fx0 * fy0; s.w01 = fx1 * fy0; s.w10 = fx0 * fy1; s.w11 = fx1 * fy1;
+  s.col = reinterpret_cast<const float4*>(P.grid) + (size_t)qb * R * R * R * 8 + ((size_t)y0 * R + x0) * 8 + ch;
+  return s;
+}
+
+// Query tq of a tile.  Dense: 2 (x) x 2 (y) x 32 (z) bricks, so a warp is one z-run and its 32 logits are one
+// 128-byte store; the axis is read from sAxis where the kernel caches it (axis_sm).  Flat: 128 consecutive queries.
+// A padding query (valid = false) reads clamped coordinates and has oidx 0.
+struct TileQuery { float px, py, pz; long long oidx; int qb; bool valid; };
+__device__ __forceinline__ TileQuery tile_query(const DecParams& P, bool dense, long long tile, int tq,
+                                                const float* sAxis, bool axis_sm, int nx) {
+  TileQuery q;
+  if (dense) {
+    unsigned t = (unsigned)tile;                        // n_tiles < 2^31 (checked at launch)
+    const int bz = (int)(t % (unsigned)P.t_nbz); t /= (unsigned)P.t_nbz;
+    const int by = (int)(t % (unsigned)P.t_nby); t /= (unsigned)P.t_nby;
+    const int bx = (int)(t % (unsigned)P.t_nbx);
+    q.qb = (int)(t / (unsigned)P.t_nbx);
+    const int ix = P.x0 + bx * 2 + (tq >> 6), iy = by * 2 + ((tq >> 5) & 1), iz = bz * 32 + (tq & 31);
+    q.valid = (ix < P.t_xend) && (iy < nx) && (iz < nx);
+    const int cx = min(ix, nx - 1), cy = min(iy, nx - 1), cz = min(iz, nx - 1);
+    q.px = axis_sm ? sAxis[cx] : __ldg(P.axis + cx);
+    q.py = axis_sm ? sAxis[cy] : __ldg(P.axis + cy);
+    q.pz = axis_sm ? sAxis[cz] : __ldg(P.axis + cz);
+    q.oidx = (((long long)q.qb * nx + ix) * nx + iy) * nx + iz;
+  } else {
+    const long long n = tile * kTcTile + tq;
+    q.valid = n < P.total;
+    const long long nn = q.valid ? n : 0;
+    q.px = __ldg(P.p + nn * 3 + 0);
+    q.py = __ldg(P.p + nn * 3 + 1);
+    q.pz = __ldg(P.p + nn * 3 + 2);
+    q.qb = (int)(nn / P.N);
+    q.oidx = nn;
+  }
+  if (!q.valid) q.oidx = 0;
+  return q;
+}
+
+// ---------------------------------------------------------------------------------------
+// CTA set-up and teardown of the tcgen05 kernels (nthreads: the CTA's thread count)
+// ---------------------------------------------------------------------------------------
+// sSmall[0, 128): fc_p (or fc_p_img[:, :3]) as Wp[3][32], bp[32]; sSmall[128, ...): the packed tail (fc_out, fc_contact)
+__device__ __forceinline__ void load_small(float* sSmall, const DecParams& P, int nb, int tid, int nthreads) {
+  for (int i = tid; i < 128; i += nthreads) sSmall[i] = P.weights[(P.use_img ? VTACO_DEC_OFF_WPI : VTACO_DEC_OFF_WP) + i];
+  for (int i = tid; i < VTACO_DEC_TAIL; i += nthreads)
+    sSmall[128 + i] = P.weights[VTACO_DEC_OFF_BLOCKS + nb * VTACO_DEC_BLOCK_STRIDE + i];
+}
+// sTip[f][j]: fc_p_img.weight[:, 3:] @ tip_feat[f]
+__device__ __forceinline__ void load_tips(float* sTip, const DecParams& P, int tid, int nthreads) {
+  if (P.n_tips > 0) {
+    for (int o = tid; o < P.n_tips * 32; o += nthreads) {
+      const int f = o >> 5, j = o & 31;
+      float a = 0.f;
+      for (int k = 0; k < 32; ++k)
+        a = fmaf(__ldg(P.weights + VTACO_DEC_OFF_WIMG + k * 32 + j), __ldg(P.tip_feat + f * 32 + k), a);
+      sTip[o] = a;
+    }
+  }
+}
+// one MMA-completion mbarrier per group
+__device__ __forceinline__ void init_group_bars(uint64_t* sBars, int n_groups, int tid) {
+  if (tid == 0) {
+    for (int i = 0; i < n_groups; ++i) mbar_init(smem_u32(sBars + i), 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+}
+// All 512 TMEM columns (one CTA per SM), allocated by warp 0; ends with a CTA barrier and returns the base address.
+__device__ __forceinline__ uint32_t tmem_alloc_all(uint32_t* sTmem, int warp) {
+  if (warp == 0) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(sTmem)), "r"(512)
+                 : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  return __shfl_sync(kFull, *sTmem, 0);
+}
+__device__ __forceinline__ void tmem_free_all(uint32_t tmem_base, int warp) {
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 0) {
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
+  }
+}
+
+// ---------------------------------------------------------------------------------------
+// Debug-only phase tracing (VTACO_TC_TRACE=1): clock64 stamps of warp 0 of block 0, the slot number in the top
+// byte.  `on` enables a stamp; the kernel provides trace, trace_n, warp and lane.
+// ---------------------------------------------------------------------------------------
+constexpr int kTraceSlots = 4096;
+#define TC_STAMP(on, slot)                                                             \
+  do {                                                                                 \
+    if ((on) && blockIdx.x == 0 && warp == 0 && lane == 0 && trace_n < kTraceSlots)    \
+      trace[trace_n++] = ((long long)(slot) << 56) | (clock64() & 0x00ffffffffffffffll); \
+  } while (0)
+// *trace = a zeroed stamp buffer when VTACO_TC_TRACE is set, else nullptr
+int tc_trace_begin(long long** trace, cudaStream_t stream);
+// nothing without a buffer; else waits for the kernel, prints the average cycles between consecutive stamps per
+// (from -> to) slot pair as "[vtaco <tag> trace]" lines on stderr, and frees the buffer
+int tc_trace_end(long long* trace, const char* tag, cudaStream_t stream);
+
+// Tiles of the tcgen05 kernels (see tile_query); the kernels count tiles in 32 bits.
+inline int set_tc_tiles(DecParams& P, bool dense) {
+  if (dense) {
+    P.t_xend = P.x1;
+    P.t_nbz = (P.nx + 31) / 32;
+    P.t_nby = (P.nx + 1) / 2;
+    P.t_nbx = (P.x1 - P.x0 + 1) / 2;
+    P.n_tiles = (long long)P.B * P.t_nbx * P.t_nby * P.t_nbz;
+  } else {
+    P.n_tiles = (P.total + kTcTile - 1) / kTcTile;
+  }
+  return P.n_tiles < (1ll << 31) ? VTACO_OK : VTACO_ERR_UNSUPPORTED;
 }
 
 }  // namespace vtaco

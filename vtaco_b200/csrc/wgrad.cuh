@@ -193,13 +193,7 @@ static inline int launch_wgrad(WParams& W, int np, cudaStream_t stream) {
   }
   if (nf > 0) {
     constexpr int smem = 2 * kW32Stage * (int)sizeof(float);
-    static std::atomic<bool> configured[64];
-    int dev = 0;
-    VTACO_CUDA_CHECK(cudaGetDevice(&dev));
-    if (!configured[dev & 63].load(std::memory_order_relaxed)) {
-      VTACO_CUDA_CHECK(cudaFuncSetAttribute(linear_wgrad32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-      configured[dev & 63].store(true, std::memory_order_relaxed);
-    }
+    VTACO_CUDA_CHECK(smem_opt_in((const void*)linear_wgrad32_kernel, smem));
     for (int i = 0; i < nf; ++i) W.list[i] = fast[i];
     linear_wgrad32_kernel<<<dim3((unsigned)chunks, (unsigned)nf), 256, smem, stream>>>(W);
     VTACO_LAUNCH_CHECK();
