@@ -109,7 +109,7 @@ int vtaco_relayout_cf(const float* src, float* dst, int B, int C, int64_t S, voi
 #define VTACO_DEC_TAIL 68
 #define VTACO_DEC_PACKED_FLOATS(n_blocks) (VTACO_DEC_OFF_BLOCKS + VTACO_DEC_BLOCK_STRIDE * (n_blocks) + VTACO_DEC_TAIL)
 #define VTACO_MAX_TIPS 8
-#define VTACO_MAX_BLOCKS 8   /* n_blocks the shared-memory-resident kernels can hold */
+#define VTACO_MAX_BLOCKS 7   /* the most n_blocks a forward decoder kernel holds (the SIMT kernel, variants 0 / 1) */
 
 /* tcgen05 operand buffer `weights_tc` (fp32, device), built from `weights` by vtaco_decoder_pack_tc in one of
  * three pack modes.  Offsets in floats.  A K-block is a 32 (n = out) x 8 (k = in) operand slice in the UMMA
@@ -190,7 +190,11 @@ typedef struct vtaco_decoder_args {
                             * 3 = single TF32 product (debug, ~1e-3); 4 = tcgen05 TF32 main product + BF16 corrections;
                             * 5 / 6 = 2 / 4 with two threads per query (768-thread CTAs, 3 tiles per SM);
                             * 7 = four tiles per SM (1024-thread CTAs): TF32 hi products + BF16 residual product, biases
-                            *     on the CUDA cores (fastest; needs fewer than 2^31 outputs per call, else 5 is used) */
+                            *     on the CUDA cores (fastest; needs fewer than 2^31 outputs per call, else 5 is used).
+                            * Where a tcgen05 variant's shared-memory layout exceeds 227 KB at n_blocks (tc2 / tc4 at
+                            * 6 and 7 blocks, tc at 7), the call runs variant 1 instead; with tip_map it returns
+                            * VTACO_ERR_UNSUPPORTED, as the byte map is read by the tcgen05 kernels only.
+                            * Features (grid / planes) are read only when n_blocks > 0. */
   /* variants 2-7: VTACO_DEC_TC_FLOATS(n_blocks) floats in pack mode VTACO_DEC_TC_MODE(variant) (layout
    * VTACO_DEC_TC_*, above), built by vtaco_decoder_pack_tc */
   const float* weights_tc;
@@ -229,7 +233,8 @@ int vtaco_sample_features(const vtaco_decoder_args* args, const float* p, int64_
  * fc_p_img.weight[:, 3:] [32][32] at OFF_WIMG).
  * d_grid / d_plane[k]: channels-last gradients [B][R..][32], ACCUMULATED into with vector
  * atomics (NULL = not wanted).  d_c_img: [B][N][32], overwritten (NULL = not wanted).
- * workspace: vtaco_decoder_backward_workspace_bytes(B*N, n_blocks) bytes of device memory. */
+ * workspace: vtaco_decoder_backward_workspace_bytes(B*N, n_blocks) bytes of device memory.
+ * n_blocks: 0 .. VTACO_MAX_BLOCKS; at 0 the features are unused and their gradients are not touched. */
 typedef struct vtaco_decoder_bwd_args {
   const float* p;          /* [B][N][3] */
   int32_t B;
@@ -280,7 +285,8 @@ int vtaco_tactile_point_map(const float* p, int64_t n, const float* axis, int32_
  * zero-initialised where no descriptor writes (padding, absent fc_c when c_dim = 0).
  * vtaco_decoder_pack_tc derives the tcgen05 operand buffer (`weights_tc`, VTACO_DEC_TC_FLOATS
  * floats) from the packed decoder buffer; `mixed` is the pack mode, VTACO_DEC_TC_MODE(variant).  It writes
- * every float of the mode's VTACO_DEC_TC_USED_FLOATS.
+ * every float of the mode's VTACO_DEC_TC_USED_FLOATS and takes n_blocks 0 .. VTACO_MAX_BLOCKS.
+ * vtaco_decoder_tc_floats(n_blocks) is VTACO_DEC_TC_FLOATS(n_blocks) for every n_blocks >= 0.
  * ------------------------------------------------------------------------- */
 #define VTACO_PACK_MAX_DESCS 64
 typedef struct vtaco_pack_desc {

@@ -1,5 +1,6 @@
 """TEST INFRASTRUCTURE ONLY — CPU restatement (torch CPU ops, fp32) of the
-reference's encoder / decoder / dense-evaluation arithmetic.
+reference's encoder / decoder / dense-evaluation arithmetic; decoder_forward also
+runs in float64 (dtype=torch.float64), the high-precision reference of the kernel tests.
 
 Every function cites the reference lines it follows (paths relative to the
 jeffsonyu/VTacO tree).  Weights are passed as a plain ``dict`` keyed exactly
@@ -200,57 +201,89 @@ def encoder_pointnet(p, W, plane_type, reso_plane=None, reso_grid=None, padding=
 # --------------------------------------------------------------------------- #
 # src/conv_onet/models/decoder.py (LocalDecoder)
 # --------------------------------------------------------------------------- #
-def sample_plane_feature(p, c, plane, padding=0.1, sample_mode='bilinear', cuda_division=False):
+def _grid_sample(c, vgrid, sample_mode, dtype):
+    """F.grid_sample of the reference's call sites; with dtype != fp32 the interpolation runs in `dtype` on
+    the fp32 grid coordinates (the coordinates themselves stay what the fp32 reference computes)."""
+    if dtype != torch.float32:
+        c, vgrid = c.to(dtype), vgrid.to(dtype)
+    return F.grid_sample(c, vgrid, padding_mode='border', align_corners=True, mode=sample_mode)
+
+
+def sample_plane_feature(p, c, plane, padding=0.1, sample_mode='bilinear', cuda_division=False,
+                         dtype=torch.float32):
     """src/conv_onet/models/decoder.py:55-60."""
     xy = normalize_coordinate(p.clone(), padding, plane, cuda_division)
     xy = xy[:, :, None].float()
     vgrid = 2.0 * xy - 1.0
-    return F.grid_sample(c, vgrid, padding_mode='border', align_corners=True,
-                         mode=sample_mode).squeeze(-1)
+    return _grid_sample(c, vgrid, sample_mode, dtype).squeeze(-1)
 
 
-def sample_grid_feature(p, c, padding=0.1, sample_mode='bilinear', cuda_division=False):
+def sample_grid_feature(p, c, padding=0.1, sample_mode='bilinear', cuda_division=False, dtype=torch.float32):
     """src/conv_onet/models/decoder.py:62-68."""
     p_nor = normalize_3d_coordinate(p.clone(), padding, cuda_division)
     p_nor = p_nor[:, :, None, None].float()
     vgrid = 2.0 * p_nor - 1.0
-    return F.grid_sample(c, vgrid, padding_mode='border', align_corners=True,
-                         mode=sample_mode).squeeze(-1).squeeze(-1)
+    return _grid_sample(c, vgrid, sample_mode, dtype).squeeze(-1).squeeze(-1)
 
 
-def sample_features(p, c_plane, padding=0.1, sample_mode='bilinear', cuda_division=False):
+def sample_features(p, c_plane, padding=0.1, sample_mode='bilinear', cuda_division=False, dtype=torch.float32):
     """Sum over present keys in the order grid,xz,xy,yz (decoder.py:72-83)."""
     c = 0
     keys = list(c_plane.keys())
     if 'grid' in keys:
-        c = c + sample_grid_feature(p, c_plane['grid'], padding, sample_mode, cuda_division)
+        c = c + sample_grid_feature(p, c_plane['grid'], padding, sample_mode, cuda_division, dtype)
     for k in ('xz', 'xy', 'yz'):
         if k in keys:
-            c = c + sample_plane_feature(p, c_plane[k], k, padding, sample_mode, cuda_division)
+            c = c + sample_plane_feature(p, c_plane[k], k, padding, sample_mode, cuda_division, dtype)
     return c.transpose(1, 2)
 
 
 def decoder_forward(p, c_plane, W, mode='forward', c_img=None, n_blocks=5, leaky=False,
-                    sample_mode='bilinear', padding=0.1, c_dim=32, cuda_division=False):
+                    sample_mode='bilinear', padding=0.1, c_dim=32, cuda_division=False,
+                    dtype=torch.float32, return_preacts=False):
     """LocalDecoder.forward (decoder.py:135-161), .forward_img (:71-103),
-    .forward_contact (:105-133) selected by `mode` in {forward, img, contact}."""
+    .forward_contact (:105-133) selected by `mode` in {forward, img, contact}.
+
+    dtype=torch.float64: the query normalisation, clamp and grid coordinates are computed in fp32 exactly as
+    the reference does (they decide which cells are read); interpolation, feature sums, every layer and the
+    heads run in float64 on float64 copies of the features, weights, points and c_img.  This is the
+    high-precision reference the fp32 kernels are measured against.
+    return_preacts: also return {'m': [m_i], 'h': [h_i], 'n_last': n} — the inputs of every ReLU (m_i = block
+    input after fc_c, h_i = fc_0 output) and of the head activation, to locate queries near a kink."""
     if c_dim != 0:
-        c = sample_features(p, c_plane, padding, sample_mode, cuda_division)
-    p = p.float()
-    if mode == 'img':
-        net = F.linear(torch.cat((p, c_img), 2), W['fc_p_img.weight'], W['fc_p_img.bias'])
+        c = sample_features(p, c_plane, padding, sample_mode, cuda_division, dtype)
+    if dtype == torch.float32:
+        p = p.float()
+        lin = F.linear
     else:
-        net = F.linear(p, W['fc_p.weight'], W['fc_p.bias'])
+        p = p.to(dtype)
+        if c_img is not None:
+            c_img = c_img.to(dtype)
+        lin = lambda x, w, b=None: F.linear(x, w.to(dtype), None if b is None else b.to(dtype))  # noqa: E731
+    if mode == 'img':
+        net = lin(torch.cat((p, c_img), 2), W['fc_p_img.weight'], W['fc_p_img.bias'])
+    else:
+        net = lin(p, W['fc_p.weight'], W['fc_p.bias'])
+    pre = {'m': [], 'h': []}
     for i in range(n_blocks):
         if c_dim != 0:
-            net = net + F.linear(c, W['fc_c.%d.weight' % i], W['fc_c.%d.bias' % i])
-        net = resnet_block_fc(net, W, 'blocks.%d.' % i)
+            net = net + lin(c, W['fc_c.%d.weight' % i], W['fc_c.%d.bias' % i])
+        if return_preacts or dtype != torch.float32:
+            # resnet_block_fc, spelled out (src/layers.py:41-50, identity shortcut)
+            pfx = 'blocks.%d.' % i
+            h = lin(F.relu(net), W[pfx + 'fc_0.weight'], W[pfx + 'fc_0.bias'])
+            pre['m'].append(net)
+            pre['h'].append(h)
+            net = net + lin(F.relu(h), W[pfx + 'fc_1.weight'], W[pfx + 'fc_1.bias'])
+        else:
+            net = resnet_block_fc(net, W, 'blocks.%d.' % i)
+    pre['n_last'] = net
     act = (lambda x: F.leaky_relu(x, 0.2)) if leaky else F.relu
-    out = F.linear(act(net), W['fc_out.weight'], W['fc_out.bias']).squeeze(-1)
+    out = lin(act(net), W['fc_out.weight'], W['fc_out.bias']).squeeze(-1)
     if mode == 'contact':
-        oc = F.linear(act(net), W['fc_out_contact.weight'], W['fc_out_contact.bias']).squeeze(-1)
-        return out, oc
-    return out
+        oc = lin(act(net), W['fc_out_contact.weight'], W['fc_out_contact.bias']).squeeze(-1)
+        out = (out, oc)
+    return (out, pre) if return_preacts else out
 
 
 # --------------------------------------------------------------------------- #

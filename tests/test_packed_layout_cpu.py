@@ -101,16 +101,16 @@ MACRO_ARGS = {'n_blocks': range(9), 'mode': range(3), 'variant': range(8), 'm': 
 
 
 def test_layout_macros_match_the_python_mirror(tmp_path):
-    """Every VTACO_DEC_* / VTACO_ENC_* layout and size macro of the header, as a C compiler evaluates it, equals
+    """VTACO_MAX_BLOCKS and every VTACO_DEC_* / VTACO_ENC_* layout and size macro of the header, as a C compiler evaluates it, equals
     its mirror in vtaco_b200._abi (VTACO_X -> _abi.X; VTACO_X(args) -> _abi.x(args) at every combination of
     MACRO_ARGS)."""
     if shutil.which('gcc') is None:
         pytest.skip('no C compiler')
     hdr = open(os.path.join(ROOT, 'include', 'vtaco_b200.h')).read()
-    consts = re.findall(r'^#define (VTACO_(?:DEC|ENC)_[A-Z0-9_]+)[ \t]', hdr, flags=re.M)
+    consts = re.findall(r'^#define (VTACO_(?:DEC|ENC)_[A-Z0-9_]+|VTACO_MAX_BLOCKS)[ \t]', hdr, flags=re.M)
     funcs = {m: tuple(a.strip() for a in args.split(','))
              for m, args in re.findall(r'^#define (VTACO_(?:DEC|ENC)_[A-Z0-9_]+)\(([^)]*)\)', hdr, flags=re.M)}
-    assert {'VTACO_DEC_BLK_W1', 'VTACO_DEC_TAIL_BCON', 'VTACO_ENC_BLK_WS', 'VTACO_ENC_FCC_B'} <= set(consts)
+    assert {'VTACO_DEC_BLK_W1', 'VTACO_DEC_TAIL_BCON', 'VTACO_ENC_BLK_WS', 'VTACO_ENC_FCC_B', 'VTACO_MAX_BLOCKS'} <= set(consts)
     assert {'VTACO_DEC_PACKED_FLOATS', 'VTACO_ENC_PACKED_FLOATS'} <= set(funcs)
     assert {'VTACO_DEC_TC_SUB_BF16', 'VTACO_DEC_TC_KBLK_FLOATS', 'VTACO_DEC_TC_MODE_TILE4'} <= set(consts)
     assert {'VTACO_DEC_TC_MODE', 'VTACO_DEC_TC_MAT', 'VTACO_DEC_TC_BIAS', 'VTACO_DEC_TC_WIMG', 'VTACO_DEC_TC_INPUT',

@@ -64,3 +64,73 @@ def randomise(module, seed):
             else:
                 val = rs.uniform(-bound, bound, size=tuple(prm.shape))
             prm.copy_(torch.from_numpy(val.astype(np.float32)))
+
+
+# --------------------------------------------------------------------------- #
+# fp32 query -> voxel coordinate, as the reference (normalize_* then grid_sample's unnormalize) and the
+# decoder kernels (common.cuh norm2d / norm3d, decoder_common.cuh unnormalize) compute it
+# --------------------------------------------------------------------------- #
+def _norm_u(v, three_d, division, padding=0.1):
+    v = np.asarray(v, dtype=np.float32)
+    d = (1.0 + padding) + (10e-4 if three_d else 10e-6)
+    if division == 'cuda':
+        u = v * np.float32(1.0 / d)
+    else:
+        u = v / np.float32(d)
+    u = (u + np.float32(0.5)).astype(np.float32)
+    u = np.where(u >= 1, np.float32(1 - (10e-4 if three_d else 10e-6)), u)
+    return np.where(u < 0, np.float32(0), u).astype(np.float32)
+
+
+def voxel_coord(v, R, three_d, division):
+    """Continuous voxel coordinate in [0, R-1] of fp32 coordinate(s) v along one axis."""
+    g = (np.float32(2) * _norm_u(v, three_d, division) - np.float32(1)).astype(np.float32)
+    return ((g + np.float32(1)) * np.float32(0.5) * np.float32(R - 1)).astype(np.float32)
+
+
+def lattice_node(k, R, three_d, division):
+    """An fp32 coordinate whose voxel coordinate is exactly the lattice node k (tap weights exactly 0 and 1),
+    or the closest one within 64 ulps of the exact preimage."""
+    d = (1.0 + 0.1) + (10e-4 if three_d else 10e-6)
+    v = np.float32((k / (R - 1) - 0.5) * d)
+    best, best_err = v, np.inf
+    for s in range(-64, 65):
+        c = np.float32(v)
+        step = np.float32(np.inf) if s > 0 else np.float32(-np.inf)
+        for _ in range(abs(s)):
+            c = np.nextafter(c, step)
+        err = abs(float(voxel_coord(c, R, three_d, division)) - k)
+        if err < best_err:
+            best, best_err = c, err
+            if err == 0:
+                break
+    return np.float32(best)
+
+
+# --------------------------------------------------------------------------- #
+# gradient checks
+# --------------------------------------------------------------------------- #
+def grad_excess(got, ref, a, r):
+    """max over elements of |got - ref| / (a * max|ref| + r * |ref|): <= 1 passes the element-wise bound.
+    Unlike a relative Frobenius norm, it sees one query's contribution missing from a tensor of thousands."""
+    got = np.asarray(got, dtype=np.float64)
+    ref = np.asarray(ref, dtype=np.float64)
+    if ref.size == 0:
+        return 0.0
+    bound = a * np.abs(ref).max() + r * np.abs(ref)
+    err = np.abs(got - ref)
+    with np.errstate(divide='ignore', invalid='ignore'):
+        q = np.where(bound > 0, err / bound, np.where(err > 0, np.inf, 0.0))
+    return float(q.max())
+
+
+def kink_mask(preacts, rel=1e-5):
+    """(B, N) bool: queries with any ReLU / LeakyReLU input within rel * (that layer's max |input|) of 0 —
+    rounding may put them on either side of the kink, so they are given zero incoming gradient."""
+    layers = list(preacts['m']) + list(preacts['h']) + [preacts['n_last']]
+    near = None
+    for t in layers:
+        t = t.detach()
+        m = (t.abs() <= rel * t.abs().max()).any(-1)
+        near = m if near is None else (near | m)
+    return near

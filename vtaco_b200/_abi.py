@@ -13,7 +13,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, 'lib', 'libvtaco_b200.so')
 
 MAX_TIPS = 8
-MAX_BLOCKS = 8
+MAX_BLOCKS = 7
 PLANE_XZ, PLANE_XY, PLANE_YZ, GRID = 0, 1, 2, 3
 KIND = {'xz': PLANE_XZ, 'xy': PLANE_XY, 'yz': PLANE_YZ, 'grid': GRID}
 DIV_RECIPROCAL, DIV_TRUE = 0, 1

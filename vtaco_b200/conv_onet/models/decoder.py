@@ -123,7 +123,8 @@ class LocalDecoder(nn.Module):
         # 2 tcgen05 3xTF32 (fp32-accurate to ~1.5e-6), 4 tcgen05 TF32 main product + BF16 corrections (3.6e-6),
         # 5 / 6 = 2 / 4 with two threads per query (8 warps per 128-query tile, 3 tiles per SM),
         # 7 = four tiles per SM (TF32 hi products + BF16 residual product; fastest, default; calls with
-        #     >= 2^31 outputs run variant 5), 3 single TF32 product (debug, ~1e-3)
+        #     >= 2^31 outputs run variant 5), 3 single TF32 product (debug, ~1e-3).  Where a tcgen05 kernel's
+        #     shared memory cannot hold n_blocks (tc2 / tc4 at 6-7 blocks, tc at 7) the call runs variant 1.
         self.kernel_variant = 7
         self._pack_cache = None
         self._pack_tc_cache = None

@@ -363,13 +363,24 @@ extern "C" int vtaco_relayout_cf(const float* src, float* dst, int B, int C, int
   return VTACO_OK;
 }
 
+// the SIMT kernel's shared memory: packed weights, the two per-query column blocks, the fingertip table
+static size_t simt_smem_bytes(int n_blocks) {
+  return ((size_t)VTACO_DEC_PACKED_FLOATS(n_blocks) + 2 * 32 * kSC + VTACO_MAX_TIPS * 32) * sizeof(float);
+}
+
 template <bool DENSE, bool F2>
-static int launch_decoder(const DecParams& P, size_t smem_bytes, cudaStream_t stream) {
+static int launch_decoder(const DecParams& P, cudaStream_t stream) {
+  const size_t smem_bytes = simt_smem_bytes(P.n_blocks);
   VTACO_CUDA_CHECK(smem_opt_in((const void*)decoder_kernel<DENSE, F2>, smem_bytes));
   const long long grid = P.n_tiles < (long long)num_sms() ? P.n_tiles : (long long)num_sms();
   decoder_kernel<DENSE, F2><<<(unsigned)grid, kThreads, smem_bytes, stream>>>(P);
   VTACO_LAUNCH_CHECK();
   return VTACO_OK;
+}
+
+int vtaco::launch_decoder_simt(const DecParams& P, bool dense, cudaStream_t stream) {
+  if (P.tip_map) return VTACO_ERR_UNSUPPORTED;   // the byte map is read by the tcgen05 kernels only
+  return dense ? launch_decoder<true, true>(P, stream) : launch_decoder<false, true>(P, stream);
 }
 
 extern "C" int vtaco_decoder_forward(const vtaco_decoder_args* a, void* stream) {
@@ -388,7 +399,8 @@ extern "C" int vtaco_decoder_forward(const vtaco_decoder_args* a, void* stream) 
   P.B = a->B; P.Rg = a->reso_grid; P.Rp = a->reso_plane;
   P.n_blocks = a->n_blocks; P.leaky = a->leaky ? 1 : 0; P.use_img = a->use_img ? 1 : 0;
   P.nearest = (a->sample_mode == VTACO_SAMPLE_NEAREST);
-  P.has_c = (a->grid || a->plane[0] || a->plane[1] || a->plane[2]) ? 1 : 0;
+  // features enter the network only through the blocks' fc_c (decoder.py:92-94): none without blocks
+  P.has_c = (a->n_blocks > 0 && (a->grid || a->plane[0] || a->plane[1] || a->plane[2])) ? 1 : 0;
   if (a->grid && a->reso_grid < 1) return VTACO_ERR_INVALID_ARG;
   if ((a->plane[0] || a->plane[1] || a->plane[2]) && a->reso_plane < 1) return VTACO_ERR_INVALID_ARG;
   P.n_tips = P.use_img ? a->n_tips : 0;
@@ -409,8 +421,7 @@ extern "C" int vtaco_decoder_forward(const vtaco_decoder_args* a, void* stream) 
   P.nc = make_norm_const(a->padding, a->div_mode);
   P.wfloats = VTACO_DEC_PACKED_FLOATS(a->n_blocks);
   if (P.wfloats % 4) return VTACO_ERR_UNSUPPORTED;
-  const size_t smem_bytes = ((size_t)P.wfloats + 2 * 32 * kSC + VTACO_MAX_TIPS * 32) * sizeof(float);
-  if (smem_bytes > 227 * 1024) return VTACO_ERR_UNSUPPORTED;  // n_blocks too large for one SM
+  if (simt_smem_bytes(a->n_blocks) > 227 * 1024) return VTACO_ERR_UNSUPPORTED;  // n_blocks too large for one SM
   if (dense) {
     if (!a->axis || a->nx < 1 || a->x0 < 0 || a->x1 > a->nx || a->x0 >= a->x1) return VTACO_ERR_INVALID_ARG;
     P.nx = a->nx; P.x0 = a->x0; P.x1 = a->x1;
@@ -445,8 +456,8 @@ extern "C" int vtaco_decoder_forward(const vtaco_decoder_args* a, void* stream) 
   if (a->variant == 7) return launch_decoder_tc4(P, dense, a->weights_tc, st);
   if (a->variant >= 2 && a->variant <= 6) return launch_decoder_tc(P, dense, a->weights_tc, st);
   const bool f2 = (a->variant == 1);
-  if (dense) return f2 ? launch_decoder<true, true>(P, smem_bytes, st) : launch_decoder<true, false>(P, smem_bytes, st);
-  return f2 ? launch_decoder<false, true>(P, smem_bytes, st) : launch_decoder<false, false>(P, smem_bytes, st);
+  if (dense) return f2 ? launch_decoder<true, true>(P, st) : launch_decoder<true, false>(P, st);
+  return f2 ? launch_decoder<false, true>(P, st) : launch_decoder<false, false>(P, st);
 }
 
 extern "C" float vtaco_key_to_float_host(int32_t key) { return key_to_float(key); }

@@ -195,5 +195,9 @@ __device__ __forceinline__ int tip_assign(const DecParams& P, float x, float y, 
   return (bi >= 0 && best < P.tip_radius && P.tip_touch[bi]) ? bi : -1;
 }
 
+// Variant 1 (exact fp32 SIMT kernel, decoder.cu), which a tcgen05 launcher runs instead when its shared-memory
+// layout does not fit at P.n_blocks.  P must still carry the SIMT tiling vtaco_decoder_forward set, so the
+// launchers call it before set_tc_tiles.  VTACO_ERR_UNSUPPORTED for a call with a tip byte map.
+int launch_decoder_simt(const DecParams& P, bool dense, cudaStream_t stream);
 
 }  // namespace vtaco

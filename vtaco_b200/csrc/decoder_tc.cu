@@ -696,7 +696,6 @@ int tc_trace_end(long long* trace, const char* tag, cudaStream_t stream) {
 
 int launch_decoder_tc(DecParams P, bool dense, const float* wtc, cudaStream_t stream) {
   if (!wtc) return VTACO_ERR_INVALID_ARG;
-  if (const int e = set_tc_tiles(P, dense)) return e;
   const bool mixed = (P.tc_products == 2);
   using Kernel = void (*)(DecParams, const float*, long long*);
   Kernel k;
@@ -715,7 +714,8 @@ int launch_decoder_tc(DecParams P, bool dense, const float* wtc, cudaStream_t st
     smem = tc_smem_layout(P.n_blocks).total;
     tag = "tc";
   }
-  if (smem > 227 * 1024) return VTACO_ERR_UNSUPPORTED;
+  if (smem > 227 * 1024) return launch_decoder_simt(P, dense, stream);
+  if (const int e = set_tc_tiles(P, dense)) return e;
   VTACO_CUDA_CHECK(smem_opt_in((const void*)k, smem));
   long long grid = (P.n_tiles + kTcGroups - 1) / kTcGroups;
   if (grid > num_sms()) grid = num_sms();

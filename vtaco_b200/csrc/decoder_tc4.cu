@@ -593,10 +593,10 @@ __global__ void __launch_bounds__(kT4Threads, 1) decoder_tc4_kernel(const __grid
 
 int launch_decoder_tc4(DecParams P, bool dense, const float* wtc, cudaStream_t stream) {
   if (!wtc) return VTACO_ERR_INVALID_ARG;
+  const Tc4Smem L = tc4_smem_layout(P.n_blocks);
+  if (L.total > 227 * 1024) return launch_decoder_simt(P, dense, stream);
   if (const int e = set_tc_tiles(P, dense)) return e;
   if ((dense ? (long long)P.B * P.nx * P.nx * P.nx : P.total) >= (1ll << 31)) return VTACO_ERR_UNSUPPORTED;   // 32-bit output index
-  const Tc4Smem L = tc4_smem_layout(P.n_blocks);
-  if (L.total > 227 * 1024) return VTACO_ERR_UNSUPPORTED;
   long long* trace;
   if (const int e = tc_trace_begin(&trace, stream)) return e;
   using Kernel = void (*)(DecParams, const float*, long long*);
