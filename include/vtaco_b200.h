@@ -213,6 +213,10 @@ typedef struct vtaco_decoder_args {
    * tip_touch[] / tip_radius unused).  Built by vtaco_fingertip_ids / vtaco_tactile_point_map.
    * tcgen05 variants only. */
   const uint8_t* tip_map;
+  /* with tip_map: tip_feat is [B][n_tips][32] — query of sample b with id k takes the projected row of
+   * tip_feat[b][k-1] (per-scene fingertip features of a batch of lattices; ids from
+   * vtaco_fingertip_lattice_ids).  tcgen05 variants only (else VTACO_ERR_UNSUPPORTED). */
+  int32_t tip_feat_per_sample;
 } vtaco_decoder_args;
 
 int vtaco_decoder_forward(const vtaco_decoder_args* args, void* stream);
@@ -274,6 +278,12 @@ int vtaco_decoder_backward(const vtaco_decoder_bwd_args* args, void* stream);
  * ------------------------------------------------------------------------- */
 int vtaco_fingertip_ids(const float* p, int64_t n, const double* tips_host, const int32_t* touch_host,
                         int32_t n_tips, double radius, uint8_t* ids, void* stream);
+/* vtaco_fingertip_lattice_ids: the fingertip form on B dense lattices axis[nx]^3 with per-scene fingertips on the
+ *   device (a captured graph re-reads them): ids[b][q] for lattice query q of scene b, from tips [B][n_tips][3]
+ *   doubles and touch [B][n_tips] int32, with the decoder's own test (tip_assign: fp32 prefilter, float64 nearest
+ *   tip, first minimum, radius, touch) — the ids equal the in-kernel assignment of a single-scene decode. */
+int vtaco_fingertip_lattice_ids(const float* axis, int32_t nx, int32_t B, const double* tips, const int32_t* touch,
+                                int32_t n_tips, double radius, uint8_t* ids, void* stream);
 int vtaco_tactile_point_map(const float* p, int64_t n, const float* axis, int32_t nx, const double* pts,
                             int32_t n_pts, double radius, int32_t value, uint8_t* map, void* stream);
 
@@ -446,12 +456,27 @@ typedef struct vtaco_mc_args {
    * holds only the first nx - halo_rows rows.  A rank then decodes its own rows only. */
   const float* halo_grid;
   int32_t halo_rows;
+  /* batched mode (n_volumes > 1, or scene_counts non-NULL): `grid` holds n_volumes contiguous volumes
+   * [n_volumes][nx][ny][nz] (nx = rows of ONE volume).  Volume b is extracted at its own level: 0.5f*(min+max)
+   * of key pair b of level_keys [n_volumes][2], or `level` for all volumes when level_keys is NULL.  Output:
+   * the meshes of all volumes concatenated in volume order, each volume's faces indexing its own vertex block
+   * (ids local to the volume); scene_counts (device int64[n_volumes][2]) receives (V, F) per volume and counts
+   * the totals.  Per volume, the result equals a single-volume call on that volume bit for bit.  Overflow as
+   * above: everything is counted, what fits is written.  Needs vtaco_mc_batch_scratch_bytes of scratch; slab
+   * mode, level_ptr and n_level_keys > 1 are not accepted. */
+  int32_t n_volumes;
+  int64_t* scene_counts;
 } vtaco_mc_args;
 
 int64_t vtaco_mc_scratch_bytes(int32_t nx, int32_t ny, int32_t nz);
+int64_t vtaco_mc_batch_scratch_bytes(int32_t n_volumes, int32_t nx, int32_t ny, int32_t nz);
 int vtaco_marching_cubes(const vtaco_mc_args* args, void* stream);
 /* keys[0..1] <- ordered-int keys of min / max of grid[0..n) (initialised by the call) */
 int vtaco_grid_minmax(const float* grid, int64_t n, int32_t* keys, void* stream);
+/* per-volume keys of n_volumes contiguous volumes of n floats each: keys[2b], keys[2b+1] are merged
+ * (atomicMin / atomicMax; the caller initialises them to INT32_MAX, INT32_MIN) with the ordered-int keys of
+ * the min / max of volume b — the keys the decoder's minmax_key holds after decoding that volume alone. */
+int vtaco_volume_keys(const float* grid, int32_t n_volumes, int64_t n, int32_t* keys, void* stream);
 /* multi-GPU iso-level exchange without a collective: copy this rank's (min,max) key pair into
  * slot `rank` (0..7) of each of the `n_peers` int32[world][2] tables given (peer-mapped pointers:
  * all ranks' tables for an all-gather, only the root's for a gather), then reset `keys` to

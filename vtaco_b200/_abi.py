@@ -52,7 +52,7 @@ class DecoderArgs(C.Structure):
         ('logits', C.c_void_p), ('contact', C.c_void_p), ('minmax_key', C.c_void_p),
         ('variant', C.c_int32), ('weights_tc', C.c_void_p),
         ('logits_peers', C.c_void_p * 8), ('n_peers', C.c_int32), ('logits_multicast', C.c_void_p),
-        ('tip_map', C.c_void_p),
+        ('tip_map', C.c_void_p), ('tip_feat_per_sample', C.c_int32),
     ]
 
 
@@ -102,6 +102,7 @@ class McArgs(C.Structure):
         ('voffset', C.c_float), ('vscale', C.c_float), ('phase', C.c_int32),
         ('x_emit', C.c_int32), ('x_origin', C.c_int32), ('level_ptr', C.c_void_p),
         ('halo_grid', C.c_void_p), ('halo_rows', C.c_int32),
+        ('n_volumes', C.c_int32), ('scene_counts', C.c_void_p),
     ]
 
 
@@ -305,6 +306,7 @@ def lib():
     for name, argtypes in _OPTIONAL.items():
         getattr(L, name).argtypes = argtypes
     L.vtaco_mc_scratch_bytes.restype = C.c_int64
+    L.vtaco_mc_batch_scratch_bytes.restype = C.c_int64
     if L.vtaco_abi_version() != 1:
         raise RuntimeError('vtaco_b200: ABI version mismatch')
     _lib = L
@@ -315,6 +317,8 @@ _OPTIONAL = {
     'vtaco_marching_cubes': [C.POINTER(McArgs), C.c_void_p],
     'vtaco_mc_scratch_bytes': [C.c_int32, C.c_int32, C.c_int32],
     'vtaco_grid_minmax': [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p],
+    'vtaco_mc_batch_scratch_bytes': [C.c_int32, C.c_int32, C.c_int32, C.c_int32],
+    'vtaco_volume_keys': [C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p],
     'vtaco_publish_keys': [C.c_void_p, C.POINTER(C.c_void_p), C.c_int32, C.c_int32, C.c_void_p],
     'vtaco_conv3d_cl': [C.POINTER(Conv3dArgs), C.c_void_p],
     'vtaco_maxpool2_cl': [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
@@ -324,6 +328,8 @@ _OPTIONAL = {
     'vtaco_depth_to_space2_cl': [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p],
     'vtaco_fingertip_ids': [C.c_void_p, C.c_int64, C.POINTER(C.c_double), C.POINTER(C.c_int32), C.c_int32, C.c_double,
                             C.c_void_p, C.c_void_p],
+    'vtaco_fingertip_lattice_ids': [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_double,
+                                    C.c_void_p, C.c_void_p],
     'vtaco_tactile_point_map': [C.c_void_p, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_double,
                                 C.c_int32, C.c_void_p, C.c_void_p],
     'vtaco_exchange_level': [C.POINTER(Exchange), C.c_void_p, C.c_void_p],

@@ -14,7 +14,7 @@ import numpy as np
 import torch
 
 from ..common import make_3d_grid, dense_axis
-from ..mcubes import MarchingCubes, new_minmax_key
+from ..mcubes import MarchingCubes, new_minmax_key, split_meshes
 from .. import dist as vdist
 
 
@@ -110,6 +110,8 @@ class Generator3D(object):
         self.halo_from_peer = True    # sharded extraction: read the two halo rows from the next rank instead of decoding them
         self._keys = None
         self._keys_init = None
+        self._batch = None          # (grid (B,nx,nx,nx), keys (B,2), initial keys, axis) of the batched path
+        self._batch_mc = None       # the batched path's extractor (its buffers are not the single-scene path's)
         self._pin = None
         self._fused = None
         self._root_ex = None
@@ -537,6 +539,123 @@ class Generator3D(object):
         if to_host:
             return self._to_host(v, f)
         return v, f
+
+    # ------------------------------------------------------------------ batched extraction (single GPU)
+    def _batch_check(self, group):
+        if vdist.rank_world(group)[1] > 1:
+            raise NotImplementedError('batched mesh extraction runs on one GPU: call generate_mesh per scene with a '
+                                      'process group')
+
+    def _batch_tips(self, tips, radius):
+        """(pos (B,F,3), feat (B,F,c_dim), touch (B,F)) -> the CUDA tensors the batched decode reads: float64
+        positions, float32 features, int32 touch mask (tensors of that kind on the device are used as they are,
+        so a captured graph re-reads them at replay)."""
+        if tips is None or not self.with_img:
+            return None
+        pos, feat, touch = tips
+        dev = self.device
+        pos = torch.as_tensor(pos).to(device=dev, dtype=torch.float64).contiguous()
+        touch = torch.as_tensor(touch).to(device=dev).to(torch.int32).contiguous()
+        feat = torch.as_tensor(feat).to(device=dev, dtype=torch.float32)
+        return pos, feat, touch, float(radius)
+
+    def lattices_and_meshes(self, c, tips=None):
+        """Batched `lattice_and_mesh`: the B lattices of the feature batch `c` in one decoder launch (with
+        `with_img`: per-scene fingertips tips = (pos (B,F,3) float64, feat (B,F,32), touch (B,F) int32, radius)
+        as CUDA tensors), the per-scene iso-levels, and the B meshes in one marching-cubes pass; no host
+        synchronisation.  The batched path has its own lattice axis and extractor, so graphs of the single-scene
+        path on this generator keep their buffers.  Returns the batch extractor's (vertex buffer, face buffer,
+        int64[4] totals, (B,2) per-scene (V,F) counts)."""
+        nx = self.resolution0 * 4
+        dev = self.device
+        B = next(t.size(0) for k, t in c.items() if torch.is_tensor(t))
+        if self._batch is None or tuple(self._batch[0].shape) != (B, nx, nx, nx):
+            init = new_minmax_key(dev, B)
+            self._batch = (torch.empty((B, nx, nx, nx), dtype=torch.float32, device=dev), init.clone(), init,
+                           dense_axis(nx, self.padding, dev))
+        if self._batch_mc is None:
+            self._batch_mc = MarchingCubes(dev)
+        grid, keys, init, axis = self._batch
+        keys.copy_(init)
+        self.model.decoder.forward_dense(c, nx, use_img=self.with_img, tips=tips, out=grid, minmax_key=keys, axis=axis)
+        return self._batch_mc.batch(grid, level_keys=keys, voffset=np.float32(nx / 2),
+                                    vscale=np.float32((1 + self.padding) / nx), sync=False)
+
+    def generate_meshes(self, inputs=None, c=None, tips=None, radius=0.05, to_host=True, group=None):
+        """Batched `generate_mesh`: inputs (B,T,3) point clouds (or their features `c`) -> encoder -> B lattices
+        decoded in one launch -> per-scene iso-level 0.5*(min+max) -> B meshes in one marching-cubes pass.
+        tips = (pos (B,F,3), feat (B,F,c_dim), touch (B,F)): every scene's own fingertips (with_img), within
+        `radius`.  Returns a list of B (vertices, faces), each equal to `generate_mesh` of that scene's features
+        and fingertips (faces index the scene's own vertices); host arrays with to_host, else device tensors.
+        One GPU."""
+        self._batch_check(group)
+        self.model.eval()
+        with torch.no_grad():
+            if c is None:
+                c = self.model.encode_inputs(inputs.to(self.device, non_blocking=True))
+            vb, fb, counts, scene_counts = self.lattices_and_meshes(c, self._batch_tips(tips, radius))
+            V, F = [int(x) for x in counts[:2].cpu()]
+            if V > vb.shape[0] or F > fb.shape[0]:   # re-run phase 2 with larger buffers
+                grid, keys, _, _ = self._batch
+                vb, fb, scene_counts = self._batch_mc.batch(grid, level_keys=keys,
+                                                            voffset=np.float32(grid.shape[1] / 2),
+                                                            vscale=np.float32((1 + self.padding) / grid.shape[1]))
+            sc = scene_counts.cpu()
+            v, f = vb[:V], fb[:F]
+            if to_host:
+                v, f = self._to_host(v, f)
+                v, f = v.copy(), f.copy()
+        return split_meshes(v, f, sc)
+
+    def capture_generate_batch(self, inputs_host, tips=None, radius=0.05, warmup=2, group=None):
+        """CUDA graph of the batched extraction for a fixed batch shape: H2D copy of the (pinned) host clouds
+        (B,T,3) -> encoder -> B lattices in one decoder launch -> B meshes in one marching-cubes pass.  Usage:
+            run = gen.capture_generate_batch(pinned_clouds, tips)   # once per shape
+            pinned_clouds.copy_(new_clouds); meshes = run()         # per batch: list of B host (vertices, faces)
+        tips = (pos (B,F,3) float64, feat (B,F,c_dim) float32, touch (B,F) int32) as CUDA tensors are read at
+        every replay: write new fingertips into them in place.  run() reads all counters with one host
+        synchronisation per batch; the copy of the meshes, sized by those counters, waits once more.  The graph
+        uses the model's and this generator's batch buffers as they are at capture; a later call with a larger
+        batch or lattice on the same model / generator may grow (re-allocate) them: capture each shape on its
+        own generator and model, or capture again."""
+        self._batch_check(group)
+        if not inputs_host.is_pinned():
+            raise ValueError('inputs_host must be a pinned host tensor (it is re-read at every replay)')
+        dev = self.device
+        dtips = self._batch_tips(tips, radius)
+        if dtips is not None and not (tips[0] is dtips[0] and tips[1] is dtips[1] and tips[2] is dtips[2]):
+            raise ValueError('capture_generate_batch re-reads the fingertips at replay: pass them as CUDA tensors '
+                             '(pos float64, feat float32, touch int32)')
+        static_in = torch.empty(inputs_host.shape, dtype=torch.float32, device=dev)
+        self.model.eval()
+
+        def body():
+            static_in.copy_(inputs_host, non_blocking=True)
+            return self.lattices_and_meshes(self.model.encode_inputs(static_in), dtips)
+
+        with torch.no_grad():
+            for _ in range(max(1, warmup)):
+                out = body()
+            V, F = [int(x) for x in out[2][:2].cpu()]
+            if V > out[0].shape[0] or F > out[1].shape[0]:
+                self._batch_mc._ensure(0, int(V * 1.5) + 16, int(F * 1.5) + 16)
+                body()
+            torch.cuda.synchronize(dev)
+            graph = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(graph):
+                out = body()
+
+        def run():
+            graph.replay()
+            counts = torch.cat([out[2][:2], out[3].reshape(-1)]).cpu()     # one D2H of all counters
+            V, F = int(counts[0]), int(counts[1])
+            if V > out[0].shape[0] or F > out[1].shape[0]:
+                raise RuntimeError('meshes larger than the captured buffers (%d vertices, %d faces): re-capture' % (V, F))
+            v, f = self._to_host(out[0][:V], out[1][:F])
+            return split_meshes(v.copy(), f.copy(), counts[2:].reshape(-1, 2))
+
+        run.graph = graph
+        return run
 
     def mesh_chamfer(self, vertices, points_obj, n_sample=2048, generator=None):
         """The Chamfer metric of generate_obj_mesh_wnf (reference generation.py:275-281): shuffle the

@@ -493,10 +493,25 @@ class LocalDecoder(nn.Module):
         use_img + c_img (nx^3, 32): dense tactile tensor as in eval_points;
         use_img + tips=(pos (F,3) float64, feat (F,32) cuda tensor, touch (F,) bool, radius):
         compact form of generation.py:190-200.  `minmax_key` (int32[2], init
-        [INT32_MAX, INT32_MIN]) receives ordered-int keys of min/max logit."""
+        [INT32_MAX, INT32_MIN]) receives ordered-int keys of min/max logit.
+
+        A feature batch of B > 1 scenes decodes all B lattices in one launch: `out` (B,nx,nx,nx) and
+        `minmax_key` (B,2) (init [INT32_MAX, INT32_MIN] per row) receive each scene's logits and keys, bit for
+        bit those of a B = 1 call on that scene's features (and fingertips).  Per-scene fingertips: use_img +
+        tips=(pos (B,F,3) float64, feat (B,F,32) float32, touch (B,F) int32 — CUDA tensors, read at launch
+        time — , radius); they go through the per-query byte map (tcgen05 variants).  Whole lattices only,
+        without a dense c_img tensor or multi-GPU outputs."""
         dev = self.fc_out.weight.device
         if torch.is_grad_enabled():
             _abi.forbid_autograd(*self._param_tuple())
+        feats = [t for k, t in c_plane.items() if k in ('grid',) + _PLANES and torch.is_tensor(t)]
+        B = feats[0].size(0) if feats and self.c_dim != 0 else (out.size(0) if out is not None and out.dim() == 4 else 1)
+        if B != 1 or (out is not None and out.dim() == 4):
+            if x0 != 0 or (x1 is not None and x1 != nx) or peers or multicast:
+                raise NotImplementedError('a batch of lattices is decoded whole, on one GPU (x0 = 0, x1 = nx, no peers)')
+            if use_img and (c_img is not None or tip_map is not None):
+                raise NotImplementedError('a batch of lattices takes tactile features as per-scene fingertips (tips)')
+            return self._forward_dense_batch(c_plane, nx, B, out, minmax_key, axis, dev, use_img, tips)
         x1 = nx if x1 is None else x1
         if out is None:
             out = torch.empty((nx, nx, nx), dtype=torch.float32, device=dev)
@@ -542,4 +557,43 @@ class LocalDecoder(nn.Module):
         if minmax_key is not None:
             a.minmax_key = minmax_key.data_ptr()
         self._run(a, dev)
+        return out
+
+    def _forward_dense_batch(self, c_plane, nx, B, out, minmax_key, axis, dev, use_img=False, tips=None):
+        """forward_dense of B scenes: one decoder launch over the B lattices, then the per-scene (min,max) keys
+        in one reduction launch over the stored logits (vtaco_volume_keys: the reduction the decoder applies to
+        a single scene)."""
+        from ...mcubes import volume_keys
+        if out is None:
+            out = torch.empty((B, nx, nx, nx), dtype=torch.float32, device=dev)
+        if tuple(out.shape) != (B, nx, nx, nx) or not out.is_contiguous() or out.dtype != torch.float32 \
+                or out.device != dev:
+            raise ValueError('out must be a contiguous float32 (%d,%d,%d,%d) tensor on %s' % (B, nx, nx, nx, dev))
+        if minmax_key is not None and (minmax_key.dtype != torch.int32 or minmax_key.device != dev or
+                                       tuple(minmax_key.shape) != (B, 2) or not minmax_key.is_contiguous()):
+            raise ValueError('minmax_key must be a contiguous int32 (%d,2) tensor on %s' % (B, dev))
+        a, keep = self._base_args(c_plane, B, B * nx ** 3)
+        if axis is None:
+            axis = dense_axis(nx, self.padding, dev)
+        a.axis = axis.data_ptr()
+        a.nx, a.x0, a.x1 = nx, 0, nx
+        a.use_img = int(use_img)
+        if use_img and tips is not None:
+            from ..tactile import fingertip_lattice_ids
+            pos, feat, touch, radius = tips
+            if not (torch.is_tensor(feat) and feat.is_cuda and feat.dtype == torch.float32 and feat.dim() == 3
+                    and tuple(feat.shape) == (B, pos.shape[1], 32)):
+                raise ValueError('tip features must be a float32 CUDA tensor (%d,F,32)' % B)
+            if pos.dim() != 3 or pos.shape[0] != B:
+                raise ValueError('tips must hold the fingertips of %d scenes' % B)
+            if a.variant not in (2, 4, 5, 6, 7):
+                raise NotImplementedError('per-scene fingertips need a tcgen05 kernel variant (2, 4, 5, 6, 7)')
+            ids = fingertip_lattice_ids(axis, pos, touch, radius)
+            featc = feat.contiguous()
+            a.tip_map, a.tip_feat, a.n_tips, a.tip_feat_per_sample = ids.data_ptr(), featc.data_ptr(), feat.shape[1], 1
+            keep += [ids, featc]
+        a.logits = out.data_ptr()
+        self._run(a, dev)
+        if minmax_key is not None:
+            volume_keys(out, minmax_key)
         return out

@@ -44,6 +44,31 @@ def fingertip_ids(p, tips, touch, radius=0.05):
     return ids
 
 
+def fingertip_lattice_ids(axis, tips, touch, radius=0.05, out=None):
+    """ids (B,nx^3) uint8 of B dense lattices axis[nx]^3 with per-scene fingertips: ids[b, q] = f+1 where f is the
+    nearest fingertip of scene b (float64, first minimum) if it is closer than `radius` and touch[b, f]; else 0 —
+    the decoder's own in-kernel assignment.  axis (nx,) float32 CUDA; tips (B,F,3) float64 and touch (B,F) int32
+    CUDA tensors, read by the launch (a captured graph re-reads them at replay)."""
+    _abi.require_cuda(axis, 'axis')
+    if not (torch.is_tensor(tips) and tips.is_cuda and tips.dtype == torch.float64 and tips.dim() == 3
+            and tips.shape[2] == 3 and tips.is_contiguous()):
+        raise ValueError('tips must be a contiguous float64 CUDA tensor (B,F,3)')
+    B, F_ = tips.shape[0], tips.shape[1]
+    if not (torch.is_tensor(touch) and touch.is_cuda and touch.dtype == torch.int32 and tuple(touch.shape) == (B, F_)
+            and touch.is_contiguous()):
+        raise ValueError('touch must be a contiguous int32 CUDA tensor (%d,%d)' % (B, F_))
+    if not 1 <= F_ <= _abi.MAX_TIPS:
+        raise ValueError('1 to %d fingertips per scene' % _abi.MAX_TIPS)
+    nx = axis.numel()
+    if out is None:
+        out = torch.empty((B, nx ** 3), dtype=torch.uint8, device=axis.device)
+    with torch.cuda.device(axis.device):
+        _abi.check(_abi.lib().vtaco_fingertip_lattice_ids(_abi.ptr(axis), nx, B, _abi.ptr(tips), _abi.ptr(touch), F_,
+                                                          float(radius), _abi.ptr(out), _abi.stream_ptr(axis.device)),
+                   'fingertip_lattice_ids')
+    return out
+
+
 def tactile_point_map(points_per_sensor, touch, radius=0.015, p=None, nx=None, padding=0.1, device=None):
     """generation.py:222-255 (encode_t2d branch): map (N,) / (nx^3,) uint8 — t+1 for every query closer than
     `radius` to any point of sensor t's back-projected tactile cloud, sensors in increasing order (later ones

@@ -414,10 +414,11 @@ extern "C" int vtaco_decoder_forward(const vtaco_decoder_args* a, void* stream) 
     P.tip_touch[f] = f < P.n_tips ? a->tip_touch[f] : 0;
   }
   P.tip_radius = a->tip_radius;
-  {
-    const double r = a->tip_radius * 1.01 + 1e-4;
-    P.tip_r2_hi = (float)(r * r);
-  }
+  // per-sample tip tables: byte-map form only (the ids select the row), tcgen05 kernels only (the SIMT launcher
+  // refuses a byte map)
+  if (a->tip_feat_per_sample && (!a->tip_map || !(a->variant >= 2 && a->variant <= 7))) return VTACO_ERR_UNSUPPORTED;
+  P.tip_ps = (a->tip_feat_per_sample && P.n_tips > 0) ? 1 : 0;
+  P.tip_r2_hi = tip_prefilter_r2(a->tip_radius);
   P.nc = make_norm_const(a->padding, a->div_mode);
   P.wfloats = VTACO_DEC_PACKED_FLOATS(a->n_blocks);
   if (P.wfloats % 4) return VTACO_ERR_UNSUPPORTED;

@@ -41,6 +41,7 @@ struct DecParams {
   int tip_touch[VTACO_MAX_TIPS];
   double tip_radius;
   float tip_r2_hi;  // fp32 prefilter threshold (squared, padded)
+  int tip_ps;       // tip_feat is [B][n_tips][32]: one table per sample (byte-map form, tcgen05 kernels)
 };
 
 __device__ __forceinline__ void store_logit(const DecParams& P, long long idx, float v) {
@@ -168,6 +169,11 @@ __device__ __forceinline__ void flush_minmax(const DecParams& P, float vmin, flo
   }
 }
 
+// fp32 prefilter threshold of tip_assign (squared, padded so that it never rejects a query within `radius`)
+__host__ __device__ __forceinline__ float tip_prefilter_r2(double radius) {
+  const double r = radius * 1.01 + 1e-4;
+  return (float)(r * r);
+}
 // generation.py:190-200: nearest fingertip in float64 (scipy cdist), within radius, touched.
 __device__ __forceinline__ int tip_assign(const DecParams& P, float x, float y, float z);
 // tactile feature row of a query: from the byte map when given, else the in-kernel fingertip test

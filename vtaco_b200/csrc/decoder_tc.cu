@@ -247,10 +247,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) decoder_tc_kernel(const __grid_
     }
     if (P.use_img && P.n_tips > 0) {
       const int f = tip_of_query(P, oidx, px, py, pz);
-      if (f >= 0) {
-#pragma unroll
-        for (int j = 0; j < 32; ++j) net[j] += sTip[f * 32 + j];
-      }
+      if (f >= 0) add_tip_row<32>(net, P, sTip, f, oidx, 0);
     }
     TC_STAMP(trace, 17);    // fc_p / tips done
     uint32_t r[32];
@@ -569,10 +566,7 @@ __global__ void __launch_bounds__(kTc2Threads, 1) decoder_tc2_kernel(const __gri
     }
     if (P.use_img && P.n_tips > 0) {
       const int f = tip_of_query(P, oidx, px, py, pz);
-      if (f >= 0) {
-#pragma unroll
-        for (int j = 0; j < 16; ++j) net[j] += sTip[f * 32 + ch0 + j];
-      }
+      if (f >= 0) add_tip_row<16>(net, P, sTip, f, oidx, ch0);
     }
     uint32_t r[16];
     float x[16];

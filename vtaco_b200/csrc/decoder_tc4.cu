@@ -122,8 +122,9 @@ __device__ __forceinline__ void issue_product_t4(uint32_t d, uint32_t a_hi, uint
 }
 
 // NB > 0: the network depth as a compile-time constant (the shipped 5): the block loop is unrolled and the operand
-// descriptors of every step are base + immediate
-template <bool DENSE, bool TRACE, int NB>
+// descriptors of every step are base + immediate.  TIP_PS: per-sample fingertip tables (P.tip_ps), an instantiation
+// of its own so that the other instantiations keep their register allocation.
+template <bool DENSE, bool TRACE, int NB, bool TIP_PS = false>
 __global__ void __launch_bounds__(kT4Threads, 1) decoder_tc4_kernel(const __grid_constant__ DecParams P,
                                                                     const float* __restrict__ wtc,
                                                                     long long* __restrict__ trace) {
@@ -466,8 +467,12 @@ __global__ void __launch_bounds__(kT4Threads, 1) decoder_tc4_kernel(const __grid
       }
     }
     if (tipf >= 0) {
+      if (TIP_PS) {
+        add_tip_row<16>(net, P, sTip, tipf, max(oidx, 0), ch0);
+      } else {
 #pragma unroll
-      for (int j = 0; j < 16; ++j) net[j] += sTip[tipf * 32 + ch0 + j];
+        for (int j = 0; j < 16; ++j) net[j] += sTip[tipf * 32 + ch0 + j];
+      }
     }
 
     // ---------------- residual blocks: 2 accumulation steps each ----------------
@@ -600,7 +605,11 @@ int launch_decoder_tc4(DecParams P, bool dense, const float* wtc, cudaStream_t s
   long long* trace;
   if (const int e = tc_trace_begin(&trace, stream)) return e;
   using Kernel = void (*)(DecParams, const float*, long long*);
-  const Kernel k = trace ? (dense ? decoder_tc4_kernel<true, true, 0> : decoder_tc4_kernel<false, true, 0>)
+  const Kernel k = P.tip_ps ? (P.n_blocks == 5 ? (dense ? decoder_tc4_kernel<true, false, 5, true>
+                                                         : decoder_tc4_kernel<false, false, 5, true>)
+                                               : (dense ? decoder_tc4_kernel<true, false, 0, true>
+                                                        : decoder_tc4_kernel<false, false, 0, true>))
+                   : trace ? (dense ? decoder_tc4_kernel<true, true, 0> : decoder_tc4_kernel<false, true, 0>)
                    : P.n_blocks == 5 ? (dense ? decoder_tc4_kernel<true, false, 5> : decoder_tc4_kernel<false, false, 5>)
                                      : (dense ? decoder_tc4_kernel<true, false, 0> : decoder_tc4_kernel<false, false, 0>);
   VTACO_CUDA_CHECK(smem_opt_in((const void*)k, L.total));

@@ -369,6 +369,26 @@ __device__ __forceinline__ void load_tips(float* sTip, const DecParams& P, int t
     }
   }
 }
+// net[0..NC) += channels [ch0, ch0 + NC) of the projected tactile row f of the query with output index oidx: from
+// sTip (one table per launch) or, with per-sample tables (tip_ps), fc_p_img.weight[:, 3:] @ tip_feat[sample][f]
+// computed here in load_tips' k order (bit-identical to the row load_tips builds; tactile queries are rare)
+template <int NC>
+__device__ __forceinline__ void add_tip_row(float* net, const DecParams& P, const float* sTip, int f, long long oidx,
+                                            int ch0) {
+  if (P.tip_ps) {
+    const float* feat = P.tip_feat + ((oidx / P.N) * P.n_tips + f) * 32;
+#pragma unroll
+    for (int j = 0; j < NC; ++j) {
+      float a = 0.f;
+#pragma unroll 1
+      for (int k = 0; k < 32; ++k) a = fmaf(__ldg(P.weights + VTACO_DEC_OFF_WIMG + k * 32 + ch0 + j), __ldg(feat + k), a);
+      net[j] += a;
+    }
+  } else {
+#pragma unroll
+    for (int j = 0; j < NC; ++j) net[j] += sTip[f * 32 + ch0 + j];
+  }
+}
 // one MMA-completion mbarrier per group
 __device__ __forceinline__ void init_group_bars(uint64_t* sBars, int n_groups, int tid) {
   if (tid == 0) {

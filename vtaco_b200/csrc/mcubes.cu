@@ -28,6 +28,12 @@
 // by rows < x_emit and faces of cells in rows < x_emit are emitted and counted.  The pieces of
 // consecutive slabs then concatenate to exactly the single-volume mesh (ids + the vertex base of
 // the slab).
+// Batched mode (n_volumes > 1 or scene_counts): B contiguous volumes are one stacked volume of B*nx
+// rows.  A run takes the level of its scene (row / nx); the last row of a scene owns no cells and no
+// x-edge (the rule slab mode applies to halo rows), so no vertex or face joins two scenes.  The
+// look-back prefix at a scene's first run is its vertex / face base: the emit pass subtracts the
+// vertex base from face ids (ids local to the scene's vertex block) and writes the per-scene counts.
+// The single-volume kernels are the BATCH = false instantiations, untouched by this mode.
 // Algorithmic bytes: 4*n (grid) + 12*V + 12*F; scratch traffic adds the active blocks' codes
 // and base ids.
 #include "common.cuh"
@@ -64,7 +70,19 @@ struct McParams {
   int32_t* faces;
   long long fcap;
   float voffset, vscale;
+  // batched mode only
+  int nxs;                        // rows per volume: row i belongs to scene i / nxs
+  unsigned scene_runs;            // runs per volume (nxs * ny * nzc)
+  int n_vol;
+  unsigned long long* sbase;      // [n_vol][2] scratch: vertex / triangle base of each scene (prefix at its first run)
+  long long* scene_counts;        // [n_vol][2]: (V, F) of each scene
 };
+
+// iso-level of scene s in batched mode: its own (min,max) key pair, else the one given level
+__device__ __forceinline__ float scene_level(const McParams& P, int s) {
+  if (P.level_keys) return 0.5f * (key_to_float(P.level_keys[2 * s]) + key_to_float(P.level_keys[2 * s + 1]));
+  return P.level;
+}
 
 __device__ __forceinline__ float mc_level(const McParams& P) {
   if (P.level_ptr) return *P.level_ptr;
@@ -129,10 +147,11 @@ __device__ __forceinline__ unsigned row_bits(const McParams& P, int i, int j, in
 // Bit-parallel over the run: own-edge masks are XORs of the "above" rows and a cell is cut iff
 // its 8 corner bits are neither all 0 nor all 1, so the ~95 % of runs that the surface does not
 // touch cost a handful of logic ops; only the set bits take the per-point path.
-__device__ __forceinline__ unsigned run_codes(const McParams& P, int i, int j, int k0, unsigned r00, unsigned r10,
-                                               unsigned r01, unsigned r11, unsigned long long& codes,
+// row_end: first row past the volume of row i (P.nx; batched mode: the end of the scene's rows).
+__device__ __forceinline__ unsigned run_codes(const McParams& P, int i, int j, int k0, int row_end, unsigned r00,
+                                               unsigned r10, unsigned r01, unsigned r11, unsigned long long& codes,
                                                const uint8_t* __restrict__ tri_count) {
-  const bool hx = i + 1 < P.nx, hy = j + 1 < P.ny;
+  const bool hx = i + 1 < row_end, hy = j + 1 < P.ny;
   const int left = P.nz - k0;                                     // points of this run inside the lattice
   const unsigned m8 = left >= kMcRun ? 0xffu : ((1u << left) - 1u);
   const unsigned mz = left - 1 >= kMcRun ? 0xffu : ((1u << max(left - 1, 0)) - 1u);   // points with k+1 < nz
@@ -182,6 +201,7 @@ __device__ __forceinline__ long long run_of(const McParams& P, int i, int j, int
 constexpr int kMcSub = 4;                          // consecutive 256-run sub-blocks per CTA: 4x fewer look-back words
 constexpr int kMcBlockRuns = kMcThreads * kMcSub;
 
+template <bool BATCH>
 __global__ void __launch_bounds__(kMcThreads) mc_fused_kernel(const __grid_constant__ McParams P) {
   constexpr int kWarps = kMcThreads / 32;
   __shared__ int s_bid;
@@ -216,7 +236,8 @@ __global__ void __launch_bounds__(kMcThreads) mc_fused_kernel(const __grid_const
     if (run < P.nruns) {
       int i, j, k0;
       run_coords(P, run, i, j, k0);
-      own[s] = row_bits(P, i, j, k0, level) | (row_bits(P, i + 1, j, k0, level) << 16);
+      const float lv = BATCH ? scene_level(P, i / P.nxs) : level;
+      own[s] = row_bits(P, i, j, k0, lv) | (row_bits(P, i + 1, j, k0, lv) << 16);
     }
     s_rows[s * kMcThreads + threadIdx.x] = own[s];
   }
@@ -230,11 +251,14 @@ __global__ void __launch_bounds__(kMcThreads) mc_fused_kernel(const __grid_const
     if (run < P.nruns) {
       int i, j, k0;
       run_coords(P, run, i, j, k0);
+      const int sc = BATCH ? i / P.nxs : 0;
+      const float lv = BATCH ? scene_level(P, sc) : level;
       unsigned nxt;
       if (j + 1 >= P.ny) nxt = own[s];                           // replicated row: its cells / edges are masked out
-      else if (local + P.nzc < kMcBlockRuns) nxt = s_rows[local + P.nzc];
-      else nxt = row_bits(P, i, j + 1, k0, level) | (row_bits(P, i + 1, j + 1, k0, level) << 16);
-      packed[s] = run_codes(P, i, j, k0, own[s] & 0xffffu, own[s] >> 16, nxt & 0xffffu, nxt >> 16, codes[s], s_tricount);
+      else if (local + P.nzc < kMcBlockRuns) nxt = s_rows[local + P.nzc];   // row (i, j+1): the same scene
+      else nxt = row_bits(P, i, j + 1, k0, lv) | (row_bits(P, i + 1, j + 1, k0, lv) << 16);
+      packed[s] = run_codes(P, i, j, k0, BATCH ? (sc + 1) * P.nxs : P.nx, own[s] & 0xffffu, own[s] >> 16,
+                            nxt & 0xffffu, nxt >> 16, codes[s], s_tricount);
     }
   }
   // ---- one scan over the (s, thread) order: four independent warp scans, then the 32 warp totals in warp 0.
@@ -326,6 +350,11 @@ __global__ void __launch_bounds__(kMcThreads) mc_fused_kernel(const __grid_const
     const unsigned long long vb = (pre & 0x7fffffffull) + (excl & 0xffffu);
     const unsigned long long tb = (pre >> 31) + (excl >> 16);
     if (P.x_emit < P.nx && run == (long long)P.x_emit * P.ny * P.nzc) P.counts[0] = (long long)vb;   // first halo run
+    if (BATCH && (unsigned)run % P.scene_runs == 0) {                // first run of a scene: its bases
+      const unsigned sc = (unsigned)run / P.scene_runs;
+      P.sbase[2 * sc] = vb;
+      P.sbase[2 * sc + 1] = tb;
+    }
     if (!packed[s]) continue;
     reinterpret_cast<unsigned long long*>(P.code)[run] = codes[s];
     P.vbase[run] = (uint32_t)vb;
@@ -351,6 +380,7 @@ __device__ __forceinline__ int32_t vertex_id(const McParams& P, int i, int j, in
 // (up to 5) triangles of its cell.  One thread per run walked the 8 points serially through ~25 dependent
 // global loads (59 us for the 6 % active runs of a 256^3 grid); here a lane's chain is work item -> codes ->
 // grid samples -> neighbour codes / bases, and the samples of the run double as the vertex weights.
+template <bool BATCH>
 __global__ void __launch_bounds__(kMcThreads) mc_emit_kernel(const __grid_constant__ McParams P) {
   // case tables in shared memory: every lane indexes them with its own case (a divergent __constant__ index costs
   // one replay per distinct address); a case row is one 16-byte load
@@ -362,9 +392,16 @@ __global__ void __launch_bounds__(kMcThreads) mc_emit_kernel(const __grid_consta
     if (threadIdx.x < 12) *reinterpret_cast<int*>(s_edge[threadIdx.x]) = __ldg(reinterpret_cast<const int*>(kMcEdge) + threadIdx.x);
   }
   __syncthreads();
+  if (BATCH && blockIdx.x == 0) {   // per-scene counts: differences of consecutive scene bases (the last against the totals)
+    for (int s = threadIdx.x; s < P.n_vol; s += kMcThreads) {
+      const long long v1 = s + 1 < P.n_vol ? (long long)P.sbase[2 * s + 2] : P.counts[0];
+      const long long f1 = s + 1 < P.n_vol ? (long long)P.sbase[2 * s + 3] : P.counts[1];
+      P.scene_counts[2 * s] = v1 - (long long)P.sbase[2 * s];
+      P.scene_counts[2 * s + 1] = f1 - (long long)P.sbase[2 * s + 1];
+    }
+  }
   const unsigned n_work = P.ctrl[1];
-  const float level = mc_level(P);
-  const double dlevel = (double)level;
+  const float level0 = mc_level(P);
   const int lane = threadIdx.x & 31, t = lane & 7;
   const unsigned warps_total = gridDim.x * (kMcThreads / 32);
   const unsigned warp_global = blockIdx.x * (kMcThreads / 32) + (threadIdx.x >> 5);
@@ -377,6 +414,9 @@ __global__ void __launch_bounds__(kMcThreads) mc_emit_kernel(const __grid_consta
     int i, j, k0;
     run_coords(P, run, i, j, k0);
     const int k = k0 + t;
+    const int sc = BATCH ? i / P.nxs : 0;
+    const float level = BATCH ? scene_level(P, sc) : level0;
+    const double dlevel = (double)level;
     // samples of the four z-rows at this point (rows / samples outside the lattice replicate the last valid one,
     // as in row_bits: their cells / edges carry no flags)
     const int i1 = min(i + 1, P.nx - 1), j1 = min(j + 1, P.ny - 1), kc = min(k, P.nz - 1);
@@ -399,7 +439,7 @@ __global__ void __launch_bounds__(kMcThreads) mc_emit_kernel(const __grid_consta
     if (flags && i < P.x_emit) {
       unsigned long long vb = (unsigned long long)P.vbase[run] + (unsigned)__popcll(below & 0x0707070707070707ull);
       const double d0 = fabs((double)g00 - dlevel);
-      const float pbase[3] = {(float)(i + P.x_origin), (float)j, (float)k};
+      const float pbase[3] = {(float)(BATCH ? i - sc * P.nxs : i + P.x_origin), (float)j, (float)k};
       const float nb[3] = {g10, g01, n00};                       // the neighbour along x, y, z
 #pragma unroll
       for (int a = 0; a < 3; ++a) {
@@ -438,7 +478,7 @@ __global__ void __launch_bounds__(kMcThreads) mc_emit_kernel(const __grid_consta
         for (int corner = 0; corner < 3; ++corner) {
           const int e = (int)((reinterpret_cast<const unsigned*>(&row)[(3 * tr + corner) >> 2] >> (8 * ((3 * tr + corner) & 3))) & 0xffu);
           const char4 ed = *reinterpret_cast<const char4*>(s_edge[e]);
-          o[corner] = vertex_id(P, i + ed.y, j + ed.z, k + ed.w, ed.x);
+          o[corner] = vertex_id(P, i + ed.y, j + ed.z, k + ed.w, ed.x) - (BATCH ? (int32_t)P.sbase[2 * sc] : 0);
         }
       }
     }
@@ -463,6 +503,26 @@ __global__ void __launch_bounds__(256) grid_minmax_kernel(const float* __restric
   if ((threadIdx.x & 31) == 0 && lo <= hi) {
     atomicMin(keys, float_to_key(lo));
     atomicMax(keys + 1, float_to_key(hi));
+  }
+}
+
+// per-volume min / max of B volumes as ordered-int keys, merged into keys[2 b], keys[2 b + 1] (volume b =
+// blockIdx.y): the reduction the decoder kernels perform on the logits they store, so the keys are the ones a
+// single-scene decode of each volume produces
+__global__ void __launch_bounds__(256) volume_keys_kernel(const float* __restrict__ g, long long n,
+                                                          int32_t* __restrict__ keys) {
+  const float* v = g + (size_t)blockIdx.y * n;
+  int32_t lo = INT32_MAX, hi = INT32_MIN;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    const int32_t k = float_to_key(v[i]);
+    lo = min(lo, k);
+    hi = max(hi, k);
+  }
+  lo = __reduce_min_sync(0xffffffffu, lo);
+  hi = __reduce_max_sync(0xffffffffu, hi);
+  if ((threadIdx.x & 31) == 0 && lo <= hi) {
+    atomicMin(keys + 2 * blockIdx.y, lo);
+    atomicMax(keys + 2 * blockIdx.y + 1, hi);
   }
 }
 
@@ -497,6 +557,23 @@ extern "C" int64_t vtaco_mc_scratch_bytes(int32_t nx, int32_t ny, int32_t nz) {
   return mc_align(nruns * 8) + mc_align(4 * nruns) + mc_align(8 * nruns) + mc_align(8 * nb + 256);
 }
 
+extern "C" int64_t vtaco_mc_batch_scratch_bytes(int32_t n_volumes, int32_t nx, int32_t ny, int32_t nz) {
+  if (n_volumes < 1 || nx < 1 || (long long)n_volumes * nx >= (1ll << 31)) return VTACO_ERR_INVALID_ARG;
+  const int64_t b = vtaco_mc_scratch_bytes(n_volumes * nx, ny, nz);
+  return b < 0 ? b : b + mc_align(16ll * n_volumes);
+}
+
+extern "C" int vtaco_volume_keys(const float* grid, int32_t n_volumes, int64_t n, int32_t* keys, void* stream) {
+  if (!grid || !keys || n <= 0 || n_volumes < 1 || n_volumes > 65535) return VTACO_ERR_INVALID_ARG;
+  long long blocks = (n + 255) / 256;
+  long long cap = (long long)num_sms() * 8 / n_volumes;
+  if (cap < 1) cap = 1;
+  if (blocks > cap) blocks = cap;
+  volume_keys_kernel<<<dim3((unsigned)blocks, (unsigned)n_volumes), 256, 0, (cudaStream_t)stream>>>(grid, n, keys);
+  VTACO_LAUNCH_CHECK();
+  return VTACO_OK;
+}
+
 extern "C" int vtaco_grid_minmax(const float* grid, int64_t n, int32_t* keys, void* stream) {
   if (!grid || !keys || n <= 0) return VTACO_ERR_INVALID_ARG;
   cudaStream_t st = (cudaStream_t)stream;
@@ -514,18 +591,26 @@ extern "C" int vtaco_marching_cubes(const vtaco_mc_args* a, void* stream) {
   if (a->nx < 1 || a->ny < 1 || a->nz < 1) return VTACO_ERR_INVALID_ARG;
   if (a->phase < 1 || a->phase > 3) return VTACO_ERR_INVALID_ARG;
   if (a->x_emit < 0 || a->x_emit > a->nx) return VTACO_ERR_INVALID_ARG;
-  const long long n = (long long)a->nx * a->ny * a->nz;
+  if (a->n_volumes < 0) return VTACO_ERR_INVALID_ARG;
+  const bool batch = a->n_volumes > 1 || a->scene_counts;
+  const int n_vol = a->n_volumes > 1 ? a->n_volumes : 1;
+  if (batch && (!a->scene_counts || a->x_emit != 0 || a->x_origin != 0 || a->halo_rows != 0 || a->level_ptr ||
+                a->n_level_keys > 1))
+    return VTACO_ERR_INVALID_ARG;   // batched mode: whole volumes, one (min,max) pair or the level per volume
+  const long long n = (long long)n_vol * a->nx * a->ny * a->nz;
   if (n >= (1ll << 31)) return VTACO_ERR_UNSUPPORTED;
-  if (vtaco_mc_scratch_bytes(a->nx, a->ny, a->nz) > a->scratch_bytes) return VTACO_ERR_CAPACITY;
+  if ((batch ? vtaco_mc_batch_scratch_bytes(n_vol, a->nx, a->ny, a->nz) : vtaco_mc_scratch_bytes(a->nx, a->ny, a->nz)) >
+      a->scratch_bytes)
+    return VTACO_ERR_CAPACITY;
   if ((a->phase & 2) && ((a->vertex_capacity > 0 && !a->vertices) || (a->face_capacity > 0 && !a->faces)))
     return VTACO_ERR_INVALID_ARG;
   cudaStream_t st = (cudaStream_t)stream;
   McParams P = {};
   if (a->halo_rows < 0 || a->halo_rows >= a->nx || (a->halo_rows > 0 && !a->halo_grid)) return VTACO_ERR_INVALID_ARG;
-  P.grid = a->grid; P.nx = a->nx; P.ny = a->ny; P.nz = a->nz; P.npts = n;
+  P.grid = a->grid; P.nx = n_vol * a->nx; P.ny = a->ny; P.nz = a->nz; P.npts = n;
   P.halo = a->halo_rows > 0 ? a->halo_grid : nullptr;
-  P.x_local = a->nx - a->halo_rows;
-  P.x_emit = a->x_emit > 0 ? a->x_emit : a->nx;
+  P.x_local = P.nx - a->halo_rows;
+  P.x_emit = a->x_emit > 0 ? a->x_emit : P.nx;
   P.x_origin = a->x_origin;
   P.level = a->level; P.level_keys = a->level_keys; P.level_ptr = a->level_ptr;
   P.n_level_keys = a->n_level_keys > 1 ? a->n_level_keys : 1;
@@ -535,7 +620,7 @@ extern "C" int vtaco_marching_cubes(const vtaco_mc_args* a, void* stream) {
     if (P.nzc == (1 << sh)) P.nzc_shift = sh;
     if (P.ny == (1 << sh)) P.ny_shift = sh;
   }
-  P.nruns = (long long)a->nx * a->ny * P.nzc;
+  P.nruns = (long long)P.nx * a->ny * P.nzc;
   P.nblocks = (int)((P.nruns + kMcBlockRuns - 1) / kMcBlockRuns);
   char* s = reinterpret_cast<char*>(a->scratch);
   P.code = reinterpret_cast<uint8_t*>(s); s += mc_align(P.nruns * 8);
@@ -547,19 +632,32 @@ extern "C" int vtaco_marching_cubes(const vtaco_mc_args* a, void* stream) {
   P.verts = a->vertices; P.vcap = a->vertex_capacity;
   P.faces = a->faces; P.fcap = a->face_capacity;
   P.voffset = a->voffset; P.vscale = a->vscale;
+  if (batch) {
+    P.nxs = a->nx;
+    P.scene_runs = (unsigned)((long long)a->nx * a->ny * P.nzc);
+    P.n_vol = n_vol;
+    P.sbase = reinterpret_cast<unsigned long long*>(reinterpret_cast<char*>(a->scratch) +
+                                                    vtaco_mc_scratch_bytes(P.nx, P.ny, P.nz));
+    P.scene_counts = reinterpret_cast<long long*>(a->scene_counts);
+  }
   // phase 1 = count only (nothing is written to the outputs); 2 and 3 = the whole extraction (classification is
   // part of the same pass, so "emit after a count" simply runs it again with the larger buffers)
   P.emit = (a->phase & 2) ? 1 : 0;
   if (!P.emit) P.vcap = 0;
   VTACO_CUDA_CHECK(cudaMemsetAsync(P.state, 0, 8ll * P.nblocks + 16, st));
   {
-    const int resident = num_sms() * 6;     // 40 registers, 4.5 KB of shared memory: 6 CTAs per SM
-    mc_fused_kernel<<<P.nblocks < resident ? P.nblocks : resident, kMcThreads, 0, st>>>(P);
+    // 40 registers, 4.5 KB of shared memory: 6 CTAs per SM (the batched instantiation: 48 registers, 5)
+    const int resident = num_sms() * (batch ? 5 : 6);
+    const unsigned grid = P.nblocks < resident ? P.nblocks : resident;
+    if (batch) mc_fused_kernel<true><<<grid, kMcThreads, 0, st>>>(P);
+    else mc_fused_kernel<false><<<grid, kMcThreads, 0, st>>>(P);
   }
-  if (P.emit) {
+  if (P.emit || batch) {   // batched mode: the emit kernel also writes the per-scene counts (phase 1: one block, no work)
     long long blocks = (long long)num_sms() * 8;   // 8 lanes per work item; the kernel strides over the list
     if (blocks > (P.nruns * 8 + kMcThreads - 1) / kMcThreads) blocks = (P.nruns * 8 + kMcThreads - 1) / kMcThreads;
-    mc_emit_kernel<<<(unsigned)blocks, kMcThreads, 0, st>>>(P);
+    if (!P.emit) blocks = 1;
+    if (batch) mc_emit_kernel<true><<<(unsigned)blocks, kMcThreads, 0, st>>>(P);
+    else mc_emit_kernel<false><<<(unsigned)blocks, kMcThreads, 0, st>>>(P);
   }
   VTACO_LAUNCH_CHECK();
   return VTACO_OK;

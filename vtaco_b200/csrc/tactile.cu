@@ -8,7 +8,7 @@
 //     back-projected tactile point of sensor t takes sensor t's feature, sensors in increasing
 //     order, later ones overwrite (the reference's hard-coded `64**3 x 8` split, which only works
 //     for nx = 128, is not needed).
-#include "common.cuh"
+#include "decoder_common.cuh"
 #include <math_constants.h>
 
 namespace vtaco {
@@ -38,6 +38,36 @@ __global__ void __launch_bounds__(256) fingertip_ids_kernel(const float* __restr
       if (d < best) { best = d; bi = f; }
     }
     ids[i] = (bi >= 0 && best < T.radius && T.touch[bi]) ? (uint8_t)(bi + 1) : (uint8_t)0;
+  }
+}
+
+// per-scene fingertips on B dense lattices (blockIdx.y = scene): the decoder's own assignment (tip_assign), so the
+// ids equal what a single-scene decode with these fingertips assigns in the kernel
+__global__ void __launch_bounds__(256) fingertip_lattice_ids_kernel(const float* __restrict__ axis, int nx,
+                                                                    const double* __restrict__ tips,
+                                                                    const int32_t* __restrict__ touch, int n_tips,
+                                                                    double radius, uint8_t* __restrict__ ids) {
+  __shared__ DecParams sP;   // only the fingertip fields, which are all tip_assign reads
+  const int b = blockIdx.y;
+  if (threadIdx.x == 0) {
+    sP.n_tips = n_tips;
+    sP.tip_radius = radius;
+    sP.tip_r2_hi = tip_prefilter_r2(radius);
+    for (int f = 0; f < n_tips; ++f) {
+      for (int d = 0; d < 3; ++d) {
+        sP.tips[f][d] = tips[((size_t)b * n_tips + f) * 3 + d];
+        sP.tipsf[f][d] = (float)sP.tips[f][d];
+      }
+      sP.tip_touch[f] = touch[(size_t)b * n_tips + f];
+    }
+  }
+  __syncthreads();
+  const long long n = (long long)nx * nx * nx;
+  uint8_t* out = ids + (size_t)b * n;
+  for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q < n; q += (long long)gridDim.x * blockDim.x) {
+    const int iz = (int)(q % nx), iy = (int)((q / nx) % nx), ix = (int)(q / ((long long)nx * nx));
+    const int f = tip_assign(sP, __ldg(axis + ix), __ldg(axis + iy), __ldg(axis + iz));
+    out[q] = (uint8_t)(f + 1);
   }
 }
 
@@ -124,6 +154,22 @@ extern "C" int vtaco_tactile_point_map(const float* p, int64_t n, const float* a
     if (!axis || nx < 1) return VTACO_ERR_INVALID_ARG;
     point_map_dense_kernel<<<n_pts, 128, 0, st>>>(axis, nx, pts, radius, (uint8_t)value, map);
   }
+  VTACO_LAUNCH_CHECK();
+  return VTACO_OK;
+}
+
+extern "C" int vtaco_fingertip_lattice_ids(const float* axis, int32_t nx, int32_t B, const double* tips,
+                                           const int32_t* touch, int32_t n_tips, double radius, uint8_t* ids,
+                                           void* stream) {
+  if (!axis || !tips || !touch || !ids || nx < 1 || B < 1 || B > 65535 || n_tips < 1 || n_tips > VTACO_MAX_TIPS)
+    return VTACO_ERR_INVALID_ARG;
+  const long long n = (long long)nx * nx * nx;
+  long long blocks = (n + 255) / 256;
+  long long cap = (long long)num_sms() * 8 / B;
+  if (cap < 1) cap = 1;
+  if (blocks > cap) blocks = cap;
+  fingertip_lattice_ids_kernel<<<dim3((unsigned)blocks, (unsigned)B), 256, 0, (cudaStream_t)stream>>>(
+      axis, nx, tips, touch, n_tips, radius, ids);
   VTACO_LAUNCH_CHECK();
   return VTACO_OK;
 }
