@@ -413,10 +413,15 @@ int vtaco_scatter_mean(const float* c, const int32_t* idx32, int32_t B, int64_t 
  * (6) marching cubes over the decoded grid.
  * Replaces skimage.measure.marching_cubes(value_grid, gradient_direction='ascent')
  * and the vertex rescale of Generator3D.generate_obj_mesh_wnf
- * (src/conv_onet/generation.py:268-272).  grid: [nx][ny][nz] fp32 (axis0 = x).
+ * (src/conv_onet/generation.py:268-272).  grid: [nx][ny][nz] fp32 (axis0 = x), contiguous,
+ * with no alignment required (grid and halo_grid may start at any float).
  * level = `level`, or 0.5f*(min+max) decoded from `level_keys` (the ordered-int keys
- * the decoder kernel / vtaco_grid_minmax maintain) — skimage's level=None.
- * A corner is above iff value > level; one vertex per cut grid edge (id order =
+ * the decoder kernel / vtaco_grid_minmax / vtaco_volume_keys maintain) — skimage's level=None.
+ * The keys order a NaN beyond +-inf by its sign bit, so a volume holding a NaN has a NaN level
+ * (as numpy's min / max propagate NaN) and an empty mesh.
+ * A corner is above iff value > level, the IEEE ordered compare, for every float: +0 is not
+ * above -0, a NaN sample is above no level and no sample is above a NaN level.
+ * One vertex per cut grid edge (id order =
  * lattice order of the owning point, then axis); faces in lattice order of the
  * cell, then table order (oracle/mc_tables.py); vertices are
  * (index_coordinate - voffset) * vscale  (0,1 -> array-index coordinates).
@@ -471,7 +476,8 @@ typedef struct vtaco_mc_args {
 int64_t vtaco_mc_scratch_bytes(int32_t nx, int32_t ny, int32_t nz);
 int64_t vtaco_mc_batch_scratch_bytes(int32_t n_volumes, int32_t nx, int32_t ny, int32_t nz);
 int vtaco_marching_cubes(const vtaco_mc_args* args, void* stream);
-/* keys[0..1] <- ordered-int keys of min / max of grid[0..n) (initialised by the call) */
+/* keys[0..1] <- ordered-int keys of min / max of grid[0..n) (initialised by the call; the reduction of
+ * vtaco_volume_keys, so a NaN is the min or max by its sign bit) */
 int vtaco_grid_minmax(const float* grid, int64_t n, int32_t* keys, void* stream);
 /* per-volume keys of n_volumes contiguous volumes of n floats each: keys[2b], keys[2b+1] are merged
  * (atomicMin / atomicMax; the caller initialises them to INT32_MAX, INT32_MIN) with the ordered-int keys of

@@ -97,6 +97,38 @@ def test_empty_and_degenerate():
     assert len(f) >= 1
 
 
+def _edge_value_fields():
+    """ties (integers at levels 0 and 1), -0.0 / +0.0 at levels +0.0 and -0.0, and +-inf samples at level 0; each
+    padded with a value below every level so that the surface is closed"""
+    rs = np.random.RandomState(1)
+    zeros = np.array([-1.0, -0.0, 0.0, 1.0], dtype=np.float32)
+    inf = rs.randn(12, 13, 14).astype(np.float32)
+    inf[rs.rand(*inf.shape) < 0.15] = np.inf
+    inf[rs.rand(*inf.shape) < 0.15] = -np.inf
+    ties = rs.randint(-2, 3, size=(12, 13, 14)).astype(np.float32)
+    signed = zeros[rs.randint(0, 4, size=(12, 13, 14))]
+    out = [(ties, 0.0), (ties, 1.0), (signed, 0.0), (signed, -0.0), (inf, 0.0)]
+    return [(np.pad(v, 1, constant_values=-10.0), lv) for v, lv in out]
+
+
+@pytest.mark.parametrize('case', range(5))
+def test_edge_values_give_closed_oriented_manifold(case):
+    vol, level = _edge_value_fields()[case]
+    v, f, _ = mc.marching_cubes(vol, level=level)
+    s = mc.mesh_stats(v, f)
+    assert s['F'] > 100 and s['closed'] and s['oriented'] and s['all_vertices_used']
+    if case in (2, 3):                   # levels +0.0 and -0.0 select the same corners
+        v2, f2, _ = mc.marching_cubes(vol, level=-level)
+        assert np.array_equal(f, f2) and np.array_equal(v, v2)
+
+
+def test_unit_extent_has_vertices_and_no_faces():
+    rs = np.random.RandomState(2)
+    for shape in [(1, 12, 13), (12, 1, 13), (12, 13, 1), (1, 1, 16)]:
+        v, f, case = mc.marching_cubes(rs.randn(*shape).astype(np.float32), level=0.0)
+        assert len(v) > 0 and f.shape == (0, 3) and case.size == 0
+
+
 def test_rescale_matches_reference_formula():
     v = np.array([[0, 64, 128]], dtype=np.float32)
     out = mc.rescale_vertices(v, 128)

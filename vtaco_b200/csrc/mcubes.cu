@@ -51,6 +51,7 @@ struct McParams {
   int x_local;                    // rows of the sub-volume that live in `grid` (== nx without a separate halo)
   int nx, ny, nz, nzc;            // nzc = ceil(nz / kMcRun) runs per (x,y) row
   int nzc_shift, ny_shift;        // log2 when the extent is a power of two (run -> coordinates by shifts), else -1
+  int vec_rows;                   // rows are read as float4: nz % 8 == 0 and grid / halo 16-byte aligned
   int x_emit;                     // rows [0, x_emit) emit vertices / faces (== nx: whole volume)
   int x_origin;                   // lattice row of the sub-volume's row 0 (vertex coordinates are global)
   long long npts, nruns;
@@ -113,6 +114,11 @@ __device__ __forceinline__ const float* mc_row(const McParams& P, int i, int j) 
                        : P.halo + ((long long)(i - P.x_local) * P.ny + j) * P.nz;
 }
 
+// The one test of a corner against the level, in both kernels, so that a cell is emitted with the case it was counted
+// with: IEEE sample > level.  The compare is ordered: a NaN on either side is not above, and +0 is not above -0 (a
+// level of -0 selects what +0 does).
+__device__ __forceinline__ bool above(float sample, float level) { return sample > level; }
+
 // "above" bits of kMcRun+1 consecutive z samples of row (i,j), bit t <-> k0+t; rows or samples
 // outside the lattice replicate the last valid sample (their cells/edges are masked out later).
 __device__ __forceinline__ unsigned row_bits(const McParams& P, int i, int j, int k0, float level) {
@@ -120,25 +126,26 @@ __device__ __forceinline__ unsigned row_bits(const McParams& P, int i, int j, in
   j = min(j, P.ny - 1);
   const float* row = mc_row(P, i, j);
   unsigned bits = 0;
-  if ((P.nz & 7) == 0) {   // uniform over the grid: the last run of a row takes this path too (a per-lane
+  if (P.vec_rows) {        // uniform over the grid: the last run of a row takes this path too (a per-lane
                            // test sent one lane of EVERY warp through the scalar path below: 750 instructions per thread)
     const float4 a = __ldg(reinterpret_cast<const float4*>(row + k0));
     const float4 b = __ldg(reinterpret_cast<const float4*>(row + k0 + 4));
     const float c = __ldg(row + min(k0 + 8, P.nz - 1));
-    // sample > level  <=>  level - sample is negative (no flush-to-zero in this build: a difference of distinct
-    // floats is never zero); the sign bits are collected by funnel shifts, highest sample first
-    bits = __funnelshift_l(__float_as_uint(level - c), bits, 1);
-    bits = __funnelshift_l(__float_as_uint(level - b.w), bits, 1);
-    bits = __funnelshift_l(__float_as_uint(level - b.z), bits, 1);
-    bits = __funnelshift_l(__float_as_uint(level - b.y), bits, 1);
-    bits = __funnelshift_l(__float_as_uint(level - b.x), bits, 1);
-    bits = __funnelshift_l(__float_as_uint(level - a.w), bits, 1);
-    bits = __funnelshift_l(__float_as_uint(level - a.z), bits, 1);
-    bits = __funnelshift_l(__float_as_uint(level - a.y), bits, 1);
-    bits = __funnelshift_l(__float_as_uint(level - a.x), bits, 1);
+    // the bits by Horner's rule in float, highest sample first (exact below 2^24): a compare that yields 1.0f or 0
+    // and an FMA per sample, where an integer shift-in takes a compare, a select and a shift
+    float f = above(c, level);
+    f = fmaf(f, 2.f, above(b.w, level));
+    f = fmaf(f, 2.f, above(b.z, level));
+    f = fmaf(f, 2.f, above(b.y, level));
+    f = fmaf(f, 2.f, above(b.x, level));
+    f = fmaf(f, 2.f, above(a.w, level));
+    f = fmaf(f, 2.f, above(a.z, level));
+    f = fmaf(f, 2.f, above(a.y, level));
+    f = fmaf(f, 2.f, above(a.x, level));
+    bits = (unsigned)f;
   } else {
 #pragma unroll
-    for (int t = 0; t <= kMcRun; ++t) bits |= (unsigned)(__ldg(row + min(k0 + t, P.nz - 1)) > level) << t;
+    for (int t = 0; t <= kMcRun; ++t) bits |= (unsigned)above(__ldg(row + min(k0 + t, P.nz - 1)), level) << t;
   }
   return bits;
 }
@@ -201,8 +208,11 @@ __device__ __forceinline__ long long run_of(const McParams& P, int i, int j, int
 constexpr int kMcSub = 4;                          // consecutive 256-run sub-blocks per CTA: 4x fewer look-back words
 constexpr int kMcBlockRuns = kMcThreads * kMcSub;
 
+// resident CTAs per SM the fused kernel is compiled for (40 registers; batched: 48) and launched with
+constexpr int mc_fused_ctas_per_sm(bool batch) { return batch ? 5 : 6; }
+
 template <bool BATCH>
-__global__ void __launch_bounds__(kMcThreads) mc_fused_kernel(const __grid_constant__ McParams P) {
+__global__ void __launch_bounds__(kMcThreads, mc_fused_ctas_per_sm(BATCH)) mc_fused_kernel(const __grid_constant__ McParams P) {
   constexpr int kWarps = kMcThreads / 32;
   __shared__ int s_bid;
   __shared__ unsigned long long s_prefix;
@@ -448,8 +458,9 @@ __global__ void __launch_bounds__(kMcThreads) mc_emit_kernel(const __grid_consta
             const double d1 = fabs((double)nb[a] - dlevel);
             // Lewiner's weights w = 1 / (eps + d): t = w1 / (w0 + w1) = (eps + d0) / ((eps + d0) + (eps + d1)), one
             // division instead of three (equal to the last bit or two of the double, far below the float32 result)
+            // An infinite sample has weight 0, so the vertex sits at the other end, where e0 / (e0 + e1) is inf / inf
             const double e0 = (double)FLT_EPSILON + d0, e1 = (double)FLT_EPSILON + d1;
-            const double tt = e0 / (e0 + e1);
+            const double tt = e0 == INFINITY && e1 < INFINITY ? 1.0 : e0 / (e0 + e1);
             float pos[3] = {pbase[0], pbase[1], pbase[2]};
             pos[a] = (float)((double)pbase[a] + tt);
             float* o = P.verts + vb * 3;
@@ -464,9 +475,10 @@ __global__ void __launch_bounds__(kMcThreads) mc_emit_kernel(const __grid_consta
     // ---- triangles of the point's cell ----
     if (nt) {
       // corner c = x | y<<1 | z<<2
-      const unsigned cs = (unsigned)(g00 > level) | ((unsigned)(g10 > level) << 1) | ((unsigned)(g01 > level) << 2) |
-                          ((unsigned)(g11 > level) << 3) | ((unsigned)(n00 > level) << 4) | ((unsigned)(n10 > level) << 5) |
-                          ((unsigned)(n01 > level) << 6) | ((unsigned)(n11 > level) << 7);
+      const unsigned cs = (unsigned)above(g00, level) | ((unsigned)above(g10, level) << 1) |
+                          ((unsigned)above(g01, level) << 2) | ((unsigned)above(g11, level) << 3) |
+                          ((unsigned)above(n00, level) << 4) | ((unsigned)above(n10, level) << 5) |
+                          ((unsigned)above(n01, level) << 6) | ((unsigned)above(n11, level) << 7);
       // triangle base of the cell: the run's + the triangle counts of the points before it (byte sum by multiplication)
       const unsigned long long tb = (unsigned long long)item.y +
           ((((below >> 3) & 0x1f1f1f1f1f1f1f1full) * 0x0101010101010101ull) >> 56);
@@ -485,30 +497,10 @@ __global__ void __launch_bounds__(kMcThreads) mc_emit_kernel(const __grid_consta
   }
 }
 
-// min / max of a grid -> ordered-int keys (for level=None when the grid did not come from
-// the decoder kernel, which tracks them itself).
-__global__ void __launch_bounds__(256) grid_minmax_kernel(const float* __restrict__ g, long long n,
-                                                          int32_t* __restrict__ keys) {
-  float lo = INFINITY, hi = -INFINITY;
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-    const float v = g[i];
-    lo = fminf(lo, v);
-    hi = fmaxf(hi, v);
-  }
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) {
-    lo = fminf(lo, __shfl_xor_sync(0xffffffffu, lo, d));
-    hi = fmaxf(hi, __shfl_xor_sync(0xffffffffu, hi, d));
-  }
-  if ((threadIdx.x & 31) == 0 && lo <= hi) {
-    atomicMin(keys, float_to_key(lo));
-    atomicMax(keys + 1, float_to_key(hi));
-  }
-}
-
 // per-volume min / max of B volumes as ordered-int keys, merged into keys[2 b], keys[2 b + 1] (volume b =
 // blockIdx.y): the reduction the decoder kernels perform on the logits they store, so the keys are the ones a
-// single-scene decode of each volume produces
+// single-scene decode of each volume produces.  A NaN orders beyond +-inf by its sign bit, so a volume that holds
+// one has a NaN level.  vtaco_grid_minmax is the case B = 1.
 __global__ void __launch_bounds__(256) volume_keys_kernel(const float* __restrict__ g, long long n,
                                                           int32_t* __restrict__ keys) {
   const float* v = g + (size_t)blockIdx.y * n;
@@ -581,7 +573,7 @@ extern "C" int vtaco_grid_minmax(const float* grid, int64_t n, int32_t* keys, vo
   long long blocks = (n + 255) / 256;
   const long long cap = (long long)num_sms() * 8;
   if (blocks > cap) blocks = cap;
-  grid_minmax_kernel<<<(unsigned)blocks, 256, 0, st>>>(grid, n, keys);
+  volume_keys_kernel<<<(unsigned)blocks, 256, 0, st>>>(grid, n, keys);
   VTACO_LAUNCH_CHECK();
   return VTACO_OK;
 }
@@ -615,6 +607,10 @@ extern "C" int vtaco_marching_cubes(const vtaco_mc_args* a, void* stream) {
   P.level = a->level; P.level_keys = a->level_keys; P.level_ptr = a->level_ptr;
   P.n_level_keys = a->n_level_keys > 1 ? a->n_level_keys : 1;
   P.nzc = (a->nz + kMcRun - 1) / kMcRun;
+  // float4 row loads need 16-byte alignment; rows and runs start at multiples of 8 floats when nz % 8 == 0, so the
+  // base pointers decide (any contiguous view is accepted, e.g. one starting one float into a buffer)
+  P.vec_rows = (a->nz % kMcRun) == 0 && (reinterpret_cast<uintptr_t>(P.grid) & 15) == 0 &&
+               (reinterpret_cast<uintptr_t>(P.halo) & 15) == 0;
   P.nzc_shift = P.ny_shift = -1;
   for (int sh = 0; sh < 31; ++sh) {
     if (P.nzc == (1 << sh)) P.nzc_shift = sh;
@@ -646,8 +642,8 @@ extern "C" int vtaco_marching_cubes(const vtaco_mc_args* a, void* stream) {
   if (!P.emit) P.vcap = 0;
   VTACO_CUDA_CHECK(cudaMemsetAsync(P.state, 0, 8ll * P.nblocks + 16, st));
   {
-    // 40 registers, 4.5 KB of shared memory: 6 CTAs per SM (the batched instantiation: 48 registers, 5)
-    const int resident = num_sms() * (batch ? 5 : 6);
+    // 4.5 KB of shared memory: registers bound the CTAs per SM
+    const int resident = num_sms() * mc_fused_ctas_per_sm(batch);
     const unsigned grid = P.nblocks < resident ? P.nblocks : resident;
     if (batch) mc_fused_kernel<true><<<grid, kMcThreads, 0, st>>>(P);
     else mc_fused_kernel<false><<<grid, kMcThreads, 0, st>>>(P);

@@ -67,8 +67,9 @@ class MarchingCubes(object):
 
     def __call__(self, volume, level=None, level_keys=None, voffset=0.0, vscale=1.0, sync=True,
                  x_emit=None, x_origin=0, level_ptr=None, halo=None):
-        """volume: (nx,ny,nz) float32 CUDA tensor (axis0 = x).  level: float, or None ->
-        0.5*(min+max) (from `level_keys` if the decoder tracked them, else computed here);
+        """volume: (nx,ny,nz) float32 CUDA tensor (axis0 = x), any alignment.  level: float, or None ->
+        0.5*(min+max) (from `level_keys` if the decoder tracked them, else computed here; NaN, and so an empty
+        mesh, when the volume holds a NaN, as in .batch);
         `level_ptr`: address of a device float holding the level (multi-GPU exchange).
         Returns (vertices (V,3) float32, faces (F,3) int32) views of internal buffers
         (valid until the next call) — or, with sync=False, the un-trimmed buffers and the
