@@ -71,6 +71,9 @@ __device__ __forceinline__ int cell_of(float u, int reso) {
   return (int)__fmul_rn(u, (float)reso);
 }
 
+// A key's flat cell index stays in int32 range: reso^3 (grid) or reso^2 (plane) below 2^31.
+inline bool cell_index_fits(int kind, int reso) { return kind == VTACO_GRID ? reso <= 1290 : reso <= 46340; }
+
 // Monotone float <-> int32 key: signed-int order == float order (for atomicMin/Max).
 __host__ __device__ __forceinline__ int32_t float_to_key(float f) {
 #ifdef __CUDA_ARCH__

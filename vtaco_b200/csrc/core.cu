@@ -123,7 +123,7 @@ extern "C" int vtaco_point_to_cell(const float* p, int64_t n_points, double padd
   if (n_points == 0) return VTACO_OK;
   if (!p || n_points < 0 || reso < 1 || kind < 0 || kind > 3) return VTACO_ERR_INVALID_ARG;
   if (div_mode != VTACO_DIV_RECIPROCAL && div_mode != VTACO_DIV_TRUE) return VTACO_ERR_INVALID_ARG;
-  if (kind == VTACO_GRID ? reso > 1290 : reso > 46340) return VTACO_ERR_UNSUPPORTED;  // int32 flat index
+  if (!cell_index_fits(kind, reso)) return VTACO_ERR_UNSUPPORTED;
   const NormConst nc = make_norm_const(padding, div_mode);
   long long blocks = (n_points + 255) / 256;
   const long long cap = (long long)num_sms() * 8;

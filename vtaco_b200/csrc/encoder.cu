@@ -121,45 +121,6 @@ __device__ __forceinline__ void axpy32(float (&acc)[32], const float* __restrict
   }
 }
 
-// Warp walks its 32 points with lane == channel: store the row, fold runs of equal slot,
-// one row-wide atomic per run.  `col0` = first shared column of the warp.
-template <bool MEAN>
-__device__ __forceinline__ void scatter_rows(const float* __restrict__ sX, int col0, long long n0, long long nmax,
-                                             int lane, int nkeys, const int (&myslot)[4], float* const (&dst)[4],
-                                             float* __restrict__ row_out) {
-  int cur[4] = {-1, -1, -1, -1};
-  float val[4] = {0.f, 0.f, 0.f, 0.f};
-  for (int i = 0; i < 32; ++i) {
-    const long long ni = n0 + i;
-    if (ni >= nmax) break;  // uniform
-    const float v = sX[lane * kES + col0 + i];
-    if (row_out) row_out[ni * 32 + lane] = v;
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      if (k < nkeys && dst[k]) {
-        const int s = __shfl_sync(kFullMask, myslot[k], i);
-        if (s != cur[k]) {
-          if (cur[k] >= 0) {
-            if (MEAN) atomicAdd(dst[k] + (long long)cur[k] * 32 + lane, val[k]);
-            else atomic_max_float(dst[k] + (long long)cur[k] * 32 + lane, val[k]);
-          }
-          cur[k] = s;
-          val[k] = v;
-        } else {
-          val[k] = MEAN ? (val[k] + v) : fmaxf(val[k], v);
-        }
-      }
-    }
-  }
-#pragma unroll
-  for (int k = 0; k < 4; ++k) {
-    if (k < nkeys && dst[k] && cur[k] >= 0) {
-      if (MEAN) atomicAdd(dst[k] + (long long)cur[k] * 32 + lane, val[k]);
-      else atomic_max_float(dst[k] + (long long)cur[k] * 32 + lane, val[k]);
-    }
-  }
-}
-
 // One ResnetBlockFC(64 -> 32) per launch (layers.py:41-50) with its input assembly:
 //   FIRST : x = fc_pos(p)                                   pointnet.py:154,156
 //   else  : x = cat[net, pool_local(net)]                   pointnet.py:157-160
@@ -180,7 +141,8 @@ __device__ __forceinline__ void axpy8(float (&acc)[8], const float* __restrict__
   acc[4] = fmaf(w1.x, x, acc[4]); acc[5] = fmaf(w1.y, x, acc[5]); acc[6] = fmaf(w1.z, x, acc[6]); acc[7] = fmaf(w1.w, x, acc[7]);
 }
 
-// scatter_rows for points [i0, i1) of a 32-point group whose columns start at sX with stride `cs`
+// Points [i0, i1) of a 32-point group whose columns start at sX with stride `cs`, lane == channel: store the row,
+// fold runs of equal slot, one row-wide atomic per run (warp-aggregated).
 template <bool MEAN>
 __device__ __forceinline__ void scatter_rows_range(const float* __restrict__ sX, int cs, int i0, int i1, long long n0,
                                                    long long nmax, int lane, int nkeys, const int (&myslot)[4],
@@ -382,78 +344,42 @@ __global__ void __launch_bounds__(256) enc_finalize_kernel(const __grid_constant
   }
 }
 
-// ---- stand-alone row kernels behind vtaco_pool_local / vtaco_scatter_mean ----
+// ---- row kernels of the stand-alone pooling (vtaco_pool_local / vtaco_scatter_mean) and of the backward ----
+// Both pool into the cell rows P.pool[0] ([slot][32]) by P.slot.
+
+// src rows [n][32] -> their cell rows: sum (MEAN) or maximum
 template <bool MEAN>
-__global__ void __launch_bounds__(kET) rows_scatter_kernel(const float* __restrict__ src, long long n, int nkeys,
-                                                           const int32_t* s0, const int32_t* s1, const int32_t* s2,
-                                                           const int32_t* s3, float* d0, float* d1, float* d2,
-                                                           float* d3) {
+__global__ void __launch_bounds__(kET) rows_scatter_kernel(const __grid_constant__ EncParams P,
+                                                           const float* __restrict__ src) {
   __shared__ float sX[32 * kES];
   const int tid = threadIdx.x, lane = tid & 31, col0 = tid & ~31;
   const long long nb0 = (long long)blockIdx.x * kET;
   const long long me = nb0 + tid;
-  const int32_t* sl[4] = {s0, s1, s2, s3};
-  float* dst[4] = {d0, d1, d2, d3};
   int myslot[4] = {0, 0, 0, 0};
-  for (int k = 0; k < nkeys; ++k) myslot[k] = me < n ? sl[k][me] : 0;
+  for (int k = 0; k < P.nkeys; ++k) myslot[k] = me < P.n ? P.slot[k][me] : 0;
   for (int i = 0; i < 32; ++i) {
     const long long ni = nb0 + col0 + i;
-    if (ni >= n) break;
+    if (ni >= P.n) break;
     sX[lane * kES + col0 + i] = src[ni * 32 + lane];
   }
   __syncwarp();
-  scatter_rows<MEAN>(sX, col0, nb0 + col0, n, lane, nkeys, myslot, dst, nullptr);
+  scatter_rows_range<MEAN>(sX + col0, kES, 0, 32, nb0 + col0, P.n, lane, P.nkeys, myslot, P.pool[0], nullptr);
 }
 
-__global__ void __launch_bounds__(256) rows_gather_kernel(float* __restrict__ out, long long n, int nkeys, int mean,
-                                                          const int32_t* s0, const int32_t* s1, const int32_t* s2,
-                                                          const int32_t* s3, const float* d0, const float* d1,
-                                                          const float* d2, const float* d3, const int32_t* c0,
-                                                          const int32_t* c1, const int32_t* c2, const int32_t* c3) {
+// out[n] = sum over keys of the cell row of n (divided by the cell count for mean pooling)
+__global__ void __launch_bounds__(256) rows_gather_kernel(const __grid_constant__ EncParams P, float* __restrict__ out) {
   const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const long long ni = t >> 5;
   const int lane = threadIdx.x & 31;
-  if (ni >= n) return;
-  const int32_t* sl[4] = {s0, s1, s2, s3};
-  const float* src[4] = {d0, d1, d2, d3};
-  const int32_t* cnt[4] = {c0, c1, c2, c3};
+  if (ni >= P.n) return;
   float s = 0.f;
-  for (int k = 0; k < nkeys; ++k) {
-    const int r = sl[k][ni];
-    float v = src[k][(long long)r * 32 + lane];
-    if (mean) v = v / (float)cnt[k][r];
+  for (int k = 0; k < P.nkeys; ++k) {
+    const int r = P.slot[k][ni];
+    float v = P.pool[0][k][(long long)r * 32 + lane];
+    if (P.pool_mean) v = v / (float)P.count[k][r];
     s += v;
   }
   out[ni * 32 + lane] = s;
-}
-
-__global__ void __launch_bounds__(256) slot_kernel(const int32_t* __restrict__ idx, const int32_t* __restrict__ map,
-                                                   int32_t* __restrict__ slot, int32_t* __restrict__ count,
-                                                   float* __restrict__ pool, float init, long long n, long long T,
-                                                   long long cells) {
-  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const int s = map[(i / T) * cells + idx[i]];
-  slot[i] = s;
-  atomicAdd(count + s, 1);
-  if (pool) fill_row(pool + i * 32, init);
-}
-
-__global__ void __launch_bounds__(256) mean_finalize_kernel(const int32_t* __restrict__ idx,
-                                                            const int32_t* __restrict__ slot,
-                                                            const int32_t* __restrict__ count,
-                                                            const float* __restrict__ sum, float* __restrict__ out_cl,
-                                                            long long n, long long T, long long cells) {
-  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n || slot[i] != (int)i) return;
-  const float cnt = (float)count[i];
-  const float4* s4 = reinterpret_cast<const float4*>(sum + i * 32);
-  float4* o4 = reinterpret_cast<float4*>(out_cl + ((i / T) * cells + idx[i]) * 32);
-#pragma unroll
-  for (int j = 0; j < 8; ++j) {
-    const float4 s = s4[j];
-    o4[j] = make_float4(s.x / cnt, s.y / cnt, s.z / cnt, s.w / cnt);
-  }
 }
 
 static inline long long align_up(long long v, long long a) { return (v + a - 1) / a * a; }
@@ -473,6 +399,127 @@ static long long cells_of(int kind, int reso) {
   return kind == VTACO_GRID ? (long long)reso * reso * reso : (long long)reso * reso;
 }
 
+// Workspace of the inference forward: per key idx, slot, count, map, three pooling buffers and the scatter_mean
+// sums, then two net buffers.  Points P at it and returns its bytes; a null base only sizes it.
+static long long carve_enc_fwd(char* base, int B, long long T, int nkeys, const int32_t* kind, const int32_t* reso,
+                               EncParams& P) {
+  const long long n = (long long)B * T;
+  Carver c{base, 0};
+  for (int k = 0; k < nkeys; ++k) {
+    P.idx[k] = c.take<int32_t>(n); P.slot[k] = c.take<int32_t>(n); P.count[k] = c.take<int32_t>(n);
+    P.map[k] = c.take<int32_t>((long long)B * cells_of(kind[k], reso[k]));
+    for (int r = 0; r < 3; ++r) P.pool[r][k] = c.take<float>(n * 32);
+    P.sum[k] = c.take<float>(n * 32);
+  }
+  P.net[0] = c.take<float>(n * 32);
+  P.net[1] = c.take<float>(n * 32);
+  return c.off;
+}
+
+// Workspace of the stand-alone pooling: per key slot, count, map and the cell rows P.pool[0].  Points P at it and
+// returns its bytes; a null base only sizes it.
+static long long carve_pool(char* base, int B, long long T, int nkeys, const int64_t* cells, EncParams& P) {
+  const long long n = (long long)B * T;
+  Carver c{base, 0};
+  for (int k = 0; k < nkeys; ++k) {
+    P.slot[k] = c.take<int32_t>(n); P.count[k] = c.take<int32_t>(n);
+    P.map[k] = c.take<int32_t>((long long)B * cells[k]);
+    P.pool[0][k] = c.take<float>(n * 32);
+  }
+  return c.off;
+}
+
+// Keys and point count of the forward and the backward: 1..4 keys of a known kind with reso >= 1 (else
+// INVALID_ARG); fewer than n_max points and flat cell indices in int32 range (else UNSUPPORTED).
+static int check_keys(int n_keys, const int32_t* kind, const int32_t* reso, long long n, long long n_max) {
+  if (n_keys < 1 || n_keys > 4) return VTACO_ERR_INVALID_ARG;
+  if (n >= n_max) return VTACO_ERR_UNSUPPORTED;
+  for (int k = 0; k < n_keys; ++k) {
+    if (kind[k] < 0 || kind[k] > 3 || reso[k] < 1) return VTACO_ERR_INVALID_ARG;
+    if (!cell_index_fits(kind[k], reso[k])) return VTACO_ERR_UNSUPPORTED;
+  }
+  return VTACO_OK;
+}
+
+// Points, keys and weights of the forward and the backward (vtaco_encoder_args / vtaco_encoder_bwd_args).
+template <class Args>
+static EncParams enc_params(const Args* a) {
+  EncParams P = {};
+  P.p = a->p; P.n = (long long)a->B * a->T; P.T = a->T; P.B = a->B;
+  P.nc = make_norm_const(a->padding, a->div_mode);
+  P.nkeys = a->n_keys; P.pool_mean = a->pool_mean ? 1 : 0; P.n_blocks = a->n_blocks; P.W = a->weights;
+  for (int k = 0; k < a->n_keys; ++k) {
+    P.kind[k] = a->kind[k]; P.reso[k] = a->reso[k]; P.cells[k] = cells_of(a->kind[k], a->reso[k]);
+  }
+  return P;
+}
+
+// Per-key reset before the cell election: map = 0x7f7f7f7f, so that atomicMin elects a cell's lowest point; count = 0.
+static int reset_cells(const EncParams& P, cudaStream_t st) {
+  for (int k = 0; k < P.nkeys; ++k) {
+    VTACO_CUDA_CHECK(cudaMemsetAsync(P.map[k], 0x7f, sizeof(int32_t) * P.B * P.cells[k], st));
+    VTACO_CUDA_CHECK(cudaMemsetAsync(P.count[k], 0, sizeof(int32_t) * P.n, st));
+  }
+  return VTACO_OK;
+}
+
+// Cell election, slots and the ResnetBlockFC stack (pointnet.py:139-160), for the inference forward and for the
+// backward's recompute.  Block i reads pool level i, scatters into level i + 1 and initialises level i + 2, each only
+// if it is below nb (there is no level 0; enc_slot_kernel initialises level 1); it reads net level i - 1 and writes
+// net level i.  pool(l, k) and net(l) are the buffers of a level.  Each launch gets its window [level i, i + 1, i + 2]
+// in P.pool[0..2] and its net levels [i - 1, i] in P.net[0..1].
+template <class PoolLevel, class NetLevel>
+static int launch_block_stack(EncParams P, const PoolLevel& pool, const NetLevel& net, cudaStream_t st) {
+  const int nb = P.n_blocks;
+  const auto window = [&](int l) {
+    for (int w = 0; w < 3; ++w)
+      for (int k = 0; k < P.nkeys; ++k) P.pool[w][k] = (l + w >= 1 && l + w < nb) ? pool(l + w, k) : nullptr;
+  };
+  const int r = reset_cells(P, st);
+  if (r != VTACO_OK) return r;
+  const unsigned g256 = (unsigned)((P.n + 255) / 256);
+  enc_index_kernel<<<g256, 256, 0, st>>>(P);
+  window(1);
+  enc_slot_kernel<<<g256, 256, 0, st>>>(P, nb > 1);
+  const long long n_groups = (P.n + kEG - 1) / kEG;
+  const unsigned gB = enc_block_grid(n_groups);
+  for (int i = 0; i < nb; ++i) {
+    window(i);
+    P.net[0] = i > 0 ? net(i - 1) : nullptr;
+    P.net[1] = net(i);
+    const int r_write = i + 1 < nb ? 1 : -1, r_init = i + 2 < nb ? 2 : -1;
+    if (i == 0) enc_block_kernel<true><<<gB, 128, kEncBlockSmem, st>>>(P, 0, -1, r_write, r_init, 0, 1, n_groups);
+    else enc_block_kernel<false><<<gB, 128, kEncBlockSmem, st>>>(P, i, 0, r_write, r_init, 0, 1, n_groups);
+  }
+  VTACO_LAUNCH_CHECK();
+  return VTACO_OK;
+}
+
+// Stand-alone pooling of src rows [n][32] into the cell rows P.pool[0] by the caller's cell indices P.idx.
+static int pool_rows(const EncParams& P, const float* src, cudaStream_t st) {
+  const int r = reset_cells(P, st);
+  if (r != VTACO_OK) return r;
+  const unsigned g256 = (unsigned)((P.n + 255) / 256), gE = (unsigned)((P.n + kET - 1) / kET);
+  for (int k = 0; k < P.nkeys; ++k) map_min_kernel<<<g256, 256, 0, st>>>(P.idx[k], P.map[k], P.n, P.T, P.cells[k]);
+  enc_slot_kernel<<<g256, 256, 0, st>>>(P, 1);
+  if (P.pool_mean) rows_scatter_kernel<true><<<gE, kET, 0, st>>>(P, src);
+  else rows_scatter_kernel<false><<<gE, kET, 0, st>>>(P, src);
+  VTACO_LAUNCH_CHECK();
+  return VTACO_OK;
+}
+
+// EncParams of the stand-alone pooling: n = B * T points, the caller's cell indices and cell counts per key.
+static EncParams pool_params(int B, long long T, int nkeys, const int32_t* const* idx, const int64_t* cells, int mean) {
+  EncParams P = {};
+  P.n = (long long)B * T; P.T = T; P.B = B;
+  P.nkeys = nkeys; P.pool_mean = mean ? 1 : 0;
+  for (int k = 0; k < nkeys; ++k) {
+    P.idx[k] = const_cast<int32_t*>(idx[k]);   // enc_slot_kernel and enc_finalize_kernel only read idx
+    P.cells[k] = cells[k];
+  }
+  return P;
+}
+
 }  // namespace vtaco
 
 using namespace vtaco;
@@ -480,67 +527,38 @@ using namespace vtaco;
 extern "C" int64_t vtaco_encoder_workspace_bytes(int32_t B, int64_t T, int32_t n_keys, const int32_t* kind,
                                                  const int32_t* reso) {
   if (B <= 0 || T <= 0 || n_keys <= 0 || n_keys > 4 || !kind || !reso) return VTACO_ERR_INVALID_ARG;
-  const long long n = (long long)B * T;
-  Carver c{nullptr, 0};
-  for (int k = 0; k < n_keys; ++k) {
-    c.take<int32_t>(n); c.take<int32_t>(n); c.take<int32_t>(n);
-    c.take<int32_t>((long long)B * cells_of(kind[k], reso[k]));
-    for (int r = 0; r < 3; ++r) c.take<float>(n * 32);
-    c.take<float>(n * 32);
-  }
-  c.take<float>(n * 32); c.take<float>(n * 32);
-  return c.off;
+  EncParams P = {};
+  return carve_enc_fwd(nullptr, B, T, n_keys, kind, reso, P);
 }
 
 extern "C" int vtaco_encoder_pointnet(const vtaco_encoder_args* a, void* stream) {
   if (!a || !a->p || !a->weights || !a->workspace) return VTACO_ERR_INVALID_ARG;
-  if (a->B <= 0 || a->T <= 0 || a->n_keys <= 0 || a->n_keys > 4 || a->n_blocks < 1) return VTACO_ERR_INVALID_ARG;
+  if (a->B <= 0 || a->T <= 0 || a->n_blocks < 1) return VTACO_ERR_INVALID_ARG;
   const long long n = (long long)a->B * a->T;
-  if (n >= (1ll << 31)) return VTACO_ERR_UNSUPPORTED;
-  for (int k = 0; k < a->n_keys; ++k) {
-    if (a->kind[k] < 0 || a->kind[k] > 3 || a->reso[k] < 1) return VTACO_ERR_INVALID_ARG;
-    if (a->kind[k] == VTACO_GRID ? a->reso[k] > 1290 : a->reso[k] > 46340) return VTACO_ERR_UNSUPPORTED;
-  }
-  if (vtaco_encoder_workspace_bytes(a->B, a->T, a->n_keys, a->kind, a->reso) > a->workspace_bytes)
+  int r = check_keys(a->n_keys, a->kind, a->reso, n, 1ll << 31);
+  if (r != VTACO_OK) return r;
+  EncParams P = enc_params(a);
+  if (carve_enc_fwd(reinterpret_cast<char*>(a->workspace), a->B, a->T, a->n_keys, a->kind, a->reso, P) >
+      a->workspace_bytes)
     return VTACO_ERR_CAPACITY;
   cudaStream_t st = (cudaStream_t)stream;
-  EncParams P = {};
-  P.p = a->p; P.n = n; P.T = a->T; P.B = a->B;
-  P.nc = make_norm_const(a->padding, a->div_mode);
-  P.nkeys = a->n_keys; P.pool_mean = a->pool_mean ? 1 : 0; P.n_blocks = a->n_blocks; P.W = a->weights;
   P.c_out = a->c_out;
-  Carver c{reinterpret_cast<char*>(a->workspace), 0};
   for (int k = 0; k < a->n_keys; ++k) {
-    P.kind[k] = a->kind[k]; P.reso[k] = a->reso[k]; P.cells[k] = cells_of(a->kind[k], a->reso[k]);
-    P.idx[k] = c.take<int32_t>(n); P.slot[k] = c.take<int32_t>(n); P.count[k] = c.take<int32_t>(n);
-    P.map[k] = c.take<int32_t>((long long)a->B * P.cells[k]);
-    for (int r = 0; r < 3; ++r) P.pool[r][k] = c.take<float>(n * 32);
-    P.sum[k] = c.take<float>(n * 32);
     P.out_cl[k] = a->out_cl[k];
-    VTACO_CUDA_CHECK(cudaMemsetAsync(P.map[k], 0x7f, sizeof(int32_t) * a->B * P.cells[k], st));
-    VTACO_CUDA_CHECK(cudaMemsetAsync(P.count[k], 0, sizeof(int32_t) * n, st));
     VTACO_CUDA_CHECK(cudaMemsetAsync(P.sum[k], 0, sizeof(float) * n * 32, st));
     if (P.out_cl[k])
       VTACO_CUDA_CHECK(cudaMemsetAsync(P.out_cl[k], 0, sizeof(float) * a->B * P.cells[k] * 32, st));
   }
-  P.net[0] = c.take<float>(n * 32);
-  P.net[1] = c.take<float>(n * 32);
-
-  const unsigned g256 = (unsigned)((n + 255) / 256);
-  enc_index_kernel<<<g256, 256, 0, st>>>(P);
-  enc_slot_kernel<<<g256, 256, 0, st>>>(P, 1);
-  const long long n_groups = (n + kEG - 1) / kEG;
-  const unsigned gB = enc_block_grid(n_groups);
   const int nb = a->n_blocks;
-  // kernel i reads pool[(i-1)%3], scatters into pool[i%3], initialises pool[(i+1)%3]
-  enc_block_kernel<true><<<gB, 128, kEncBlockSmem, st>>>(P, 0, -1, nb > 1 ? 0 : -1, nb > 2 ? 1 : -1, 0, 0, n_groups);
-  for (int i = 1; i < nb; ++i) {
-    const bool last = (i == nb - 1);
-    enc_block_kernel<false><<<gB, 128, kEncBlockSmem, st>>>(P, i, (i - 1) % 3, last ? -1 : i % 3,
-                                                            (i + 1 < nb - 1) ? (i + 1) % 3 : -1, (i - 1) & 1, i & 1, n_groups);
-  }
-  enc_final_kernel<<<gB, 128, kEncFinalSmem, st>>>(P, (nb - 1) & 1, n_groups);
-  enc_finalize_kernel<<<g256, 256, 0, st>>>(P);
+  const auto pool_level = [&](int l, int k) { return P.pool[(l - 1) % 3][k]; };   // three buffers in turn
+  const auto net_level = [&](int l) { return P.net[l & 1]; };                      // two buffers in turn
+  r = launch_block_stack(P, pool_level, net_level, st);
+  if (r != VTACO_OK) return r;
+  EncParams F = P;   // fc_c reads the output of the last block
+  F.net[0] = net_level(nb - 1);
+  const long long n_groups = (n + kEG - 1) / kEG;
+  enc_final_kernel<<<enc_block_grid(n_groups), 128, kEncFinalSmem, st>>>(F, 0, n_groups);
+  enc_finalize_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(P);
   VTACO_LAUNCH_CHECK();
   for (int k = 0; k < a->n_keys; ++k)
     if (a->index_out[k])
@@ -550,14 +568,8 @@ extern "C" int vtaco_encoder_pointnet(const vtaco_encoder_args* a, void* stream)
 
 extern "C" int64_t vtaco_pool_workspace_bytes(int32_t B, int64_t T, int32_t n_keys, const int64_t* cells) {
   if (B <= 0 || T <= 0 || n_keys <= 0 || n_keys > 4 || !cells) return VTACO_ERR_INVALID_ARG;
-  const long long n = (long long)B * T;
-  Carver c{nullptr, 0};
-  for (int k = 0; k < n_keys; ++k) {
-    c.take<int32_t>(n); c.take<int32_t>(n);
-    c.take<int32_t>((long long)B * cells[k]);
-    c.take<float>(n * 32);
-  }
-  return c.off;
+  EncParams P = {};
+  return carve_pool(nullptr, B, T, n_keys, cells, P);
 }
 
 extern "C" int vtaco_pool_local(const float* feat, int32_t B, int64_t T, int32_t n_keys, const int32_t* const* idx32,
@@ -565,35 +577,14 @@ extern "C" int vtaco_pool_local(const float* feat, int32_t B, int64_t T, int32_t
                                 float* out, void* stream) {
   if (!feat || !idx32 || !cells || !workspace || !out) return VTACO_ERR_INVALID_ARG;
   if (B <= 0 || T <= 0 || n_keys <= 0 || n_keys > 4) return VTACO_ERR_INVALID_ARG;
-  if (vtaco_pool_workspace_bytes(B, T, n_keys, cells) > workspace_bytes) return VTACO_ERR_CAPACITY;
-  const long long n = (long long)B * T;
-  if (n >= (1ll << 31)) return VTACO_ERR_UNSUPPORTED;
+  EncParams P = pool_params(B, T, n_keys, idx32, cells, mean);
+  if (carve_pool(reinterpret_cast<char*>(workspace), B, T, n_keys, cells, P) > workspace_bytes)
+    return VTACO_ERR_CAPACITY;
+  if (P.n >= (1ll << 31)) return VTACO_ERR_UNSUPPORTED;
   cudaStream_t st = (cudaStream_t)stream;
-  Carver c{reinterpret_cast<char*>(workspace), 0};
-  int32_t* slot[4] = {nullptr, nullptr, nullptr, nullptr};
-  int32_t* count[4] = {nullptr, nullptr, nullptr, nullptr};
-  float* pool[4] = {nullptr, nullptr, nullptr, nullptr};
-  const unsigned g256 = (unsigned)((n + 255) / 256);
-  for (int k = 0; k < n_keys; ++k) {
-    slot[k] = c.take<int32_t>(n); count[k] = c.take<int32_t>(n);
-    int32_t* map = c.take<int32_t>((long long)B * cells[k]);
-    pool[k] = c.take<float>(n * 32);
-    VTACO_CUDA_CHECK(cudaMemsetAsync(map, 0x7f, sizeof(int32_t) * B * cells[k], st));
-    VTACO_CUDA_CHECK(cudaMemsetAsync(count[k], 0, sizeof(int32_t) * n, st));
-    map_min_kernel<<<g256, 256, 0, st>>>(idx32[k], map, n, T, cells[k]);
-    slot_kernel<<<g256, 256, 0, st>>>(idx32[k], map, slot[k], count[k], pool[k], mean ? 0.f : -INFINITY, n, T,
-                                      cells[k]);
-  }
-  const unsigned gE = (unsigned)((n + kET - 1) / kET);
-  if (mean)
-    rows_scatter_kernel<true><<<gE, kET, 0, st>>>(feat, n, n_keys, slot[0], slot[1], slot[2], slot[3], pool[0],
-                                                  pool[1], pool[2], pool[3]);
-  else
-    rows_scatter_kernel<false><<<gE, kET, 0, st>>>(feat, n, n_keys, slot[0], slot[1], slot[2], slot[3], pool[0],
-                                                   pool[1], pool[2], pool[3]);
-  rows_gather_kernel<<<(unsigned)((n * 32 + 255) / 256), 256, 0, st>>>(
-      out, n, n_keys, mean, slot[0], slot[1], slot[2], slot[3], pool[0], pool[1], pool[2], pool[3], count[0], count[1],
-      count[2], count[3]);
+  const int r = pool_rows(P, feat, st);
+  if (r != VTACO_OK) return r;
+  rows_gather_kernel<<<(unsigned)((P.n * 32 + 255) / 256), 256, 0, st>>>(P, out);
   VTACO_LAUNCH_CHECK();
   return VTACO_OK;
 }
@@ -601,25 +592,16 @@ extern "C" int vtaco_pool_local(const float* feat, int32_t B, int64_t T, int32_t
 extern "C" int vtaco_scatter_mean(const float* c, const int32_t* idx32, int32_t B, int64_t T, int64_t cells,
                                   void* workspace, int64_t workspace_bytes, float* out_cl, void* stream) {
   if (!c || !idx32 || !workspace || !out_cl || B <= 0 || T <= 0 || cells <= 0) return VTACO_ERR_INVALID_ARG;
-  const int64_t cells1[1] = {cells};
-  if (vtaco_pool_workspace_bytes(B, T, 1, cells1) > workspace_bytes) return VTACO_ERR_CAPACITY;
-  const long long n = (long long)B * T;
-  if (n >= (1ll << 31)) return VTACO_ERR_UNSUPPORTED;
+  EncParams P = pool_params(B, T, 1, &idx32, &cells, 1);
+  if (carve_pool(reinterpret_cast<char*>(workspace), B, T, 1, &cells, P) > workspace_bytes) return VTACO_ERR_CAPACITY;
+  if (P.n >= (1ll << 31)) return VTACO_ERR_UNSUPPORTED;
   cudaStream_t st = (cudaStream_t)stream;
-  Carver cv{reinterpret_cast<char*>(workspace), 0};
-  int32_t* slot = cv.take<int32_t>(n);
-  int32_t* count = cv.take<int32_t>(n);
-  int32_t* map = cv.take<int32_t>((long long)B * cells);
-  float* sum = cv.take<float>(n * 32);
-  VTACO_CUDA_CHECK(cudaMemsetAsync(map, 0x7f, sizeof(int32_t) * B * cells, st));
-  VTACO_CUDA_CHECK(cudaMemsetAsync(count, 0, sizeof(int32_t) * n, st));
+  P.sum[0] = P.pool[0][0];
+  P.out_cl[0] = out_cl;
   VTACO_CUDA_CHECK(cudaMemsetAsync(out_cl, 0, sizeof(float) * B * cells * 32, st));
-  const unsigned g256 = (unsigned)((n + 255) / 256), gE = (unsigned)((n + kET - 1) / kET);
-  map_min_kernel<<<g256, 256, 0, st>>>(idx32, map, n, T, cells);
-  slot_kernel<<<g256, 256, 0, st>>>(idx32, map, slot, count, sum, 0.f, n, T, cells);
-  rows_scatter_kernel<true><<<gE, kET, 0, st>>>(c, n, 1, slot, nullptr, nullptr, nullptr, sum, nullptr, nullptr,
-                                                nullptr);
-  mean_finalize_kernel<<<g256, 256, 0, st>>>(idx32, slot, count, sum, out_cl, n, T, cells);
+  const int r = pool_rows(P, c, st);
+  if (r != VTACO_OK) return r;
+  enc_finalize_kernel<<<(unsigned)((P.n + 255) / 256), 256, 0, st>>>(P);
   VTACO_LAUNCH_CHECK();
   return VTACO_OK;
 }
